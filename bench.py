@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU: the oracle port of the reference
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic start states:
 H-step model rollout (policy -> PENS ensemble -> FakeEnv statics -> ModelBuffer write-out), GAE +
@@ -404,6 +405,39 @@ def run_reference(args, rank, world):
 # ------------------------------------------------------------------------------------------------
 # CUDA arm
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 48 << 20      # budget of the sampled per-path fields of --dump-outputs (the whole dump stays below 64 MB)
+
+
+def dump_outputs(out_dir, bufs, sums):
+    """--dump-outputs: what the last timed pass leaves for its caller, as <out_dir>/<name>.npy in float32 / float64.
+    `adv_stats_sums` are the 8 float64 advantage-statistics sums of the whole batch (all ranks).  Every per-step and
+    per-path field of the rollout buffers is written for a fixed sample of paths (seed 0, listed in `path_index`,
+    as many as fit DUMP_BYTES) in the reference's [path, step, ...] layout, with the steps at or past a path's
+    length zeroed: they are not part of its sample list.  Integer fields are written as float32 (exact: small)."""
+    import torch
+    from cmbpo_b200.rollout import STEP_FIELDS_VEC, STEP_FIELDS, GAE_FIELDS
+    step_fields = STEP_FIELDS_VEC + STEP_FIELDS + GAE_FIELDS + ("term",)
+    path_fields = ("length", "end_reason", "last_val", "last_cval", "cum_dkl", "final_obs")
+    path_bytes = sum(bufs.T * getattr(bufs, f)[0, 0].numel() * 4 for f in step_fields) + \
+        sum(getattr(bufs, f)[0].numel() * 8 for f in path_fields)
+    n = min(bufs.B, DUMP_BYTES // path_bytes)
+    idx = np.sort(np.random.default_rng(0).choice(bufs.B, n, replace=False))
+    sel = torch.from_numpy(idx).to(bufs.length.device)
+    alive = torch.arange(bufs.T, device=sel.device)[None, :] < bufs.length.index_select(0, sel).long()[:, None]
+    out = {"path_index": torch.from_numpy(idx.astype(np.float64)), "adv_stats_sums": sums}
+    for f in step_fields:
+        x = getattr(bufs, f).index_select(1, sel).transpose(0, 1)           # time-major [T, B, ...] -> [n, T, ...]
+        out[f] = torch.where(alive if x.dim() == 2 else alive[..., None], x, torch.zeros((), dtype=x.dtype, device=x.device))
+    for f in path_fields:
+        out[f] = getattr(bufs, f).index_select(0, sel)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in out.items():
+        a = x.cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 class Rig:
     """One rank's engine with the synthetic networks of a task shape loaded (weights generated on rank 0 and
     broadcast once over NCCL, then uploaded from device memory)."""
@@ -472,8 +506,9 @@ class Rig:
     def row_bytes(self):
         return (2 * self.O + 3 * self.A + 6) * 4 + 2          # SURVEY.md 8d: write-out bytes per stored transition
 
-    def timed_rollouts(self, B, T, steps, warmup, seed0=1234, with_stats=True):
-        """`steps` passes of rollout -> GAE -> statistics -> normalise over B device-resident start states.
+    def timed_rollouts(self, B, T, steps, warmup, seed0=1234, with_stats=True, dump=True):
+        """`steps` passes of rollout -> GAE -> statistics -> normalise over B device-resident start states; with
+        --dump-outputs and `dump`, rank 0 then writes the outputs of the last pass.
         Returns dict(ms, n_tr (whole job), launches, dyn_launch_ms, gae_launch_ms, breakdown, clocks)."""
         torch, eng, L = self.torch, self.eng, self.L
         obs_host, _ = self.wl.make_states(100 + self.rank, B, self.O, self.A, self.dyn)
@@ -506,7 +541,8 @@ class Rig:
         ev0.record()
         n_acc = torch.zeros(1, device=self.dev, dtype=torch.float64)
         for s_ in range(steps):
-            n_acc += hot_path(s_)[0:1]    # with N > 1 the statistics are all-reduced: already the whole-job count
+            sums = hot_path(s_)
+            n_acc += sums[0:1]            # with N > 1 the statistics are all-reduced: already the whole-job count
         ev1.record()
         self.barrier()
         clk = clocks.stop()
@@ -517,6 +553,8 @@ class Rig:
             t_ms, n = eng.profile_read(k, True)
             res[name + "_ms"], res[name + "_n"] = t_ms, n
         eng.profile(False)
+        if dump and self.args.dump_outputs and self.rank == 0:
+            dump_outputs(self.args.dump_outputs, bufs, sums)
         del bufs
         return res
 
@@ -932,7 +970,8 @@ def bench_sweep(rig, args, cfg):
         B = max(1, Btot // world)
         for H in Hs:
             steps = max(2, min(args.steps, int(2e8 / max(B * H, 1)) + 2))       # small cells: more repetitions
-            res = rig.timed_rollouts(B, H + 1, steps, max(1, min(args.warmup, 2)))
+            last_cell = Btot == Bs[-1] and H == Hs[-1]          # the cell `value` reports is the one dumped
+            res = rig.timed_rollouts(B, H + 1, steps, max(1, min(args.warmup, 2)), dump=last_cell)
             (ms, dyn_launch_ms, gae_launch_ms), (n_tr, launches) = rig.reduce_result(res)
             launches_total += launches
             clk = res["clocks"]
@@ -951,6 +990,7 @@ def bench_sweep(rig, args, cfg):
     big = cells[-1]
     line = base_line(rig, args, cfg, big["transitions_per_s"], big["ms_per_pass"], {
         "value_is": "the largest cell (H=%d, B_total=%d)" % (big["H"], big["B_total"]), "horizons": Hs, "batches_total": Bs,
+        "passes_per_cell": "max(2, min(--steps, 2e8 / (B_per_gpu x H) + 2)), listed as cells[].passes",
         "l2": "cells below ~50k start states per GPU fit the 126 MB L2; no explicit flush",
         "flop_per_transition": fdyn + fact + fvvc})
     line["roofline"] = {"bound": "tensor", "kernel": "dynamics-ensemble GEMM chain (K1), largest cell", "achieved": big["k1_TFLOPs"],
@@ -971,7 +1011,9 @@ L_PROF_DYN, L_PROF_GAE = 0, 1
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed passes of the hot path; --config sweep: per cell max(2, min(STEPS, 2e8 / (B x H) + 2)), "
+                         "reported as cells[].passes")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--precision", default="fp16", choices=["fp32", "fp16", "bf16"])
@@ -986,7 +1028,15 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not pin ranks to their GPU's NUMA-local cores")
     ap.add_argument("--sweep-h", default="1,2,5,10,20,30")
     ap.add_argument("--sweep-b", default="10000,100000,1000000,4000000")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0; a fixed "
+                         "sample of paths, < 64 MB; --config sweep: the last cell, the one `value` reports); the inputs "
+                         "depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
     # stdout carries exactly ONE JSON line: anything libraries print at C level while the job runs
     # (NCCL's version banner) goes to stderr; the real stdout is restored for the final print
     global _REAL_STDOUT

@@ -1,6 +1,6 @@
 """CPU: the PE checkpoint reader (cmbpo_b200/checkpoint.py) against files laid out like PE.save
-(models/pens/pe.py:736-764) writes them; where /root/reference is present the layer descriptions are
-produced by the reference's own FC.__repr__ (models/pens/fc.py:46-50)."""
+(models/pens/pe.py:736-764) writes them; where the reference source tree (CMBPO_REFERENCE_ROOT) is present, the layer
+descriptions are also produced by the reference's own FC.__repr__ (models/pens/fc.py:46-50)."""
 import os
 
 import numpy as np
@@ -75,7 +75,7 @@ def test_malformed_files_fail_loudly(tmp_path):
         ck.read_pe_checkpoint(str(tmp_path), "M", 1)
 
 
-@pytest.mark.skipif(not ref_stubs.reference_available(), reason="/root/reference not present")
+@pytest.mark.skipif(not ref_stubs.reference_available(), reason="reference source tree not present")
 def test_layer_lines_are_the_references_repr(tmp_path):
     ref = ref_stubs.load()
     import importlib

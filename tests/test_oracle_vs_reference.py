@@ -1,16 +1,18 @@
-"""CPU, build container only: the oracle against the reference's UNMODIFIED host code, live
+"""CPU: the oracle against the reference's UNMODIFIED host code, live
 (FakeEnv / ModelSampler / ModelBuffer / CPOBuffer / statics / average_dkl / discount_cumsum imported
-from /root/reference through oracle/ref_stubs.py).  Skipped where /root/reference is absent."""
+through oracle/ref_stubs.py from the reference source tree, CMBPO_REFERENCE_ROOT).  The tests that import it
+are skipped where that tree is absent."""
 import numpy as np
 import pytest
 
 from oracle import cmbpo_oracle as orc, ref_stubs
 
-pytestmark = pytest.mark.skipif(not ref_stubs.reference_available(), reason="/root/reference not present")
+needs_reference = pytest.mark.skipif(not ref_stubs.reference_available(), reason="reference source tree not present")
 GAE = dict(gamma=0.99, lam=0.95, cgamma=0.97, clam=0.5)
 TASKS = [("HalfCheetahSafe-v2", 17, 6), ("AntSafe-v2", 29, 8), ("HumanoidSafe-v2", 47, 17)]
 
 
+@needs_reference
 @pytest.mark.parametrize("task,O,A", TASKS)
 @pytest.mark.parametrize("mode", [False, "uncertainty"])
 def test_full_cycle_bit_exact(task, O, A, mode):
@@ -46,12 +48,14 @@ def test_choice_equals_randint_positions():
     assert np.array_equal(a, b)
 
 
+@needs_reference
 def test_mpi_statistics_scalar():
     ref = ref_stubs.load()
     x = np.random.default_rng(0).standard_normal(5001).astype(np.float32) * 3 + 1
     assert ref.mpi_statistics_scalar(x) == orc.stats_scalar(x)
 
 
+@needs_reference
 def test_boltz_dist_and_policy_kl_formula_live():
     """Oracle boltz_dist / epochs_list against the reference's CPOBuffer methods on a fresh case."""
     from oracle import gen_golden
