@@ -64,7 +64,6 @@ SIGNATURES = {
     "cmbpo_ctx_set_stream": (_i, [_vp, _vp]),
     "cmbpo_ctx_synchronize": (_i, [_vp]),
     "cmbpo_ctx_launch_count": (_i64, [_vp]),
-    "cmbpo_ctx_set_debug": (_i, [_vp, _i, _i]),
     "cmbpo_ctx_profile": (_i, [_vp, _i]),
     "cmbpo_ctx_profile_read": (_i, [_vp, _i, C.POINTER(_d), C.POINTER(_i64), _i]),
     "cmbpo_net_set_weights": (_i, [_vp, _i, _i, _i, C.POINTER(_i), C.POINTER(_vp), C.POINTER(_vp),

@@ -93,13 +93,6 @@ extern "C" int cmbpo_ctx_synchronize(cmbpo_ctx* ctx) {
 
 extern "C" int64_t cmbpo_ctx_launch_count(cmbpo_ctx* ctx) { return ctx ? ctx->launches : 0; }
 
-extern "C" int cmbpo_ctx_set_debug(cmbpo_ctx* ctx, int tc_debug, int trace_only) {
-    CMBPO_CHECK(ctx, "null context");
-    ctx->tc_debug = tc_debug;
-    ctx->tc_trace_only = trace_only;
-    return 0;
-}
-
 extern "C" int cmbpo_ctx_profile(cmbpo_ctx* ctx, int enable) {
     CMBPO_CHECK(ctx, "null context");
     ctx->profile = enable != 0;

@@ -72,7 +72,6 @@ struct ProfSlot {
 
 struct cmbpo_ctx {
     bool profile = false;
-    int tc_debug = 0, tc_trace_only = 0;   // cmbpo_ctx_set_debug: protocol tracing of the tcgen05 kernels (tools/)
     ProfSlot prof[CMBPO_PROF_SLOTS];
     int device = 0;
     cudaStream_t stream = nullptr;

@@ -62,7 +62,6 @@ struct TcParams {
     float* out; long long out_member_stride;   // out[e*stride + row*Nout + c]
     int ntiles;
     int member_act[CMBPO_MAX_E];   // ACT == 0 kernels (merged nets): hidden activation per member
-    unsigned long long* dbg;   // optional [grid][16] cycle counters (protocol timing aid)
     FusedStep fz;              // FUSE kernels only: the rollout step around the GEMM chain (step_common.cuh)
 };
 
@@ -233,34 +232,6 @@ __device__ __forceinline__ void fused_rows(const FusedStep& f, const FzSmem& sm,
 }
 
 
-// event trace of CTA 0, member 8 (steady state), kept in shared memory so that tracing does not
-// perturb the timeline; 5 streams (MMA thread, the lane-quarter-0 warp of each epilogue warpgroup) x 40
-// events of (tag, clock)
-#define TRACE_EVENTS 48
-#define TRACE_WORDS (2 + 2 * TRACE_EVENTS)
-#define TRACE_STREAMS 5
-#define TRACE(stream, tag)                                                                    \
-    if (DBG && p.dbg && blockIdx.x == 0 && m == 8 && lane == 0 && (warp == 1 || (warp & 3) == 0)) { \
-        uint32_t* t_ = trace_smem + (stream) * TRACE_WORDS;                                   \
-        uint32_t n_ = t_[0];                                                                  \
-        if (n_ < TRACE_EVENTS) { t_[2 + n_ * 2] = (tag); t_[3 + n_ * 2] = (uint32_t)clock64(); t_[0] = n_ + 1; } \
-    }
-
-// debug builds only: 1 = also accumulate the cycles spent in every wait (perturbs the timeline),
-// 0 = event trace only (CMBPO_TC_TRACE_ONLY=1)
-__constant__ int g_tc_count_waits = 1;
-
-template <bool DBG>
-__device__ __forceinline__ void wait_t(uint64_t* bar, uint32_t parity, unsigned long long& acc) {
-    if (DBG && g_tc_count_waits) {
-        long long t0 = clock64();
-        mbar_wait(bar, parity);
-        acc += (unsigned long long)(clock64() - t0);
-    } else {
-        mbar_wait(bar, parity);
-    }
-}
-
 // 32 accumulator columns of this thread's row -> (+bias), act -> 16-bit pairs -> 16 TMEM columns.
 // The accumulator buffer is released (`d_empty`) as soon as the values sit in registers; the
 // destination is only waited for (`dst_free`, 0 = none) right before the store.
@@ -269,15 +240,15 @@ __device__ __forceinline__ void wait_t(uint64_t* bar, uint32_t parity, unsigned 
 // accumulator already holds t = x/2 and swish(x) = t + t tanh t needs one MUFU and one FFMA.  `bias`
 // points at this warp's 32 biases in shared memory (every lane reads the same address: a broadcast
 // LDS.128 per four elements; the earlier per-element SHFL of a lane-held bias shared the MIO queue with
-// the MUFU instructions) or is null when the bias rides in the GEMM (layer 0, see `fold`).
+// the MUFU instructions) or is null when the bias rides in the GEMM (layer 0, see `fold`).  ACT == 0: the
+// activation is a per-member runtime value (merged policy ensemble), swish when `rt_swish`, else tanh.
 template <int FMT, int ACT>
 __device__ __forceinline__ void drain32(uint32_t d_addr, const float* bias, uint32_t dst_addr,
                                         uint32_t d_empty, uint32_t dst_free, uint32_t dst_parity,
-                                        uint32_t* tr = nullptr, bool rt_swish = false) {
+                                        bool rt_swish = false) {
     uint32_t r[32];
     tmem_ld32(d_addr, r);
     tmem_ld_wait();
-    if (tr) tr[0] = (uint32_t)clock64();
     tc_fence_before();
     __syncwarp();
     if ((threadIdx.x & 31) == 0) mbar_arrive_a(d_empty);
@@ -306,29 +277,10 @@ __device__ __forceinline__ void drain32(uint32_t d_addr, const float* bias, uint
     }
 #pragma unroll
     for (int c = 0; c < 16; ++c) q[c] = Cvt<FMT>::pack(v[2 * c], v[2 * c + 1]);
-    if (tr) tr[1] = (uint32_t)clock64();
     if (dst_free) { mbar_wait_a(dst_free, dst_parity); tc_fence_after(); }
     tmem_st16(dst_addr, q);
     tmem_st_wait();
     tc_fence_before();
-    if (tr) tr[2] = (uint32_t)clock64();
-}
-
-// ACT == 0: the activation is a per-member runtime value (merged policy ensemble)
-template <int FMT, int ACT>
-__device__ __forceinline__ void drain32_act(int act_rt, uint32_t d_addr, const float* bias, uint32_t dst_addr,
-                                            uint32_t d_empty, uint32_t dst_free, uint32_t dst_parity,
-                                            uint32_t* tr = nullptr) {
-#ifndef CMBPO_TWO_DRAIN_COPIES
-    if (ACT == 0) { drain32<FMT, 0>(d_addr, bias, dst_addr, d_empty, dst_free, dst_parity, nullptr, act_rt != CMBPO_ACT_TANH); return; }
-#endif
-    if (ACT != 0) {
-        drain32<FMT, ACT>(d_addr, bias, dst_addr, d_empty, dst_free, dst_parity, tr);
-    } else if (act_rt == CMBPO_ACT_TANH) {
-        drain32<FMT, CMBPO_ACT_TANH>(d_addr, bias, dst_addr, d_empty, dst_free, dst_parity);
-    } else {
-        drain32<FMT, CMBPO_ACT_SWISH>(d_addr, bias, dst_addr, d_empty, dst_free, dst_parity);
-    }
 }
 
 // G > 1: GROUPED mode for narrow members (width HD/G): G members form one unit whose layer 0 is one
@@ -349,11 +301,11 @@ __device__ __forceinline__ void drain32_act(int act_rt, uint32_t d_addr, const f
 // x 64 B/clk is more than the L2 slices deliver (~6300 B/clk chip-wide = 42 B/clk per SM, B300_MICROARCH.md):
 // the phase ran at ~47 cycles per MMA.  Everything else (MMAs, tensor memory, epilogue) stays per CTA (cta_group::1);
 // only a ring slot's release is a pair-wide event (both issuers commit to both CTAs' W_EMPTY barriers).
-template <int HD, int FMT, int ACT, bool DBG, int G, bool FUSE, int NMID = 0, int CL = 1>
+template <int HD, int FMT, int ACT, int G, bool FUSE, int NMID = 0, int CL = 1>
 __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams p) {
-    static_assert(CL == 1 || (CL == 2 && G == 1 && !FUSE && !DBG), "cluster pairs: ordinary ensembles only");
-    static_assert(!FUSE || (G == 1 && !DBG), "the fused step kernel exists for ordinary (ungrouped) ensembles");
-    static_assert(NMID == 0 || (HD <= 256 && G == 1 && !FUSE && !DBG), "deep variant: width <= 256, ungrouped");
+    static_assert(CL == 1 || (CL == 2 && G == 1 && !FUSE), "cluster pairs: ordinary ensembles only");
+    static_assert(!FUSE || G == 1, "the fused step kernel exists for ordinary (ungrouped) ensembles");
+    static_assert(NMID == 0 || (HD <= 256 && G == 1 && !FUSE), "deep variant: width <= 256, ungrouped");
     constexpr int W2S = FUSE ? W2SLOT_F : W2SLOT;          // layer-2 ring slot bytes
     constexpr int NC = HD / 64;                     // 64-column chunks of a hidden layer
     constexpr int KP = HD / 64 / G;                 // 64-wide K panels of layer 1 (per member)
@@ -373,8 +325,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     constexpr int BAR_OFF = FUSE ? SMEM_BAR_F : SMEM_BAR;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + BAR_OFF);
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + BAR_OFF + NBAR * 8);
-    uint32_t* trace_smem = reinterpret_cast<uint32_t*>(smem + BAR_OFF + NBAR * 8 + 16);   // DBG only (1960 B)
-    if (DBG && threadIdx.x < TRACE_STREAMS) trace_smem[threadIdx.x * TRACE_WORDS] = 0;
 
     // Warp roles: 0 = main weight producer, 1 = layer-0/1 MMA issuer, 2 = TMEM allocator + layer-2 MMA
     // issuer, 3 = W2 producer, 4-19 = epilogue (four warpgroups).  A warp may only touch the TMEM lane
@@ -436,26 +386,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     if (warp == 0) {
         // ===== main weight producer: layer-0 and layer-1 tiles, 32 KB per stage =====
         uint32_t s = 0, ph = 0;
-        unsigned long long c_wempty = 0;
-        const long long t_begin = DBG ? clock64() : 0;
         for (int u = u0; u < u1; ++u) {
             {
                 const int e = (int)(u % n_groups);
                 const uint8_t* src = p.wmain + (unsigned long long)e * p.main_bytes;
                 auto push = [&](uint32_t bytes) {
-                    wait_t<DBG>(bar + W_EMPTY + s, ph ^ 1, c_wempty);
+                    mbar_wait(bar + W_EMPTY + s, ph ^ 1);
                     if (elect_one()) {
-#ifdef CMBPO_EXP_HALF_W   // timing experiment only (wrong results): half the L2 -> shared-memory bytes
-                        mbar_expect_tx(bar + W_FULL + s, bytes / 2);
-                        bulk_g2s(sW + s * STAGE, src, bytes / 2, bar + W_FULL + s);
-#else
                         mbar_expect_tx(bar + W_FULL + s, bytes);
                         if (CL == 2)      // my half of the stage, into both CTAs' rings; the peer sends the other half
                             bulk_g2s_mc(sW + s * STAGE + cta_rank * (bytes / 2), src + cta_rank * (bytes / 2), bytes / 2,
                                         bar + W_FULL + s, (uint16_t)3);
                         else
                             bulk_g2s(sW + s * STAGE, src, bytes, bar + W_FULL + s);
-#endif
                     }
                     __syncwarp();
                     src += bytes;
@@ -467,19 +410,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                         for (int kq = 0; kq < KP / TPS; ++kq) push(TPS * TILE);
             }
         }
-        if (DBG && p.dbg && lane == 0) {
-            p.dbg[blockIdx.x * 16 + 0] = (unsigned long long)(clock64() - t_begin);
-            p.dbg[blockIdx.x * 16 + 1] = c_wempty;
-        }
     } else if (warp == 3) {
         // ===== layer-2 weight producer: the W2 tiles of `cps` consecutive chunks per slot =====
         uint32_t s2 = 0, ph2 = 0, mb = 0;
-        unsigned long long dummy = 0;
         for (int u = u0; u < u1; ++u, ++mb) {
             {
                 const int e = (int)(u % n_groups);
                 {   // hidden-layer biases [b0 | b1] of this unit -> bias buffer (mb & 1)
-                    wait_t<false>(bar + B_EMPTY + (mb & 1), ((mb >> 1) & 1) ^ 1, dummy);
+                    mbar_wait(bar + B_EMPTY + (mb & 1), ((mb >> 1) & 1) ^ 1);
                     if (elect_one()) {
                         mbar_expect_tx(bar + B_FULL + (mb & 1), (1 + NHID) * HD * 4);
                         bulk_g2s(sBias + (mb & 1) * (BIAS_SLOT / 4), p.bias + (long long)e * p.bias_stride, (1 + NHID) * HD * 4,
@@ -491,7 +429,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 for (int j0 = 0; j0 < NC; j0 += p.cps) {
                     const int nchunks = (NC - j0) < p.cps ? (NC - j0) : p.cps;
                     const uint32_t bytes = (uint32_t)nchunks * w2_chunk_bytes;
-                    wait_t<false>(bar + W2_EMPTY + s2, ph2 ^ 1, dummy);
+                    mbar_wait(bar + W2_EMPTY + s2, ph2 ^ 1);
                     if (elect_one()) {
                         mbar_expect_tx(bar + W2_FULL + s2, bytes);
                         bulk_g2s(sW2 + s2 * W2S, src, bytes, bar + W2_FULL + s2);
@@ -510,16 +448,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         const uint32_t idesc_o = idesc_f16(FMT, NPp);
         const uint64_t dW2 = smem_desc_sw128(smem_u32(sW2));
         uint32_t s2 = 0, ph2 = 0, c1 = 0, m = 0;
-        unsigned long long c_w2 = 0, c_h2 = 0, c_out = 0;
         for (int u = u0; u < u1; ++u) {
             int jin = 0;
             for (int jj = 0; jj < NC; ++jj) {
                 // barrier pair = chunk parity (one per epilogue pair), also when H2 is single buffered:
                 // every waiter then sees consecutive phases of "its" barrier and the parity test is exact
                 const uint32_t hbar = c1 & 1, hn = c1 >> 1, hb = (nh2 == 2) ? hbar : 0;
-                if (jin == 0) wait_t<DBG>(bar + W2_FULL + s2, ph2, c_w2);
-                if (jj == 0) wait_t<DBG>(bar + OUT_EMPTY, (m & 1) ^ 1, c_out);
-                wait_t<DBG>(bar + H2_FULL + hbar, hn & 1, c_h2);
+                if (jin == 0) mbar_wait(bar + W2_FULL + s2, ph2);
+                if (jj == 0) mbar_wait(bar + OUT_EMPTY, (m & 1) ^ 1);
+                mbar_wait(bar + H2_FULL + hbar, hn & 1);
                 tc_fence_after();
                 const bool last_in_slot = (jin == p.cps - 1) || (jj == NC - 1);
                 if (elect_one()) {
@@ -540,10 +477,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             }
             ++m;
         }
-        if (DBG && p.dbg && lane == 0) {
-            unsigned long long* d = p.dbg + blockIdx.x * 16;
-            d[6] = c_h2; d[7] = c_out; d[11] = c_w2;
-        }
     } else if (warp == 1) {
         // ===== layer-0/1 MMA issuer.  Wide members (G == 1): ONE elected thread runs the whole loop, waits
         // included, so that no warp-level election / reconvergence sits between two batches of MMAs
@@ -557,52 +490,37 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         const uint64_t dXA = smem_desc_sw128(smem_u32(sXA));
         const uint64_t dW0 = smem_desc_sw128(smem_u32(sW));
         uint32_t s = 0, ph = 0, g = 0, m = 0, it = 0;
-        unsigned long long c_w = 0, c_d = 0, c_h1 = 0, c_x = 0;
-        const long long t_begin = DBG ? clock64() : 0;
         auto next_stage = [&]() { if (++s == NSM) { s = 0; ph ^= 1; } };
-#ifndef CMBPO_NO_SPLIT_ISSUE
         // SPLIT (single-thread issuer, 4-tile stages): the issuing thread's bookkeeping between two batches of MMAs
         // (a try_wait costs ~60 cycles even when the phase completed long ago) is not covered by queued MMAs -- the
         // layer-1 phase ran at ~44 cycles per MMA with all-zero operands too, i.e. not a power or data effect.  So
         // every wait is issued in the MIDDLE of a batch (after its first 8 MMAs): the W_FULL wait of the NEXT stage
         // and the hoisted accumulator hand-off; at a batch boundary only the commits remain.
         constexpr bool SPLIT = SINGLE && TPS == 4;
-#else
-        constexpr bool SPLIT = false;
-#endif
         // stages this CTA consumes in total (the W_FULL wait runs one stage ahead only while a next stage exists)
         const uint32_t total_stages = (uint32_t)(u1 - u0) * (uint32_t)(NC / G0 + NHID * NC * (KP / TPS));
         uint32_t q_stage = 0;
         uint32_t pre_n = 0;                 // upcoming ring stages whose W_FULL phase was already seen complete
-        // C8 (512-wide ordinary members): a whole layer-1 chunk (2 stages, 32 MMAs) per asm statement with the next
-        // chunk's barrier tests embedded (mma_f16_ts_chunk8, tc_common.cuh)
-        // (measured 10 % SLOWER than two half-stage batches per stage -- 0.436 vs 0.394 ms -- and kept for reference only)
-#ifdef CMBPO_C8
-        constexpr bool C8 = SPLIT && !DBG && (KP / TPS == 2);
-#else
-        constexpr bool C8 = false;
-#endif
-        const uint32_t bar_a1 = smem_u32(bar);
         if (!SINGLE || elect_one()) {
         int cur_tile = -1;
         for (int u = u0; u < u1; ++u) {
             const int tile = CMBPO_TILE_OF(u);
             if (tile != cur_tile) {                 // a new row tile: its XA panel must have landed
                 cur_tile = tile;
-                wait_t<DBG>(bar + X_FULL, it & 1, c_x);
+                mbar_wait(bar + X_FULL, it & 1);
                 tc_fence_after();
                 ++it;
             }
             {
                 for (int j0 = 0; j0 < NC; j0 += G0) {       // layer 0: D = XA x W0 chunk (G0 chunks per stage)
-                    if (pre_n) --pre_n; else wait_t<DBG>(bar + W_FULL + s, ph, c_w);
+                    if (pre_n) --pre_n; else mbar_wait(bar + W_FULL + s, ph);
                     ++q_stage;
 #pragma unroll
                     for (int jj = 0; jj < G0; ++jj) {
                         // one chunk per instruction, buffer = chunk parity: the two epilogue pairs run as
                         // independent streams (one computes while the other is in its hand-off)
                         const uint32_t buf = g & 1, n = g >> 1;
-                        wait_t<DBG>(bar + D_EMPTY + buf, (n & 1) ^ 1, c_d);
+                        mbar_wait(bar + D_EMPTY + buf, (n & 1) ^ 1);
                         tc_fence_after();
                         if (SINGLE || elect_one()) {
                             const uint64_t dB = dW0 + (uint64_t)((s * STAGE + jj * TILE) >> 4);
@@ -612,74 +530,42 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                             if (jj == G0 - 1) { if (CL == 2) mma_commit_mc(bar + W_EMPTY + s, 3); else mma_commit(bar + W_EMPTY + s); }
                         }
                         if (!SINGLE) __syncwarp();
-                        TRACE(0, 100 + j0 + jj);
                         g += 1;
                     }
                     next_stage();
                 }
                 for (int lyr = 0; lyr < NHID; ++lyr) {      // the HD x HD layers: middle ones (deep nets), then the last hidden
                 const uint32_t col_a = (NMID > 0 && (lyr & 1)) ? COL_HB : COL_H1;     // A operand: the buffer the layer before wrote
-                wait_t<DBG>(bar + H1_FULL, (m * NHID + lyr) & 1, c_h1);
+                mbar_wait(bar + H1_FULL, (m * NHID + lyr) & 1);
                 tc_fence_after();
-                TRACE(0, 200);
                 // layer 1.  The accumulator hand-off of chunk j+1 is waited for BEFORE the last stage of chunk j
                 // is issued: the issue of that stage is back-pressured by the tensor pipe anyway, so the latency
                 // of the (normally long satisfied) wait hides behind queued MMAs instead of opening a gap
                 // between two chunks.
                 {
                     const uint32_t buf0 = g & 1, n0 = g >> 1;
-                    wait_t<DBG>(bar + D_EMPTY + buf0, (n0 & 1) ^ 1, c_d);
+                    mbar_wait(bar + D_EMPTY + buf0, (n0 & 1) ^ 1);
                     tc_fence_after();
                 }
                 constexpr bool HOIST = (KP / TPS > 1);      // single-stage chunks (narrow members): wait per chunk
                 for (int j = 0; j < NC; ++j) {
                     const uint32_t buf = g & 1;
                     if (!HOIST && j > 0) {
-                        wait_t<DBG>(bar + D_EMPTY + buf, ((g >> 1) & 1) ^ 1, c_d);
+                        mbar_wait(bar + D_EMPTY + buf, ((g >> 1) & 1) ^ 1);
                         tc_fence_after();
                     }
-                    TRACE(0, 300 + j);
-                    if (C8) {
-                        const uint32_t s0 = s, ph0 = ph;
-                        next_stage();
-                        const uint32_t s1 = s, ph1 = ph;
-                        next_stage();                                   // (s, ph): the first stage after this chunk
-                        if (pre_n) --pre_n; else mbar_wait_a(bar_a1 + 8 * (W_FULL + s0), ph0);
-                        if (pre_n) --pre_n; else mbar_wait_a(bar_a1 + 8 * (W_FULL + s1), ph1);
-                        q_stage += 2;
-                        const uint32_t ns1 = (s + 1 == NSM) ? 0u : s + 1, nph1 = (s + 1 == NSM) ? (ph ^ 1u) : ph;
-                        const uint32_t g1 = g + 1;
-                        const uint32_t flags = (q_stage < total_stages ? 1u : 0u) | (q_stage + 1 < total_stages ? 2u : 0u) |
-                                               (j + 1 < NC ? 4u : 0u);
-                        const uint32_t w0a = bar_a1 + 8 * (W_FULL + s), w1a = bar_a1 + 8 * (W_FULL + ns1);
-                        const uint32_t dea = bar_a1 + 8 * (D_EMPTY + (g1 & 1)), dep = ((g1 >> 1) & 1) ^ 1;
-                        const uint32_t ok = mma_f16_ts_chunk8<CL == 2>(tmem + COL_D + buf * 64, tmem_rt + col_a,
-                                                              dW0 + (uint64_t)((s0 * STAGE) >> 4), dW0 + (uint64_t)((s1 * STAGE) >> 4),
-                                                              idesc_h, 0u, w0a, ph, w1a, nph1, dea, dep, flags,
-                                                              bar_a1 + 8 * (W_EMPTY + s0));
-                        if (!ok) {                                      // rare: something the next chunk needs is not there yet
-                            if (flags & 1u) mbar_wait_a(w0a, ph);
-                            if (flags & 2u) mbar_wait_a(w1a, nph1);
-                            if (flags & 4u) mbar_wait_a(dea, dep);
-                        }
-                        if (flags & 4u) tc_fence_after();
-                        pre_n = (flags & 1u) + ((flags >> 1) & 1u);
-                        if (CL == 2) mma_commit_mc_a(bar_a1 + 8 * (W_EMPTY + s1), 3);      // (the first stage was released inside)
-                        else mma_commit_a(bar_a1 + 8 * (W_EMPTY + s1));
-                        mma_commit_a(bar_a1 + 8 * (D_FULL + buf));
-                    } else
                     for (int kq = 0; kq < KP / TPS; ++kq) {
-                        if (pre_n) --pre_n; else wait_t<DBG>(bar + W_FULL + s, ph, c_w);      // TMA completion: no tcgen05 fence needed
+                        if (pre_n) --pre_n; else mbar_wait(bar + W_FULL + s, ph);      // TMA completion: no tcgen05 fence needed
                         ++q_stage;
                         auto mid_waits = [&]() {
                             if (SPLIT && q_stage < total_stages) {       // the NEXT stage's weights
                                 const uint32_t ns = (s + 1 == NSM) ? 0u : s + 1, nph = (s + 1 == NSM) ? (ph ^ 1u) : ph;
-                                wait_t<DBG>(bar + W_FULL + ns, nph, c_w);
+                                mbar_wait(bar + W_FULL + ns, nph);
                                 pre_n = 1;
                             }
                             if (HOIST && kq == KP / TPS - 1 && j + 1 < NC) {
                                 const uint32_t g1 = g + 1;
-                                wait_t<DBG>(bar + D_EMPTY + (g1 & 1), ((g1 >> 1) & 1) ^ 1, c_d);
+                                mbar_wait(bar + D_EMPTY + (g1 & 1), ((g1 >> 1) & 1) ^ 1);
                                 tc_fence_after();
                             }
                         };
@@ -689,17 +575,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                             if (SPLIT) {
                                 const uint32_t a0 = tmem_rt + col_a + ((j / CPM) * KP + kq * TPS) * 32;
                                 const uint64_t b0 = dW0 + (uint64_t)((s * STAGE) >> 4);
-#ifdef CMBPO_SPLIT4
-                                mma_f16_ts_tiles<1>(tmem + COL_D + buf * 64, a0, b0, idesc_h, kq > 0);
-                                mid_waits();
-                                mma_f16_ts_tiles<1>(tmem + COL_D + buf * 64, a0 + 32, b0 + (uint64_t)((1 * TILE) >> 4), idesc_h, 1u);
-                                mma_f16_ts_tiles<1>(tmem + COL_D + buf * 64, a0 + 64, b0 + (uint64_t)((2 * TILE) >> 4), idesc_h, 1u);
-                                mma_f16_ts_tiles<1>(tmem + COL_D + buf * 64, a0 + 96, b0 + (uint64_t)((3 * TILE) >> 4), idesc_h, 1u);
-#else
                                 mma_f16_ts_tiles<2>(tmem + COL_D + buf * 64, a0, b0, idesc_h, kq > 0);
                                 mid_waits();
                                 mma_f16_ts_tiles<2>(tmem + COL_D + buf * 64, a0 + 64, b0 + (uint64_t)((2 * TILE) >> 4), idesc_h, 1u);
-#endif
                             } else
                             mma_f16_ts_tiles<TPS>(tmem + COL_D + buf * 64, tmem_rt + col_a + ((j / CPM) * KP + kq * TPS) * 32,
                                                   dW0 + (uint64_t)((s * STAGE) >> 4), idesc_h, kq > 0);
@@ -710,7 +588,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                         next_stage();
                     }
                     ++g;
-                    TRACE(0, 400 + j);
                 }
                 }   // hidden-layer loop
                 ++m;
@@ -718,11 +595,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         }
         }
         __syncwarp();
-        if (DBG && p.dbg && lane == 0) {
-            unsigned long long* d = p.dbg + blockIdx.x * 16;
-            d[2] = (unsigned long long)(clock64() - t_begin);
-            d[3] = c_w; d[4] = c_d; d[5] = c_h1; d[8] = c_x;
-        }
     }
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
@@ -734,9 +606,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         const uint32_t lane_base = (uint32_t)(wq * 32) << 16;
         const uint32_t bar_a = smem_u32(bar);
         uint32_t g = 0, m = 0, c1 = 0;
-        unsigned long long c_dfull = 0, c_drain = 0, c_outw = 0;
-        uint32_t dtr[3] = {0, 0, 0};
-        const long long t_begin = DBG ? clock64() : 0;
         // deferred OUT epilogue: the four warpgroups split the NP output columns (16 or 32 each)
         int prev_e = 0; long long prev_grow = 0; uint32_t prev_m = 0; bool have_prev = false;
         int prev_tile = 0;
@@ -760,7 +629,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         }
         const int out_cw = (G > 1) ? p.NP : ((p.NP <= 64) ? 16 : 32);
         auto out_epilogue = [&]() {
-            wait_t<DBG>(bar + OUT_FULL, prev_m & 1, c_outw);
+            mbar_wait(bar + OUT_FULL, prev_m & 1);
             tc_fence_after();
             const int c_begin = wg * out_cw;
             uint32_t r[32];
@@ -912,22 +781,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 for (int i = 0; i < NC / 2; ++i) {               // layer-0 chunk j -> H1 columns
                     const int j = 2 * i + (int)pair;
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1;
-                    wait_t<DBG>(bar + D_FULL + buf, n & 1, c_dfull);
+                    mbar_wait(bar + D_FULL + buf, n & 1);
                     tc_fence_after();
-                    TRACE(1 + wg, 1000 + j);
-                    const long long td = (DBG && g_tc_count_waits) ? clock64() : 0;
-                    drain32_act<FMT, ACT>((ACT == 0) ? p.member_act[e * G + j / CPM] : ACT, tmem + COL_D + buf * 64 + half * 32 + lane_base,
-                                      p.fold ? nullptr : sb + j * 64 + half * 32,
+                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, p.fold ? nullptr : sb + j * 64 + half * 32,
                                       tmem + COL_H1 + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u,
-                                      DBG ? dtr : nullptr);
-                    if (DBG && m == 8 && lane == 0 && (warp & 3) == 0 && p.dbg && blockIdx.x == 0) {
-                        uint32_t* t_ = trace_smem + (1 + wg) * TRACE_WORDS; uint32_t n_ = t_[0];
-                        if (n_ + 3 <= TRACE_EVENTS) { for (int q_ = 0; q_ < 3; ++q_) { t_[2 + (n_ + q_) * 2] = 1200 + q_; t_[3 + (n_ + q_) * 2] = dtr[q_]; } t_[0] = n_ + 3; }
-                    }
-                    if (DBG && g_tc_count_waits) c_drain += (unsigned long long)(clock64() - td);
+                                      ACT == 0 && p.member_act[e * G + j / CPM] != CMBPO_ACT_TANH);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * H1_FULL);
-                    TRACE(1 + wg, 1100 + j);
                 }
                 g += NC;
                 // The previous member's OUT accumulator is drained HERE, after this member's layer-0
@@ -940,10 +800,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                         for (int i = 0; i < NC / 2; ++i) {
                             const int j = 2 * i + (int)pair;
                             const uint32_t gg = g + j, buf = pair, n = gg >> 1;
-                            wait_t<DBG>(bar + D_FULL + buf, n & 1, c_dfull);
+                            mbar_wait(bar + D_FULL + buf, n & 1);
                             tc_fence_after();
-                            drain32_act<FMT, ACT>(ACT, tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + lyr * HD + j * 64 + half * 32,
-                                                  tmem + col_dst + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u, nullptr);
+                            drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + lyr * HD + j * 64 + half * 32,
+                                              tmem + col_dst + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u);
                             __syncwarp();
                             if (lane == 0) mbar_arrive_a(bar_a + 8 * H1_FULL);
                         }
@@ -962,22 +822,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     const uint32_t hbar = cc & 1, hn = cc >> 1, hb = (nh2 == 2) ? hbar : 0;
                     const uint32_t h2_free = (nh2 == 2) ? bar_a + 8 * (H2_EMPTY + hbar) : (cc == 0 ? 0u : bar_a + 8 * (H2_EMPTY + (hbar ^ 1)));
                     const uint32_t h2_par = (nh2 == 2) ? ((hn & 1) ^ 1) : ((((cc - 1) >> 1)) & 1);
-                    wait_t<DBG>(bar + D_FULL + buf, n & 1, c_dfull);
+                    mbar_wait(bar + D_FULL + buf, n & 1);
                     tc_fence_after();
-                    TRACE(1 + wg, 2000 + j);
-                    const long long td = (DBG && g_tc_count_waits) ? clock64() : 0;
-                    drain32_act<FMT, ACT>((ACT == 0) ? p.member_act[e * G + j / CPM] : ACT, tmem + COL_D + buf * 64 + half * 32 + lane_base,
-                                      sb + NHID * HD + j * 64 + half * 32,
+                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + NHID * HD + j * 64 + half * 32,
                                       tmem + COL_H2 + hb * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf),
-                                      h2_free, h2_par, DBG ? dtr : nullptr);
-                    if (DBG && m == 8 && lane == 0 && (warp & 3) == 0 && p.dbg && blockIdx.x == 0) {
-                        uint32_t* t_ = trace_smem + (1 + wg) * TRACE_WORDS; uint32_t n_ = t_[0];
-                        if (n_ + 3 <= TRACE_EVENTS) { for (int q_ = 0; q_ < 3; ++q_) { t_[2 + (n_ + q_) * 2] = 2200 + q_; t_[3 + (n_ + q_) * 2] = dtr[q_]; } t_[0] = n_ + 3; }
-                    }
-                    if (DBG && g_tc_count_waits) c_drain += (unsigned long long)(clock64() - td);
+                                      h2_free, h2_par, ACT == 0 && p.member_act[e * G + j / CPM] != CMBPO_ACT_TANH);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * (H2_FULL + hbar));
-                    TRACE(1 + wg, 2100 + j);
                 }
                 __syncwarp();
                 if (lane == 0) mbar_arrive_a(bar_a + 8 * (B_EMPTY + (m & 1)));     // the bias buffer may be refilled
@@ -987,18 +838,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             }
         }
         if (have_prev) out_epilogue();
-        if (DBG && p.dbg && warp == 4 && lane == 0) {
-            unsigned long long* d = p.dbg + blockIdx.x * 16;
-            d[9] = (unsigned long long)(clock64() - t_begin);
-            d[10] = c_dfull; d[12] = c_drain; d[13] = c_outw;
-        }
     }
     tc_fence_before();
     __syncthreads();
     if (CL == 2) cluster_sync_all();      // the peer may still be signalling this CTA's barriers
 #undef CMBPO_TILE_OF
-    if (DBG && p.dbg && blockIdx.x == 0)
-        for (int i = threadIdx.x; i < TRACE_STREAMS * TRACE_WORDS; i += NTHREADS) p.dbg[4096 + i] = trace_smem[i];
     if (warp == 2) tmem_dealloc(tmem, 512);
 }
 
@@ -1117,11 +961,11 @@ int chunks_per_w2_slot(int HD, int NP, int slot_bytes = W2SLOT) {
     return p2 < NC ? p2 : NC;
 }
 
-template <int HD, int FMT, int ACT, bool DBG, int G = 1, bool FUSE = false, int NMID = 0>
+template <int HD, int FMT, int ACT, int G = 1, bool FUSE = false, int NMID = 0>
 int launch_tc(cmbpo_ctx* ctx, const TcParams& p) {
-    const int smem = (FUSE ? SMEM_TOTAL_F : SMEM_TOTAL) + 1024 + (DBG ? 1968 : 0);
-    static_assert(SMEM_TOTAL + 1024 + 1968 <= 232448, "shared memory budget");
-    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, DBG, G, FUSE, NMID>;
+    const int smem = (FUSE ? SMEM_TOTAL_F : SMEM_TOTAL) + 1024;
+    static_assert(SMEM_TOTAL + 1024 <= 232448, "shared memory budget");
+    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, G, FUSE, NMID>;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const long long units = (long long)p.ntiles * ((p.E + G - 1) / G);
     const int grid = units < ctx->sm_count ? (int)units : ctx->sm_count;
@@ -1136,7 +980,7 @@ int launch_tc(cmbpo_ctx* ctx, const TcParams& p) {
 template <int HD, int FMT, int ACT>
 int launch_tc_pairs(cmbpo_ctx* ctx, const TcParams& p) {
     const int smem = SMEM_TOTAL + 1024;
-    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, false, 1, false, 0, 2>;
+    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, 1, false, 0, 2>;
     static int max_pairs = -1;
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
@@ -1156,7 +1000,7 @@ int launch_tc_pairs(cmbpo_ctx* ctx, const TcParams& p) {
         // pairs are worth ~2 %; a part whose GPC layout leaves more than two SMs without a partner loses more than that
         if (2 * max_pairs < ctx->sm_count - 2) max_pairs = 0;
     }
-    if (max_pairs == 0) return launch_tc<HD, FMT, ACT, false>(ctx, p);
+    if (max_pairs == 0) return launch_tc<HD, FMT, ACT>(ctx, p);
     const long long units = (long long)((p.ntiles + 1) / 2) * p.E;
     const int pairs = units < max_pairs ? (int)units : max_pairs;
     cfg.gridDim = dim3(2 * pairs);
@@ -1169,47 +1013,45 @@ int launch_tc_pairs(cmbpo_ctx* ctx, const TcParams& p) {
 // the fused rollout step: swish dynamics ensembles of any supported width
 template <int FMT>
 int launch_tc_fused(cmbpo_ctx* ctx, const TcParams& p, int hd) {
-    if (hd == 128) return launch_tc<128, FMT, CMBPO_ACT_SWISH, false, 1, true>(ctx, p);
-    if (hd == 256) return launch_tc<256, FMT, CMBPO_ACT_SWISH, false, 1, true>(ctx, p);
-    return launch_tc<512, FMT, CMBPO_ACT_SWISH, false, 1, true>(ctx, p);
+    if (hd == 128) return launch_tc<128, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
+    if (hd == 256) return launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
+    return launch_tc<512, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
 }
 
 template <int HD, int FMT>
 int launch_tc_act(cmbpo_ctx* ctx, const TcParams& p, int act) {
-    if (act == 0) return launch_tc<HD, FMT, 0, false>(ctx, p);
-    if (act == CMBPO_ACT_SWISH) return launch_tc<HD, FMT, CMBPO_ACT_SWISH, false>(ctx, p);
-    return launch_tc<HD, FMT, CMBPO_ACT_TANH, false>(ctx, p);
+    if (act == 0) return launch_tc<HD, FMT, 0>(ctx, p);
+    if (act == CMBPO_ACT_SWISH) return launch_tc<HD, FMT, CMBPO_ACT_SWISH>(ctx, p);
+    return launch_tc<HD, FMT, CMBPO_ACT_TANH>(ctx, p);
 }
 
 // 3 / 4 hidden layers at (padded) width 256
 template <int FMT>
 int launch_tc_deep(cmbpo_ctx* ctx, const TcParams& p, int act, int nmid) {
     if (act == CMBPO_ACT_SWISH)
-        return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_SWISH, false, 1, false, 1>(ctx, p)
-                         : launch_tc<256, FMT, CMBPO_ACT_SWISH, false, 1, false, 2>(ctx, p);
-    return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_TANH, false, 1, false, 1>(ctx, p)
-                     : launch_tc<256, FMT, CMBPO_ACT_TANH, false, 1, false, 2>(ctx, p);
+        return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, false, 1>(ctx, p)
+                         : launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, false, 2>(ctx, p);
+    return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_TANH, 1, false, 1>(ctx, p)
+                     : launch_tc<256, FMT, CMBPO_ACT_TANH, 1, false, 2>(ctx, p);
 }
 
 template <int FMT>
 int launch_tc_grouped(cmbpo_ctx* ctx, const TcParams& p, int act) {       // 4 members of width 128 per unit
-    if (act == 0) return launch_tc<512, FMT, 0, false, 4>(ctx, p);
-    if (act == CMBPO_ACT_SWISH) return launch_tc<512, FMT, CMBPO_ACT_SWISH, false, 4>(ctx, p);
-    return launch_tc<512, FMT, CMBPO_ACT_TANH, false, 4>(ctx, p);
+    if (act == 0) return launch_tc<512, FMT, 0, 4>(ctx, p);
+    if (act == CMBPO_ACT_SWISH) return launch_tc<512, FMT, CMBPO_ACT_SWISH, 4>(ctx, p);
+    return launch_tc<512, FMT, CMBPO_ACT_TANH, 4>(ctx, p);
 }
 
 template <int FMT>
 int launch_tc_hd(cmbpo_ctx* ctx, const TcParams& p, int hd, int act) {
     if (hd == 128) return launch_tc_act<128, FMT>(ctx, p, act);
     if (hd == 256) return launch_tc_act<256, FMT>(ctx, p, act);
-#ifndef CMBPO_NO_PAIRS
     if (p.ntiles >= 2) {
         if (act == CMBPO_ACT_SWISH) return launch_tc_pairs<512, FMT, CMBPO_ACT_SWISH>(ctx, p);
         return launch_tc_pairs<512, FMT, CMBPO_ACT_TANH>(ctx, p);
     }
-#endif
-    if (act == CMBPO_ACT_SWISH) return launch_tc<512, FMT, CMBPO_ACT_SWISH, false>(ctx, p);
-    return launch_tc<512, FMT, CMBPO_ACT_TANH, false>(ctx, p);
+    if (act == CMBPO_ACT_SWISH) return launch_tc<512, FMT, CMBPO_ACT_SWISH>(ctx, p);
+    return launch_tc<512, FMT, CMBPO_ACT_TANH>(ctx, p);
 }
 
 }  // namespace
@@ -1294,9 +1136,6 @@ int ens_tc_fused_rp_shift(int O) {
 
 int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* out_raw, int precision,
                    const int64_t* n_dev, const FusedStep* fz) {
-    CMBPO_CHECK(precision == CMBPO_PREC_FP16 || precision == CMBPO_PREC_BF16,
-                "precision %d: the packed 16-bit activation modes (*_X2) were removed -- the MUFU rate is per "
-                "element, so they gained nothing, and their code path slowed the default kernels by 4 %%", precision);
     CMBPO_CHECK(precision == CMBPO_PREC_BF16 || precision == CMBPO_PREC_FP16, "bad precision %d", precision);
     CMBPO_CHECK(net.tc_pack[precision], "tcgen05 weights not packed");
     if (N <= 0) return 0;
@@ -1312,7 +1151,7 @@ int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* o
     p.main_bytes = net.tc_pack_bytes[precision];
     p.w2 = p.wmain + (size_t)((net.E + net.tc_group - 1) / net.tc_group) * p.main_bytes;
     p.w2_bytes = (unsigned long long)(HD * net.tc_group / 64) * p.NP * 128;
-    const int group = net.tc_group, n_units = (net.E + group - 1) / group;
+    const int group = net.tc_group;
     p.bias = net.tc_bias; p.bias_stride = group * ((net.n_layers - 1) * HD + p.NP);
     p.E = net.E; p.K0 = net.dims[0]; p.fold = net.tc_fold; p.KS0 = (p.K0 + (p.fold ? 2 : 0) + 15) / 16;
     p.x = x; p.N = N; p.ldx = net.dims[0];
@@ -1320,7 +1159,6 @@ int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* o
     p.mu_in = net.has_in ? net.mu_in : nullptr; p.sig_in = net.sig_in;
     p.out = out_raw; p.out_member_stride = (long long)N * p.Nout;
     p.ntiles = (int)((N + 127) / 128);
-    p.dbg = nullptr;
     for (int i = 0; i < CMBPO_MAX_E; ++i) p.member_act[i] = net.member_act[i];
     if (fz) {
         CMBPO_CHECK(ens_tc_fusable(net) && fz->rp_shift >= 5, "this ensemble cannot run the fused rollout step");
@@ -1329,50 +1167,6 @@ int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* o
     }
     memset(&p.fz, 0, sizeof(p.fz));
     const int act_sel = net.member_act[0] >= 0 ? 0 : net.acts[0];
-    // protocol tracing is switched on per context by cmbpo_ctx_set_debug (tools/tcdbg.py); never by the environment
-    const bool dbg_big = ctx->tc_debug == 1 && HD == 512 && group == 1 && net.acts[0] == CMBPO_ACT_SWISH;
-    const bool dbg_grp = ctx->tc_debug == 2 && group == 4 && act_sel == 0;
-    if ((dbg_big || dbg_grp) && precision == CMBPO_PREC_FP16) {
-        // protocol timing: per-CTA cycle counters printed once per launch (debug aid, off by default)
-        unsigned long long* d;
-        const size_t dbg_words = 4096 + 3 * 1024;
-        if (cmbpo_ws_get(ctx, 1, dbg_words * 8, (void**)&d)) return 1;
-        CUDA_TRY(cudaMemsetAsync(d, 0, dbg_words * 8, ctx->stream));
-        p.dbg = d;
-        {
-            const int count_waits = ctx->tc_trace_only ? 0 : 1;
-            CUDA_TRY(cudaMemcpyToSymbolAsync(g_tc_count_waits, &count_waits, sizeof(int), 0, cudaMemcpyHostToDevice, ctx->stream));
-        }
-        if (dbg_big ? launch_tc<512, 0, CMBPO_ACT_SWISH, true>(ctx, p) : launch_tc<512, 0, 0, true, 4>(ctx, p)) return 1;
-        std::vector<unsigned long long> h(dbg_words);
-        CUDA_TRY(cudaMemcpyAsync(h.data(), d, h.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-        const char* names[14] = {"prod_total", "prod_wait_wempty", "mma_total", "mma_wait_wfull", "mma_wait_dempty",
-                                 "mma_wait_h1", "mma_wait_h2full", "mma_wait_outempty", "mma_wait_x", "epi_total",
-                                 "epi_wait_dfull", "l2_wait_w2full", "epi_drain", "epi_wait_outfull"};
-        for (int k = 0; k < 14; ++k) {
-            double sum = 0, lo = 1e30, hi = 0; int n = 0;
-            for (int b = 0; b < ctx->sm_count && b < p.ntiles; ++b) {
-                const double v = (double)h[(size_t)b * 16 + k];
-                sum += v; lo = v < lo ? v : lo; hi = v > hi ? v : hi; ++n;
-            }
-            fprintf(stderr, "tcdbg %-18s %12.0f cycles/CTA (min %.0f, max %.0f)\n", names[k], sum / (n ? n : 1), lo, hi);
-        }
-        static int printed = 0;
-        if (!printed++) {
-            static const char* names_s[TRACE_STREAMS] = {"mma", "epi wg0", "epi wg1", "epi wg2", "epi wg3"};
-            for (int st = 0; st < TRACE_STREAMS; ++st) {
-                const unsigned long long* t = h.data() + 4096 + st * TRACE_WORDS;
-                uint32_t t0 = (uint32_t)h[4096 + 3];     // first MMA event
-                fprintf(stderr, "trace stream %d (%s):", st, names_s[st]);
-                for (unsigned long long i = 0; i < t[0] && i < TRACE_EVENTS; ++i)
-                    fprintf(stderr, " %llu@%d", t[2 + i * 2], (int)((uint32_t)t[3 + i * 2] - t0));
-                fprintf(stderr, "\n");
-            }
-        }
-        return 0;
-    }
-    (void)n_units;
     if (nmid > 0) {
         CMBPO_CHECK(HD == 256 && group == 1 && (nmid == 1 || nmid == 2) && net.member_act[0] < 0, "deep tcgen05 variant: bad shape");
         return precision == CMBPO_PREC_FP16 ? launch_tc_deep<0>(ctx, p, act_sel, nmid) : launch_tc_deep<1>(ctx, p, act_sel, nmid);

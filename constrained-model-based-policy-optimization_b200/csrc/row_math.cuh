@@ -52,26 +52,6 @@ __device__ inline float philox_normal(uint64_t seed, int64_t path, int step, int
     return (k & 1) ? z1 : z0;
 }
 
-// the first n standard normals of (path, step, stream): one Philox block and two Box-Muller pairs per
-// four values -- same values as philox_normal(k), without recomputing the block for every k
-__device__ inline void philox_normals(uint64_t seed, int64_t path, int step, int stream, int n, float* z) {
-    for (int k0 = 0; k0 < n; k0 += 4) {
-        uint32_t o[4];
-        philox4x32_10((uint32_t)path, (uint32_t)((uint64_t)path >> 32), (uint32_t)step,
-                      ((uint32_t)stream << 16) | (uint32_t)(k0 >> 2), (uint32_t)seed,
-                      (uint32_t)(seed >> 32), o);
-        float a0, a1, b0, b1;
-        box_muller(o[0], o[1], a0, a1);
-        z[k0] = a0;
-        if (k0 + 1 < n) z[k0 + 1] = a1;
-        if (k0 + 2 < n) {
-            box_muller(o[2], o[3], b0, b1);
-            z[k0 + 2] = b0;
-            if (k0 + 3 < n) z[k0 + 3] = b1;
-        }
-    }
-}
-
 // uniform elite position in [0, n_elite): what np.random.choice(elite_inds, N) draws (fake_env.py:176)
 __device__ inline int philox_elite_pos(uint64_t seed, int64_t path, int step, int n_elite) {
     uint32_t o[4];
@@ -81,33 +61,11 @@ __device__ inline int philox_elite_pos(uint64_t seed, int64_t path, int step, in
 }
 
 // ------------------------------------------------------------------------------------------
-// numpy's float32 pairwise sum for n < 128 contiguous elements (np.mean over the last axis):
+// numpy's float32 pairwise sum for n < 128 elements (np.mean over the last axis):
 // 8 running partial sums, a fixed combination tree, then the n%8 tail added sequentially.
 // ------------------------------------------------------------------------------------------
-// exact numpy order over an array already in registers / local memory
-template <int MAXN>
-__device__ inline float np_sum_f32(const float (&a)[MAXN], int n) {
-    if (n < 8) {
-        float s = 0.f;
-        for (int i = 0; i < n; ++i) s = __fadd_rn(s, a[i]);
-        return s;
-    }
-    float r[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) r[j] = a[j];
-    int i = 8;
-    for (; i < n - (n & 7); i += 8) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], a[i + j]);
-    }
-    float s = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
-                        __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
-    for (; i < n; ++i) s = __fadd_rn(s, a[i]);
-    return s;
-}
-
-// The same sum over a strided array (element i at a[i * stride]); used by the fused step kernel,
-// whose staging is [dim][row].
+// Element i at a[i * stride]: stride 1 for the row kernels' [row][dim] staging, the rows per pass
+// for the fused step kernel's [dim][row] staging.
 __device__ inline float np_sum_strided(const float* a, int n, int stride) {
     if (n < 8) {
         float s = 0.f;
@@ -191,27 +149,6 @@ __device__ __forceinline__ float actor_dim(float mu, float ls, float eps, float&
     return __fmul_rn(-0.5f, t);
 }
 
-// numpy pairwise-sum order over an array in memory (see np_sum_f32)
-__device__ inline float np_sum_ptr(const float* a, int n) {
-    if (n < 8) {
-        float s = 0.f;
-        for (int i = 0; i < n; ++i) s = __fadd_rn(s, a[i]);
-        return s;
-    }
-    float r[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) r[j] = a[j];
-    int i = 8;
-    for (; i < n - (n & 7); i += 8) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], a[i + j]);
-    }
-    float s = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
-                        __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
-    for (; i < n; ++i) s = __fadd_rn(s, a[i]);
-    return s;
-}
-
 // ------------------------------------------------------------------------------------------
 // FakeEnv.step split per (row, obs dimension) -- the unit of work of the dense row kernels.
 // env_dim: everything that only needs the E members' outputs for ONE dimension
@@ -229,8 +166,10 @@ struct EnvDimOut { float kl, epv, nx; };
 // EC > 0: ensemble size known at compile time (loops fully unrolled, no predicates); EC == 0: runtime E.
 // FAST (the tensor-core precision modes): closed-form KL and approximate divisions (2 ulp) -- the IEEE
 // division is a subroutine call per use, and the all-pairs loop is 49 x 12 instructions of code.
+// Kernels are instantiated for (EC = 7, FAST) -- the 7-member ensemble of every config in the
+// tensor-core precision modes -- and for (EC = 0, exact): runtime E, IEEE divisions, all-pairs KL.
 template <int EC, bool FAST, class Raw>
-__device__ __forceinline__ EnvDimOut env_dim_t(const EnvRowCfg& c, Raw raw, int o, int member, float obs_o, float eps) {
+__device__ __forceinline__ EnvDimOut env_dim(const EnvRowCfg& c, Raw raw, int o, int member, float obs_o, float eps) {
     constexpr int EMAX = EC > 0 ? EC : CMBPO_MAX_E;
     const int E = EC > 0 ? EC : c.E;
     float nd[EMAX], ls[EMAX], vr[EMAX], rv[EMAX];
@@ -322,15 +261,8 @@ __device__ __forceinline__ EnvDimOut env_dim_t(const EnvRowCfg& c, Raw raw, int 
     return out;
 }
 
-// Kernels are instantiated for (EC = 7, FAST) -- the 7-member ensemble of every config in the
-// tensor-core precision modes -- and for (EC = 0, exact): runtime E, IEEE divisions, all-pairs KL.
-template <int EC, bool FAST, class Raw>
-__device__ __forceinline__ EnvDimOut env_dim(const EnvRowCfg& c, Raw raw, int o, int member, float obs_o, float eps) {
-    return env_dim_t<EC, FAST>(c, raw, o, member, obs_o, eps);
-}
-
 // next state of ONE dimension from the chosen member only -- the same operations, in the same order,
-// as the `sel` / `nx` values of env_dim_t (the fused step kernel recomputes it at write-out time instead
+// as the `sel` / `nx` values of env_dim (the fused step kernel recomputes it at write-out time instead
 // of staging all of next_obs)
 template <bool FAST, class Raw>
 __device__ __forceinline__ float env_dim_nx(const EnvRowCfg& c, Raw raw, int o, int member, float obs_o, float eps) {
@@ -383,8 +315,8 @@ template <bool FAST, class Raw>
 __device__ inline EnvRowOut env_row_finish(const EnvRowCfg& c, Raw raw, int member, const float* kl,
                                            const float* epv, const float* nx, const unsigned char* fin) {
     const int O = c.O;
-    const float ks = np_sum_ptr(kl, O);
-    const float es = np_sum_ptr(epv, O);
+    const float ks = np_sum_strided(kl, O, 1);
+    const float es = np_sum_strided(epv, O, 1);
     bool all_finite = true;
     for (int o = 0; o < O; ++o) all_finite = all_finite && fin[o];
     return env_row_core<FAST>(c, raw, member, ks, es, all_finite, nx[0], O > 2 ? nx[2] : 0.f, O > 3 ? nx[3] : 0.f,

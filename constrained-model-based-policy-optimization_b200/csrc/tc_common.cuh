@@ -48,9 +48,7 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
 // few tens of cycles, and the spin loops of the ~10 waiting warps of a CTA issue as many instructions as
 // the warps doing the epilogue arithmetic -- on the same issue ports and the same MIO queues as their
 // MUFU / LDS instructions (ncu: 25 M try_wait executions per launch against 0.7 M useful waits).
-#ifndef MBAR_SUSPEND_NS
-#define MBAR_SUSPEND_NS 20000u
-#endif
+constexpr uint32_t MBAR_SUSPEND_NS = 20000;
 // Bounded spin: a protocol bug must not hang the GPU (a hung box is a lost box).  On timeout the
 // kernel traps, which surfaces as a launch failure on the host.
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
@@ -72,7 +70,7 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     }
     // No printf here: a device-side call in each of the ~20 inlined wait sites costs the kernel 10 %
     // (caller-saved registers around the call constrain the allocation of the hot loops).  The trap
-    // surfaces as a launch failure on the host; CMBPO_TC_DEBUG builds narrow it down.
+    // surfaces as a launch failure on the host.
     __trap();
 }
 
@@ -238,12 +236,7 @@ __device__ __forceinline__ float tanh_approx(float x) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-// swish(x) = x*sigmoid(x) = t + t*tanh(t), t = x/2  (one MUFU)
-__device__ __forceinline__ float swish_fast(float x) {
-    float t = 0.5f * x;
-    return fmaf(t, tanh_approx(t), t);
-}
-// same, for a pre-halved argument t = x/2
+// swish(x) = x*sigmoid(x) = t + t*tanh(t) for a pre-halved argument t = x/2  (one MUFU)
 __device__ __forceinline__ float swish_half(float t) { return fmaf(t, tanh_approx(t), t); }
 
 }  // namespace tc
@@ -311,76 +304,5 @@ __device__ __forceinline__ void mma_f16_ts_tiles(uint32_t d_tmem, uint32_t a_tme
             "}" ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate_first)
             : "memory");
     }
-}
-
-// One whole layer-1 chunk of a 512-wide member from ONE asm statement: 8 B tiles (two ring stages of 4, bases b0 / b1)
-// x 4 K-steps = 32 TS-form MMAs into one accumulator, and -- between the first tiles -- three NON-BLOCKING barrier
-// tests (mbarrier.test_wait) for what the NEXT chunk needs (its two weight stages, its accumulator buffer).  The
-// issuing thread's waits otherwise sit between two batches of MMAs, where nothing covers their latency (the MMA queue
-// is shallow: ~350 of a chunk's ~1380 cycles were such gaps); inside the statement ptxas keeps every operand in
-// uniform registers, sets them up once per chunk, and the tests' latency overlaps the MMA issue.  Returns 1 when
-// every requested test (flags bit 0, 1, 2) found its phase complete; the caller falls back to blocking waits otherwise.
-#define CMBPO_C8_STEP(P)                                                                  \
-    "tcgen05.mma.cta_group::1.kind::f16 [%1], [ta], db, %5, " P ";\n\t"                   \
-    "add.u32 ta, ta, 8;\n\tadd.u64 db, db, 2;\n\t"
-#define CMBPO_C8_TILE(P0)                                                                 \
-    CMBPO_C8_STEP(P0) CMBPO_C8_STEP("pt") CMBPO_C8_STEP("pt") CMBPO_C8_STEP("pt")         \
-    "add.u64 db, db, 504;\n\t"
-template <bool MC>      // MC: the stage release is delivered to both CTAs of a cluster pair
-__device__ __forceinline__ uint32_t mma_f16_ts_chunk8(uint32_t d_tmem, uint32_t a_tmem, uint64_t b0, uint64_t b1,
-                                                      uint32_t idesc, uint32_t accumulate_first, uint32_t w0_addr,
-                                                      uint32_t w0_par, uint32_t w1_addr, uint32_t w1_par,
-                                                      uint32_t d_addr, uint32_t d_par, uint32_t flags,
-                                                      uint32_t release0_addr) {
-    // order: tile 0 | test next stage 0 | tile 1 | test next stage 1 | tiles 2-3 | RELEASE this chunk's first stage |
-    //        tiles 4-5 | test the next chunk's accumulator (late: its previous contents are still being read out
-    //        when this chunk starts) | tiles 6-7
-    uint32_t ok;
-#define CMBPO_C8_HEAD                                                                                                \
-        "{\n\t.reg .pred p0, pt, q0, q1, q2, t0, t1, t2;\n\t.reg .b32 ta, fl;\n\t.reg .b64 db;\n\t.reg .b16 mk;\n\t"      \
-        "setp.ne.b32 p0, %6, 0;\n\tsetp.eq.b32 pt, 0, 0;\n\t"                                                       \
-        "and.b32 fl, %13, 1;\n\tsetp.ne.b32 t0, fl, 0;\n\t"                                                         \
-        "and.b32 fl, %13, 2;\n\tsetp.ne.b32 t1, fl, 0;\n\t"                                                         \
-        "and.b32 fl, %13, 4;\n\tsetp.ne.b32 t2, fl, 0;\n\t"                                                         \
-        "setp.eq.b32 q0, 0, 0;\n\tsetp.eq.b32 q1, 0, 0;\n\tsetp.eq.b32 q2, 0, 0;\n\t"                               \
-        "mov.b16 mk, 3;\n\t"                                                                                        \
-        "mov.b32 ta, %2;\n\tmov.b64 db, %3;\n\t"                                                                   \
-        CMBPO_C8_TILE("p0")                                                                                         \
-        "@t0 mbarrier.test_wait.parity.shared::cta.b64 q0, [%7], %8;\n\t"                                           \
-        CMBPO_C8_TILE("pt")                                                                                         \
-        "@t1 mbarrier.test_wait.parity.shared::cta.b64 q1, [%9], %10;\n\t"                                          \
-        CMBPO_C8_TILE("pt") CMBPO_C8_TILE("pt")
-#define CMBPO_C8_TAIL                                                                                                \
-        "mov.b64 db, %4;\n\t"                                                                                       \
-        CMBPO_C8_TILE("pt") CMBPO_C8_TILE("pt")                                                                     \
-        "@t2 mbarrier.test_wait.parity.shared::cta.b64 q2, [%11], %12;\n\t"                                         \
-        CMBPO_C8_TILE("pt") CMBPO_C8_TILE("pt")                                                                     \
-        "and.pred q0, q0, q1;\n\tand.pred q0, q0, q2;\n\tselp.u32 %0, 1, 0, q0;\n\t"                                \
-        "}"
-#define CMBPO_C8_OPERANDS                                                                                            \
-        : "=r"(ok)                                                                                                   \
-        : "r"(d_tmem), "r"(a_tmem), "l"(b0), "l"(b1), "r"(idesc), "r"(accumulate_first), "r"(w0_addr), "r"(w0_par), \
-          "r"(w1_addr), "r"(w1_par), "r"(d_addr), "r"(d_par), "r"(flags), "r"(release0_addr)                         \
-        : "memory"
-    if (MC)
-        asm volatile(CMBPO_C8_HEAD
-                     "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%14], mk;\n\t"
-                     CMBPO_C8_TAIL CMBPO_C8_OPERANDS);
-    else
-        asm volatile(CMBPO_C8_HEAD
-                     "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%14];\n\t"
-                     CMBPO_C8_TAIL CMBPO_C8_OPERANDS);
-#undef CMBPO_C8_HEAD
-#undef CMBPO_C8_TAIL
-#undef CMBPO_C8_OPERANDS
-    return ok;
-}
-__device__ __forceinline__ void mma_commit_a(uint32_t bar_addr) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_addr) : "memory");
-}
-__device__ __forceinline__ void mma_commit_mc_a(uint32_t bar_addr, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar_addr),
-                 "h"(cta_mask)
-                 : "memory");
 }
 }  // namespace tc

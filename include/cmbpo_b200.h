@@ -79,10 +79,6 @@ int64_t cmbpo_ctx_launch_count(cmbpo_ctx* ctx);
  * time and the number of bracketed launches, and optionally resets the slot.
  */
 enum { CMBPO_PROF_DYN = 0, CMBPO_PROF_GAE = 1, CMBPO_PROF_STEP = 2, CMBPO_PROF_POLICY = 3, CMBPO_PROF_SLOTS = 4 };
-/* Developer aid (tools/tcdbg.py): tc_debug 1 / 2 makes the wide / grouped tcgen05 kernel print per-CTA protocol
- * counters and an event trace to stderr (synchronises); trace_only drops the wait counters.  0 = off (default).
- * Nothing in the library reads environment variables. */
-int cmbpo_ctx_set_debug(cmbpo_ctx* ctx, int tc_debug, int trace_only);
 int cmbpo_ctx_profile(cmbpo_ctx* ctx, int enable);
 int cmbpo_ctx_profile_read(cmbpo_ctx* ctx, int slot, double* total_ms_host, int64_t* launches_host,
                            int reset);
