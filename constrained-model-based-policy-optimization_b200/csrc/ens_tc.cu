@@ -1056,7 +1056,9 @@ int launch_tc_hd(cmbpo_ctx* ctx, const TcParams& p, int hd, int act) {
 
 }  // namespace
 
-// 2 hidden layers: any equal width <= 512 (padded to 128 / 256 / 512), <= 64 inputs, <= 128 outputs.
+// 2 hidden layers: any equal width <= 512 (padded to 128 / 256 / 512), <= 64 inputs, <= 128 outputs; <= 96 outputs
+// above width 256 (tensor memory: at width 512 the OUT accumulator of a 128-column output, 512 - NP = column 384,
+// would overlap the single H2 buffer at columns 384-415).
 // 3 or 4 hidden layers (e.g. the (200,200,200,200) default of algorithms/cmbpo.py:54): equal width <= 256, <= 64 outputs
 // (tensor-memory budget of the second hidden buffer).
 bool ens_tc_supported(const Net& n) {
@@ -1064,7 +1066,7 @@ bool ens_tc_supported(const Net& n) {
     const int hd = n.dims[1], L = n.n_layers;
     for (int l = 1; l < L; ++l) if (n.dims[l] != hd) return false;
     if (hd < 1 || hd > (L == 3 ? 512 : 256)) return false;
-    if (n.dims[0] > 64 || n.dims[L] > (L == 3 ? 128 : 64)) return false;
+    if (n.dims[0] > 64 || n.dims[L] > (L == 3 ? (hd > 256 ? 96 : 128) : 64)) return false;
     for (int l = 1; l < L - 1; ++l) if (n.acts[l] != n.acts[0]) return false;
     if (n.acts[L - 1] != CMBPO_ACT_NONE) return false;
     return n.acts[0] == CMBPO_ACT_SWISH || n.acts[0] == CMBPO_ACT_TANH;

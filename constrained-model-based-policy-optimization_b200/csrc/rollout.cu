@@ -475,10 +475,11 @@ int policy_forward(cmbpo_ctx* ctx, PolicyRowsArgs a, bool with_actor, int precis
     float *raw_v, *raw_vc, *raw_mu = nullptr;
     if (cmbpo_ws_get(ctx, 3, (size_t)(v.E + vc.E) * a.N * sizeof(float), (void**)&raw_v)) return 1;
     raw_vc = raw_v + (size_t)v.E * a.N;
-    // small nets: tcgen05 path only if supported, else fp32
-    int pv = (precision != CMBPO_PREC_FP32 && ens_tc_supported(v)) ? precision : CMBPO_PREC_FP32;
+    // small nets: tcgen05 path only if supported, else fp32 (decided per net: V and VC may differ in shape)
+    const int pv = (precision != CMBPO_PREC_FP32 && ens_tc_supported(v)) ? precision : CMBPO_PREC_FP32;
+    const int pvc = (precision != CMBPO_PREC_FP32 && ens_tc_supported(vc)) ? precision : CMBPO_PREC_FP32;
     if (ens_forward(ctx, v, a.obs, a.N, false, raw_v, pv)) return 1;
-    if (ens_forward(ctx, vc, a.obs, a.N, false, raw_vc, pv)) return 1;
+    if (ens_forward(ctx, vc, a.obs, a.N, false, raw_vc, pvc)) return 1;
     if (with_actor) {
         CMBPO_CHECK(actor.loaded && ctx->log_std, "actor not loaded");
         CMBPO_CHECK(a.A <= CMBPO_MAX_ACT, "act dim too large");

@@ -466,5 +466,8 @@ extern "C" int cmbpo_net_set_scalers(cmbpo_ctx* ctx, int which, const float* mu_
     }
     cudaFree(tmp);
     CUDA_TRY(cudaGetLastError());
+    // the merged policy pack copies V's input scaler and folds every member's scaler into its first layer
+    if (which != CMBPO_NET_DYN && policy_pack_build(ctx)) return 1;
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
     return 0;
 }
