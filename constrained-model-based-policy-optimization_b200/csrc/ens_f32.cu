@@ -203,7 +203,7 @@ int ens_forward(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, bool x_is_3
     CMBPO_CHECK(!x_is_3d, "tcgen05 path takes 2-D inputs only");
     CMBPO_CHECK(ens_tc_supported(net),
                 "tcgen05 path needs 2 hidden layers of equal width <= 512 (<= 64 inputs, <= 128 outputs, <= 96 above width 256) or 3-4 hidden "
-                "layers of equal width <= 256 (<= 64 outputs), swish or tanh; use precision fp32 for this network");
+                "layers of equal width <= 256 (<= 64 inputs, <= 128 outputs), swish or tanh; use precision fp32 for this network");
     return ens_forward_tc(ctx, net, x, N, out_raw, precision, n_dev);
 }
 

@@ -70,6 +70,9 @@ enum { W_FULL = 0, W_EMPTY = NSM, W2_FULL = 2 * NSM, W2_EMPTY = 2 * NSM + NS2, D
        D_EMPTY = D_FULL + 2, H1_FULL = D_FULL + 4, H2_FULL = D_FULL + 5, H2_EMPTY = D_FULL + 7,
        OUT_FULL = D_FULL + 9, OUT_EMPTY = D_FULL + 10, X_FULL = D_FULL + 11, B_FULL = D_FULL + 12,
        B_EMPTY = D_FULL + 14, NBAR = D_FULL + 16 };
+// wide-output deep kernels (WO, no H2 buffers): "last-hidden chunk j drained", j < 4, in the four H2 barriers
+constexpr int HL_FULL = H2_FULL;
+static_assert(H2_EMPTY == H2_FULL + 2, "HL_FULL spans the H2_FULL and H2_EMPTY pairs");
 constexpr int SMEM_W2 = XA_BYTES + NSM * STAGE;
 constexpr int SMEM_BIAS = SMEM_W2 + NS2 * W2SLOT;
 constexpr int SMEM_IN_BYTES = 512;   // input scaler: mu[64] | sigma[64]
@@ -295,17 +298,33 @@ __device__ __forceinline__ void drain32(uint32_t d_addr, const float* bias, uint
 // padded width <= 256 and NP <= 64.  No extra barriers: the tensor pipe executes in order, so by the time a
 // chunk's accumulator is handed to the epilogue every MMA that read the buffer it is about to overwrite has
 // finished; H1_FULL simply completes once per hidden layer instead of once per unit.
+// WO (deep nets with 64 < NP <= 128): there is no room for H2 next to a 128-column OUT, so the last hidden layer
+// writes its whole output into the idle hidden buffer, like a middle layer (it reads buffer NMID&1 and writes
+// buffer LAST = (NMID+1)&1), and layer 2 reads its A operand straight from there, one N = NP MMA per K step:
+//   H1 [0,128)   D [128,256)   HB [256,384)   OUT [512-NP,512) within [384,512)
+// The W2 stream is unchanged: the two NP/2-row tiles of a chunk are, back to back, one NP-row tile.  The layer-2
+// issuer takes K panel j as soon as last-hidden chunk j is drained (HL_FULL + j, once per unit).  The buffers:
+//  * the last-hidden drains overwrite buffer LAST only after everything that read it earlier: the layer before
+//    (the D_FULL of a last-hidden chunk follows it in the layer-0/1 issuer's order) and the previous unit's layer 2
+//    (see the next point);
+//  * the next unit writes buffer LAST again -- at NMID = 1 (LAST = H1) in its layer-0 drains, at NMID = 2
+//    (LAST = HB) in its first middle-layer drains.  Those stores must wait for this unit's layer-2 MMAs, which a
+//    different thread issues (no tensor-pipe order with the layer-0/1 issuer's commits).  At NMID = 2 they follow
+//    the deferred OUT epilogue, whose OUT_FULL wait is exactly that; at NMID = 1 the layer-0 drains come first, so
+//    each epilogue warp's first layer-0 store of a unit waits for the previous unit's OUT_FULL itself.  This also
+//    keeps the epilogue less than a unit ahead of the layer-2 issuer, which makes one HL_FULL phase per unit exact.
 // CL == 2: the CTAs run as CLUSTER PAIRS that stream ONE copy of the weights from L2: both CTAs of a pair work on
 // the same member (two neighbouring row tiles), each fetches half of every main-ring stage and MULTICASTS it into
 // both CTAs' rings.  Why: the layer-1 phase needs a 2 KB weight tile per 32-cycle MMA = 64 B/clk per SM, and 148 SMs
 // x 64 B/clk is more than the L2 slices deliver (~6300 B/clk chip-wide = 42 B/clk per SM, B300_MICROARCH.md):
 // the phase ran at ~47 cycles per MMA.  Everything else (MMAs, tensor memory, epilogue) stays per CTA (cta_group::1);
 // only a ring slot's release is a pair-wide event (both issuers commit to both CTAs' W_EMPTY barriers).
-template <int HD, int FMT, int ACT, int G, bool FUSE, int NMID = 0, int CL = 1>
+template <int HD, int FMT, int ACT, int G, bool FUSE, int NMID = 0, int CL = 1, bool WO = false>
 __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams p) {
     static_assert(CL == 1 || (CL == 2 && G == 1 && !FUSE), "cluster pairs: ordinary ensembles only");
     static_assert(!FUSE || G == 1, "the fused step kernel exists for ordinary (ungrouped) ensembles");
     static_assert(NMID == 0 || (HD <= 256 && G == 1 && !FUSE), "deep variant: width <= 256, ungrouped");
+    static_assert(!WO || (NMID > 0 && HD == 256 && CL == 1), "wide-output variant: deep nets at padded width 256");
     constexpr int W2S = FUSE ? W2SLOT_F : W2SLOT;          // layer-2 ring slot bytes
     constexpr int NC = HD / 64;                     // 64-column chunks of a hidden layer
     constexpr int KP = HD / 64 / G;                 // 64-wide K panels of layer 1 (per member)
@@ -313,8 +332,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     constexpr int TPS = KP < 4 ? KP : 4;            // layer-1 tiles (K panels) per main-ring stage
     constexpr int G0 = NC < 4 ? NC : 4;             // layer-0 chunk tiles per main-ring stage
     constexpr uint32_t COL_H1 = 0, COL_D = HD / 2, COL_H2 = COL_D + 128;
-    constexpr uint32_t COL_HB = COL_H2 + 64;       // second hidden-activation buffer (NMID > 0 only)
+    constexpr uint32_t COL_HB = WO ? COL_H2 : COL_H2 + 64;     // second hidden-activation buffer (NMID > 0 only)
     constexpr int NHID = 1 + NMID;                 // HD x HD layers: NMID middle ones + the last hidden layer
+    constexpr uint32_t COL_LAST = ((NMID + 1) & 1) ? COL_HB : COL_H1;     // WO: the last hidden layer's output
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t* sXA = smem;
@@ -340,7 +360,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         for (int i = 0; i < NS2; ++i) { mbar_init(bar + W2_FULL + i, 1); mbar_init(bar + W2_EMPTY + i, 1); }
         for (int i = 0; i < 2; ++i) {
             mbar_init(bar + D_FULL + i, 1); mbar_init(bar + D_EMPTY + i, 8);
-            mbar_init(bar + H2_FULL + i, 8); mbar_init(bar + H2_EMPTY + i, 1);
+            mbar_init(bar + H2_FULL + i, 8); mbar_init(bar + H2_EMPTY + i, WO ? 8 : 1);    // WO: HL_FULL + 2 + i
         }
         mbar_init(bar + H1_FULL, 8 * NC);
         mbar_init(bar + OUT_FULL, 1); mbar_init(bar + OUT_EMPTY, 16);
@@ -445,7 +465,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         // A warp of its own: the bookkeeping of a partial (three barrier waits, two commits) costs the
         // issuing thread ~1000 cycles per chunk, which on the layer-1 issuer's instruction stream was
         // the kernel's critical path.  The two issuers only meet in the tensor pipe.
-        const uint32_t idesc_o = idesc_f16(FMT, NPp);
+        const uint32_t idesc_o = idesc_f16(FMT, WO ? p.NP : NPp);
         const uint64_t dW2 = smem_desc_sw128(smem_u32(sW2));
         uint32_t s2 = 0, ph2 = 0, c1 = 0, m = 0;
         for (int u = u0; u < u1; ++u) {
@@ -456,10 +476,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 const uint32_t hbar = c1 & 1, hn = c1 >> 1, hb = (nh2 == 2) ? hbar : 0;
                 if (jin == 0) mbar_wait(bar + W2_FULL + s2, ph2);
                 if (jj == 0) mbar_wait(bar + OUT_EMPTY, (m & 1) ^ 1);
-                mbar_wait(bar + H2_FULL + hbar, hn & 1);
+                if constexpr (WO) mbar_wait(bar + HL_FULL + jj, m & 1);
+                else mbar_wait(bar + H2_FULL + hbar, hn & 1);
                 tc_fence_after();
                 const bool last_in_slot = (jin == p.cps - 1) || (jj == NC - 1);
                 if (elect_one()) {
+                    if constexpr (WO) {      // K panel jj of the last hidden layer x the chunk's NP-row W2 tile
+                        const uint64_t dB = dW2 + (uint64_t)((s2 * W2S + jin * p.NP * 128) >> 4);
+#pragma unroll
+                        for (int ks = 0; ks < 4; ++ks)
+                            mma_f16_ts(tmem + col_out, tmem + COL_LAST + jj * 32 + ks * 8, dB + 2 * ks, idesc_o,
+                                       !(jj == 0 && ks == 0));
+                    } else {
                     for (int q = 0; q < p.parts; ++q) {
                         const uint64_t dB = dW2 + (uint64_t)((s2 * W2S + (jin * p.parts + q) * NPp * 128) >> 4);
 #pragma unroll
@@ -468,6 +496,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                                        dB + 2 * ks, idesc_o, !(jj % CPM == 0 && ks == 0));
                     }
                     mma_commit(bar + H2_EMPTY + hbar);
+                    }
                     if (last_in_slot) mma_commit(bar + W2_EMPTY + s2);
                     if (jj == NC - 1) mma_commit(bar + OUT_FULL);
                 }
@@ -783,8 +812,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1;
                     mbar_wait(bar + D_FULL + buf, n & 1);
                     tc_fence_after();
+                    // WO, NMID = 1: H1 is the previous unit's layer-2 A operand (see the kernel comment)
+                    const uint32_t h1_free = (WO && COL_LAST == COL_H1 && have_prev && i == 0) ? bar_a + 8 * OUT_FULL : 0u;
                     drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, p.fold ? nullptr : sb + j * 64 + half * 32,
-                                      tmem + COL_H1 + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u,
+                                      tmem + COL_H1 + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf),
+                                      h1_free, WO ? (prev_m & 1) : 0u,
                                       ACT == 0 && p.member_act[e * G + j / CPM] != CMBPO_ACT_TANH);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * H1_FULL);
@@ -810,6 +842,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                         g += NC;
                     }
                 }
+                if constexpr (WO) {
+                for (int i = 0; i < NC / 2; ++i) {               // last hidden layer, chunk j -> buffer LAST, K panel j
+                    const int j = 2 * i + (int)pair;
+                    const uint32_t gg = g + j, buf = pair, n = gg >> 1;
+                    mbar_wait(bar + D_FULL + buf, n & 1);
+                    tc_fence_after();
+                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + NHID * HD + j * 64 + half * 32,
+                                      tmem + COL_LAST + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u);
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_a(bar_a + 8 * (HL_FULL + j));
+                }
+                } else
                 for (int i = 0; i < NC / 2; ++i) {               // last hidden layer, chunk j -> an H2 buffer
                     const int j = 2 * i + (int)pair;
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1, cc = c1 + j;
@@ -929,7 +973,8 @@ OutShape out_shape(int Nout) {
 
 // the order in which the MMA warp consumes weight tiles (must match the kernel's loops):
 // main stream = layer-0 chunk tiles, then per chunk the layer-1 K-panel tiles; W2 stream = per chunk
-// the layer-2 tile(s)
+// the layer-2 tile(s).  The wide-output deep kernels (WO) read a two-part chunk as ONE tile of NP rows: tile
+// rows are 128 B apart and NP/2 is a multiple of 8, so the q = 1 tile starts exactly at row NP/2 of it.
 void stage_programs(int HD, int NP, int parts, int group, int nhid, std::vector<Stage>* main_prog,
                     unsigned long long* main_bytes, std::vector<Stage>* w2_prog, unsigned long long* w2_bytes) {
     // nhid = number of HD x HD layers (1 + NMID); Stage.layer indexes the master copies: 0, 1 .. nhid, nhid + 1 = output
@@ -961,11 +1006,11 @@ int chunks_per_w2_slot(int HD, int NP, int slot_bytes = W2SLOT) {
     return p2 < NC ? p2 : NC;
 }
 
-template <int HD, int FMT, int ACT, int G = 1, bool FUSE = false, int NMID = 0>
+template <int HD, int FMT, int ACT, int G = 1, bool FUSE = false, int NMID = 0, bool WO = false>
 int launch_tc(cmbpo_ctx* ctx, const TcParams& p) {
     const int smem = (FUSE ? SMEM_TOTAL_F : SMEM_TOTAL) + 1024;
     static_assert(SMEM_TOTAL + 1024 <= 232448, "shared memory budget");
-    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, G, FUSE, NMID>;
+    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, G, FUSE, NMID, 1, WO>;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const long long units = (long long)p.ntiles * ((p.E + G - 1) / G);
     const int grid = units < ctx->sm_count ? (int)units : ctx->sm_count;
@@ -1025,14 +1070,19 @@ int launch_tc_act(cmbpo_ctx* ctx, const TcParams& p, int act) {
     return launch_tc<HD, FMT, CMBPO_ACT_TANH>(ctx, p);
 }
 
-// 3 / 4 hidden layers at (padded) width 256
+// 3 / 4 hidden layers at (padded) width 256; more than 64 output columns take the wide-output kernel (WO)
+template <int FMT, int ACT, int NMID>
+int launch_tc_deep_out(cmbpo_ctx* ctx, const TcParams& p) {
+    if (p.NP > 64) return launch_tc<256, FMT, ACT, 1, false, NMID, true>(ctx, p);
+    return launch_tc<256, FMT, ACT, 1, false, NMID>(ctx, p);
+}
 template <int FMT>
 int launch_tc_deep(cmbpo_ctx* ctx, const TcParams& p, int act, int nmid) {
     if (act == CMBPO_ACT_SWISH)
-        return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, false, 1>(ctx, p)
-                         : launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, false, 2>(ctx, p);
-    return nmid == 1 ? launch_tc<256, FMT, CMBPO_ACT_TANH, 1, false, 1>(ctx, p)
-                     : launch_tc<256, FMT, CMBPO_ACT_TANH, 1, false, 2>(ctx, p);
+        return nmid == 1 ? launch_tc_deep_out<FMT, CMBPO_ACT_SWISH, 1>(ctx, p)
+                         : launch_tc_deep_out<FMT, CMBPO_ACT_SWISH, 2>(ctx, p);
+    return nmid == 1 ? launch_tc_deep_out<FMT, CMBPO_ACT_TANH, 1>(ctx, p)
+                     : launch_tc_deep_out<FMT, CMBPO_ACT_TANH, 2>(ctx, p);
 }
 
 template <int FMT>
@@ -1059,14 +1109,15 @@ int launch_tc_hd(cmbpo_ctx* ctx, const TcParams& p, int hd, int act) {
 // 2 hidden layers: any equal width <= 512 (padded to 128 / 256 / 512), <= 64 inputs, <= 128 outputs; <= 96 outputs
 // above width 256 (tensor memory: at width 512 the OUT accumulator of a 128-column output, 512 - NP = column 384,
 // would overlap the single H2 buffer at columns 384-415).
-// 3 or 4 hidden layers (e.g. the (200,200,200,200) default of algorithms/cmbpo.py:54): equal width <= 256, <= 64 outputs
-// (tensor-memory budget of the second hidden buffer).
+// 3 or 4 hidden layers (e.g. the (200,200,200,200) default of algorithms/cmbpo.py:54): equal width <= 256, <= 64
+// inputs, <= 128 outputs (tensor memory: two hidden buffers, the accumulators and OUT fill the 512 columns; above 64
+// outputs the last hidden layer's buffer is layer 2's A operand, see WO at the kernel).
 bool ens_tc_supported(const Net& n) {
     if (!n.loaded || n.n_layers < 3 || n.n_layers > 5) return false;
     const int hd = n.dims[1], L = n.n_layers;
     for (int l = 1; l < L; ++l) if (n.dims[l] != hd) return false;
     if (hd < 1 || hd > (L == 3 ? 512 : 256)) return false;
-    if (n.dims[0] > 64 || n.dims[L] > (L == 3 ? (hd > 256 ? 96 : 128) : 64)) return false;
+    if (n.dims[0] > 64 || n.dims[L] > ((L == 3 && hd > 256) ? 96 : 128)) return false;
     for (int l = 1; l < L - 1; ++l) if (n.acts[l] != n.acts[0]) return false;
     if (n.acts[L - 1] != CMBPO_ACT_NONE) return false;
     return n.acts[0] == CMBPO_ACT_SWISH || n.acts[0] == CMBPO_ACT_TANH;
