@@ -127,11 +127,8 @@ static inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 int ens_forward_f32(cmbpo_ctx* ctx, const Net& net, const float* x, int64_t N, bool x_is_3d,
                     float* out_raw);
 // tcgen05 MLP chain (2 hidden layers), same contract
-struct FusedStep;       // step_common.cuh
 int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* out_raw,
-                   int precision, const int64_t* n_dev = nullptr, const FusedStep* fz = nullptr);
-bool ens_tc_fusable(const Net& net);
-int ens_tc_fused_rp_shift(int obs_dim);
+                   int precision, const int64_t* n_dev = nullptr);
 bool ens_tc_supported(const Net& net);
 int ens_tc_prepare(cmbpo_ctx* ctx, Net& net);
 int policy_pack_build(cmbpo_ctx* ctx);

@@ -28,9 +28,7 @@
 // Replaces models/pens/fc.py:74-95 x3 + the input scaler of models/pens/utils.py:156 (fused into the
 // XA load).  The output scaler / exp are applied by the consumer (ens_head_kernel or the rollout row
 // math) exactly as on the fp32 path.
-#include <cstring>
 #include "tc_common.cuh"
-#include "step_common.cuh"
 
 using namespace tc;
 
@@ -62,7 +60,6 @@ struct TcParams {
     float* out; long long out_member_stride;   // out[e*stride + row*Nout + c]
     int ntiles;
     int member_act[CMBPO_MAX_E];   // ACT == 0 kernels (merged nets): hidden activation per member
-    FusedStep fz;              // FUSE kernels only: the rollout step around the GEMM chain (step_common.cuh)
 };
 
 // barrier indices
@@ -78,162 +75,10 @@ constexpr int SMEM_BIAS = SMEM_W2 + NS2 * W2SLOT;
 constexpr int SMEM_IN_BYTES = 512;   // input scaler: mu[64] | sigma[64]
 constexpr int SMEM_BAR = SMEM_BIAS + 2 * BIAS_SLOT + SMEM_IN_BYTES;
 constexpr int SMEM_TOTAL = SMEM_BAR + NBAR * 8 + 16;
-// FUSE kernels (the rollout step fused around the GEMM chain): the layer-2 ring shrinks to 2 x 12 KB (a
-// 2 x 8 KB ring measured the same as 2 x 24 KB) and the freed shared memory stages the row math:
-//   stage  12 KB   kl, epv per (obs dimension, row) of one pass of RP rows (RP = 64 / 32 by obs dim)
-//   misc    5 KB   per-row member / path / state / non-finite flag, the 4 next-state coordinates the statics
-//                  read, output-scaler vectors, log_std, elite list, the "last arriver" flag
-constexpr int W2SLOT_F = 12288;
-constexpr int FZ_STAGE = 12288, FZ_MISC = 5120;
-constexpr int SMEM_BIAS_F = SMEM_W2 + NS2 * W2SLOT_F;
-constexpr int SMEM_BAR_F = SMEM_BIAS_F + 2 * BIAS_SLOT + SMEM_IN_BYTES;
-constexpr int SMEM_FZ = SMEM_BAR_F + NBAR * 8 + 16;
-constexpr int SMEM_TOTAL_F = SMEM_FZ + FZ_STAGE + FZ_MISC;
-static_assert(SMEM_FZ % 16 == 0 && SMEM_TOTAL_F + 1024 <= 232448, "fused shared-memory budget");
-
-struct FzSmem {          // views into the misc area
-    float *kl, *epv;                 // [O][RP]
-    int *member, *path;              // [128]
-    int* nonfin;                     // [128]
-    float* spec;                     // [4][128]: next_obs[0], [2], [3], [O-1]
-    float *sig, *mu, *l2s;           // [64] output scaler (pens/utils.py:167,187)
-    float* log_std;                  // [32]
-    int* elite;                      // [8]
-    unsigned char* state;            // [128]
-    int* flag;
-};
-__device__ __forceinline__ FzSmem fz_views(uint8_t* base) {
-    FzSmem m;
-    m.kl = reinterpret_cast<float*>(base);
-    m.epv = nullptr;                 // set per launch geometry: kl + O * RP
-    uint8_t* q = base + FZ_STAGE;
-    m.member = reinterpret_cast<int*>(q); q += 512;
-    m.path = reinterpret_cast<int*>(q); q += 512;
-    m.nonfin = reinterpret_cast<int*>(q); q += 512;
-    m.spec = reinterpret_cast<float*>(q); q += 2048;
-    m.sig = reinterpret_cast<float*>(q); q += 256;
-    m.mu = reinterpret_cast<float*>(q); q += 256;
-    m.l2s = reinterpret_cast<float*>(q); q += 256;
-    m.log_std = reinterpret_cast<float*>(q); q += 128;
-    m.elite = reinterpret_cast<int*>(q); q += 32;
-    m.state = q; q += 128;
-    m.flag = reinterpret_cast<int*>(q); q += 16;
-    return m;                        // 4656 B <= FZ_MISC
-}
 
 __device__ __forceinline__ void epi_bar() {      // named barrier 1: the 512 epilogue threads
     asm volatile("bar.sync 1, 512;" ::: "memory");
 }
-
-// ---- the rollout step's row math for one finished row tile (all E members' outputs sit in the L2
-// scratch), run by the 512 epilogue threads of the CTA that delivered the tile's last member.
-// Same phases and literally the same per-row functions as rollout_step_kernel (rollout.cu):
-//   0  one thread per row: elite member, carried per-path scalars
-//   1  one thread per (obs dim, row), lanes along rows (coalesced scratch reads): member statistics, KL
-//   2  one thread per row: ordered sums over dims (numpy order), statics, sampler rules, per-step scalars
-//   3  one thread per (row, dim), lanes along dims (coalesced buffer writes): next state of the chosen
-//      member recomputed (bit-identical), obs / next_obs / act / mu rows, carried state
-__device__ __forceinline__ void fused_rows(const FusedStep& f, const FzSmem& sm, int tile, long long n_rows, int etid) {
-    const int O = f.O, A = f.A, W = 2 * f.c.D, t = f.rules.t, sh = f.rp_shift, RP = 1 << sh;
-    const float* tbase = f.raw_tiles + (size_t)tile * f.c.E * W * 128;
-    EnvRowCfg c = f.c;
-    c.sig_out = sm.sig; c.mu_out = sm.mu; c.l2s_out = sm.l2s; c.elite = sm.elite;
-    float* s_kl = sm.kl;
-    float* s_epv = sm.kl + O * RP;
-    const int lane = etid & 31;
-    for (int r0 = 0; r0 < 128; r0 += RP) {
-        const long long base = (long long)tile * 128 + r0;
-        if (base >= n_rows) break;                                   // uniform
-        float pf_v = 0.f, pf_vc = 0.f, pf_logp = 0.f;
-        double pf_dkl = 0.0, pf_ret = 0.0, pf_cost = 0.0;
-        if (etid < RP) {
-            const long long r = base + etid;
-            int member = -1, path = -1;
-            if (r < n_rows) {
-                path = f.row_path ? f.row_path[r] : (int)r;
-                if (f.rules.alive[path]) {
-                    const int pos = f.elite_pos ? f.elite_pos[path] : philox_elite_pos(f.seed, f.path_base + path, t, f.n_elite);
-                    member = sm.elite[pos];
-                    pf_v = f.vrow[r]; pf_vc = f.vcrow[r]; pf_logp = f.logp[r];
-                    pf_dkl = f.rules.b.cum_dkl[path]; pf_ret = f.rules.b.path_return[path]; pf_cost = f.rules.b.path_cost[path];
-                }
-            }
-            sm.member[etid] = member; sm.path[etid] = path; sm.state[etid] = 0; sm.nonfin[etid] = 0;
-        }
-        epi_bar();
-        const int NI = RP * O;
-        for (int idx = etid; idx < NI; idx += 512) {
-            const int rr = idx & (RP - 1), dim = idx >> sh;
-            const int member = sm.member[rr];
-            if (member < 0) continue;
-            const long long pth = sm.path[rr];
-            float eps = 1.0f;
-            if (!c.deterministic)
-                eps = f.state_eps ? f.state_eps[pth * O + dim] : philox_normal(f.seed, f.path_base + pth, t, RNG_STREAM_STATE, dim);
-            RawTile raw(tbase, W, r0 + rr);
-            const EnvDimOut d = env_dim<7, true>(c, raw, dim, member, f.cur_obs[(base + rr) * O + dim], eps);
-            s_kl[idx] = d.kl; s_epv[idx] = d.epv;
-            if (!isfinite(d.nx)) sm.nonfin[rr] = 1;
-            if (dim == 0) sm.spec[rr] = d.nx;
-            if (dim == 2) sm.spec[128 + rr] = d.nx;
-            if (dim == 3) sm.spec[256 + rr] = d.nx;
-            if (dim == O - 1) sm.spec[384 + rr] = d.nx;
-        }
-        epi_bar();
-        double st0 = 0.0, st1 = 0.0, st2 = 0.0, st3 = 0.0;
-        if (etid < RP) {
-            const int member = sm.member[etid];
-            if (member >= 0) {
-                const long long pth = sm.path[etid];
-                RawTile raw(tbase, W, r0 + etid);
-                const float ks = np_sum_strided(s_kl + etid, O, RP), es = np_sum_strided(s_epv + etid, O, RP);
-                const EnvRowOut o = env_row_core<true>(c, raw, member, ks, es, sm.nonfin[etid] == 0, sm.spec[etid],
-                                                       sm.spec[128 + etid], sm.spec[256 + etid], sm.spec[384 + etid]);
-                RowCarry pf;
-                pf.v = pf_v; pf.vc = pf_vc; pf.logp = pf_logp; pf.dkl = pf_dkl; pf.ret = pf_ret; pf.cost = pf_cost;
-                sm.state[etid] = (unsigned char)step_row_commit(f.rules, pth, o, pf, st0, st1, st2, st3);
-            }
-            // per-step statistics: one reduction per warp of row threads, four REDs per warp
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                st0 += __shfl_down_sync(0xffffffffu, st0, off); st1 += __shfl_down_sync(0xffffffffu, st1, off);
-                st2 += __shfl_down_sync(0xffffffffu, st2, off); st3 += __shfl_down_sync(0xffffffffu, st3, off);
-            }
-            if (lane == 0 && st0 != 0.0) {
-                double* ss = f.rules.b.step_stats + (long long)t * 4;
-                atomicAdd(ss + 0, st0); atomicAdd(ss + 1, st1); atomicAdd(ss + 2, st2); atomicAdd(ss + 3, st3);
-            }
-        }
-        epi_bar();
-        for (int idx = etid; idx < NI; idx += 512) {
-            const int rr = idx / O, dim = idx - rr * O;
-            if (sm.state[rr] != 1) continue;
-            const int member = sm.member[rr];
-            const long long pth = sm.path[rr], row = (long long)t * f.rules.B + pth;
-            float eps = 1.0f;
-            if (!c.deterministic)
-                eps = f.state_eps ? f.state_eps[pth * O + dim] : philox_normal(f.seed, f.path_base + pth, t, RNG_STREAM_STATE, dim);
-            RawTile raw(tbase, W, r0 + rr);
-            const float ob = f.cur_obs[(base + rr) * O + dim];
-            const float nx = env_dim_nx<true>(c, raw, dim, member, ob, eps);
-            if (!f.rules.no_store) {
-                f.rules.b.obs[row * O + dim] = ob;
-                f.rules.b.nextobs[row * O + dim] = nx;
-            }
-            f.cur_obs[(base + rr) * O + dim] = nx;                 // model_sampler.py:350
-        }
-        if (!f.rules.no_store)
-        for (int idx = etid; idx < RP * A; idx += 512) {
-            const int rr = idx / A, i = idx - rr * A;
-            if (sm.state[rr] != 1) continue;
-            const long long pth = sm.path[rr], row = (long long)t * f.rules.B + pth;
-            f.rules.b.act[row * A + i] = f.pi[(base + rr) * A + i];
-            f.rules.b.mu[row * A + i] = f.mu[(base + rr) * A + i];
-        }
-        epi_bar();                                                   // the staging is reused by the next pass / tile
-    }
-}
-
 
 // 32 accumulator columns of this thread's row -> (+bias), act -> 16-bit pairs -> 16 TMEM columns.
 // The accumulator buffer is released (`d_empty`) as soon as the values sit in registers; the
@@ -319,13 +164,11 @@ __device__ __forceinline__ void drain32(uint32_t d_addr, const float* bias, uint
 // x 64 B/clk is more than the L2 slices deliver (~6300 B/clk chip-wide = 42 B/clk per SM, B300_MICROARCH.md):
 // the phase ran at ~47 cycles per MMA.  Everything else (MMAs, tensor memory, epilogue) stays per CTA (cta_group::1);
 // only a ring slot's release is a pair-wide event (both issuers commit to both CTAs' W_EMPTY barriers).
-template <int HD, int FMT, int ACT, int G, bool FUSE, int NMID = 0, int CL = 1, bool WO = false>
+template <int HD, int FMT, int ACT, int G, int NMID = 0, int CL = 1, bool WO = false>
 __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams p) {
-    static_assert(CL == 1 || (CL == 2 && G == 1 && !FUSE), "cluster pairs: ordinary ensembles only");
-    static_assert(!FUSE || G == 1, "the fused step kernel exists for ordinary (ungrouped) ensembles");
-    static_assert(NMID == 0 || (HD <= 256 && G == 1 && !FUSE), "deep variant: width <= 256, ungrouped");
+    static_assert(CL == 1 || (CL == 2 && G == 1), "cluster pairs: ordinary ensembles only");
+    static_assert(NMID == 0 || (HD <= 256 && G == 1), "deep variant: width <= 256, ungrouped");
     static_assert(!WO || (NMID > 0 && HD == 256 && CL == 1), "wide-output variant: deep nets at padded width 256");
-    constexpr int W2S = FUSE ? W2SLOT_F : W2SLOT;          // layer-2 ring slot bytes
     constexpr int NC = HD / 64;                     // 64-column chunks of a hidden layer
     constexpr int KP = HD / 64 / G;                 // 64-wide K panels of layer 1 (per member)
     constexpr int CPM = NC / G;                     // chunks per member
@@ -340,11 +183,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     uint8_t* sXA = smem;
     uint8_t* sW = smem + XA_BYTES;
     uint8_t* sW2 = smem + SMEM_W2;
-    float* sBias = reinterpret_cast<float*>(smem + (FUSE ? SMEM_BIAS_F : SMEM_BIAS));
+    float* sBias = reinterpret_cast<float*>(smem + SMEM_BIAS);
     float* sIn = sBias + 2 * BIAS_SLOT / 4;
-    constexpr int BAR_OFF = FUSE ? SMEM_BAR_F : SMEM_BAR;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + BAR_OFF);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + BAR_OFF + NBAR * 8);
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + SMEM_BAR);
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + SMEM_BAR + NBAR * 8);
 
     // Warp roles: 0 = main weight producer, 1 = layer-0/1 MMA issuer, 2 = TMEM allocator + layer-2 MMA
     // issuer, 3 = W2 producer, 4-19 = epilogue (four warpgroups).  A warp may only touch the TMEM lane
@@ -452,7 +294,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     mbar_wait(bar + W2_EMPTY + s2, ph2 ^ 1);
                     if (elect_one()) {
                         mbar_expect_tx(bar + W2_FULL + s2, bytes);
-                        bulk_g2s(sW2 + s2 * W2S, src, bytes, bar + W2_FULL + s2);
+                        bulk_g2s(sW2 + s2 * W2SLOT, src, bytes, bar + W2_FULL + s2);
                     }
                     __syncwarp();
                     src += bytes;
@@ -482,14 +324,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 const bool last_in_slot = (jin == p.cps - 1) || (jj == NC - 1);
                 if (elect_one()) {
                     if constexpr (WO) {      // K panel jj of the last hidden layer x the chunk's NP-row W2 tile
-                        const uint64_t dB = dW2 + (uint64_t)((s2 * W2S + jin * p.NP * 128) >> 4);
+                        const uint64_t dB = dW2 + (uint64_t)((s2 * W2SLOT + jin * p.NP * 128) >> 4);
 #pragma unroll
                         for (int ks = 0; ks < 4; ++ks)
                             mma_f16_ts(tmem + col_out, tmem + COL_LAST + jj * 32 + ks * 8, dB + 2 * ks, idesc_o,
                                        !(jj == 0 && ks == 0));
                     } else {
                     for (int q = 0; q < p.parts; ++q) {
-                        const uint64_t dB = dW2 + (uint64_t)((s2 * W2S + (jin * p.parts + q) * NPp * 128) >> 4);
+                        const uint64_t dB = dW2 + (uint64_t)((s2 * W2SLOT + (jin * p.parts + q) * NPp * 128) >> 4);
 #pragma unroll
                         for (int ks = 0; ks < 4; ++ks)
                             mma_f16_ts(tmem + col_out + (jj / CPM) * p.NP + q * NPp, tmem + COL_H2 + hb * 32 + ks * 8,
@@ -637,7 +479,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         uint32_t g = 0, m = 0, c1 = 0;
         // deferred OUT epilogue: the four warpgroups split the NP output columns (16 or 32 each)
         int prev_e = 0; long long prev_grow = 0; uint32_t prev_m = 0; bool have_prev = false;
-        int prev_tile = 0;
         const int etid = (int)threadIdx.x - 128;                      // 0..511 among the epilogue threads
         // input scaler -> shared memory (identity when the net has none)
         if (etid < 64) {
@@ -645,17 +486,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             sIn[64 + etid] = (p.mu_in && etid < p.K0) ? p.sig_in[etid] : 1.f;
         }
         epi_bar();
-        FzSmem fsm;
-        if (FUSE) {
-            fsm = fz_views(smem + SMEM_FZ);
-            // small read-only vectors of the row math -> shared memory (no L1 in this carve-out: a global load per use
-            // is an L2 round trip)
-            const FusedStep& f = p.fz;
-            for (int i = etid; i < f.c.D; i += 512) { fsm.sig[i] = f.c.sig_out[i]; fsm.mu[i] = f.c.mu_out[i]; fsm.l2s[i] = f.c.l2s_out[i]; }
-            if (etid < f.A) fsm.log_std[etid] = f.log_std[etid];
-            if (etid < f.n_elite && etid < 8) fsm.elite[etid] = f.c.elite[etid];
-            epi_bar();
-        }
         const int out_cw = (G > 1) ? p.NP : ((p.NP <= 64) ? 16 : 32);
         auto out_epilogue = [&]() {
             mbar_wait(bar + OUT_FULL, prev_m & 1);
@@ -671,34 +501,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(bar + OUT_EMPTY);          // accumulator free again (16 warps arrive)
-            if (FUSE) {
-                // raw outputs -> tile-transposed L2 scratch (column-major inside the tile: a warp stores 32
-                // consecutive floats per column), then the "last arriver" protocol: the CTA that delivers
-                // the tile's E-th member runs the row math for the tile
-                const FusedStep& f = p.fz;
-                if (mine) {
-                    const float* b2 = p.bias + (long long)prev_e * p.bias_stride + (1 + NHID) * HD;
-                    float* dst = f.raw_tiles + ((size_t)prev_tile * p.E + prev_e) * p.Nout * 128 + row;
-#pragma unroll
-                    for (int i = 0; i < 32; ++i) {
-                        const int c = c_begin + i;
-                        if (i < out_cw && c < p.Nout) __stcg(dst + (size_t)c * 128, __uint_as_float(r[i]) + __ldg(b2 + c));
-                    }
-                }
-                __threadfence();
-                epi_bar();
-                if (etid == 0) {
-                    const int old = atomicAdd(f.tile_cnt + prev_tile, 1);
-                    const int last = (old == p.E - 1) ? 1 : 0;
-                    if (last) f.tile_cnt[prev_tile] = 0;              // ready for the next step's launch
-                    *fsm.flag = last;
-                }
-                epi_bar();
-                if (*fsm.flag) {
-                    __threadfence();
-                    fused_rows(f, fsm, prev_tile, n_rows, etid);
-                }
-            } else
             if (mine && prev_grow < n_rows) {
                 const int cb = (G > 1) ? 0 : c_begin;          // first output column of this warpgroup's slice
                 float* orow = p.out + (long long)(prev_e * G + (G > 1 ? wg : 0)) * p.out_member_stride + prev_grow * p.Nout;
@@ -733,33 +535,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             cur_tile = tile;
             grow = (long long)tile * 128 + row;
             if (new_tile && wg == 0) {
-                bool feed = grow < n_rows;
+                const bool feed = grow < n_rows;
                 const float* xr = p.x + grow * p.ldx;
-                if (FUSE) {
-                    // policy head of this row (what policy_rows_kernel does on the step-wise path): value heads,
-                    // pending bootstraps, Gaussian head; the action goes to the per-row stash and, with the
-                    // observation, into the XA panel below.  A tile shared by two CTAs is done by both: same
-                    // inputs, same values.
-                    const FusedStep& f = p.fz;
-                    if (feed) {
-                        const long long pth = f.row_path ? (long long)f.row_path[grow] : grow;
-                        const float v = value_of(f.v, f.rules.B, grow), vc = value_of(f.vc, f.rules.B, grow);
-                        const uint8_t pend = f.rules.pending[pth];
-                        if (pend) {                                   // model_sampler.py:401-407 on s_{t+1}
-                            if (pend & 1) f.rules.b.last_val[pth] = v;
-                            if (pend & 2) f.rules.b.last_cval[pth] = vc;
-                            f.rules.pending[pth] = 0;
-                        }
-                        feed = f.rules.alive[pth] != 0;
-                        if (feed) {
-                            f.vrow[grow] = v; f.vcrow[grow] = vc;
-                            f.logp[grow] = policy_head_row<true>(f.pol_raw + grow * f.A, fsm.log_std,
-                                                                 f.act_eps ? f.act_eps + pth * f.A : nullptr, f.seed,
-                                                                 f.path_base + pth, f.rules.t, f.A, f.pi + grow * f.A,
-                                                                 f.mu + grow * f.A);
-                        }
-                    }
-                }
                 // XA: this row of the input, scaled (pens/utils.py:156), 16-bit, zero padded to 64.  All global
                 // loads of a 16-column batch are issued before the first use (one L2 round trip per 16 columns; the
                 // earlier 8-column loop with the scaler vectors in global memory cost ~10 k cycles per row
@@ -773,10 +550,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
                             const int k = h * 16 + i;
-                            if (k < p.K0 && feed) {
-                                if (FUSE) v[i] = (k < p.fz.O) ? p.fz.cur_obs[grow * p.fz.O + k] : p.fz.pi[grow * p.fz.A + (k - p.fz.O)];
-                                else v[i] = xr[k];
-                            }
+                            if (k < p.K0 && feed) v[i] = xr[k];
                         }
 #pragma unroll
                         for (int i = 0; i < 16; ++i) {
@@ -877,7 +651,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 __syncwarp();
                 if (lane == 0) mbar_arrive_a(bar_a + 8 * (B_EMPTY + (m & 1)));     // the bias buffer may be refilled
                 g += NC; c1 += NC;
-                prev_e = e; prev_grow = grow; prev_m = m; prev_tile = tile; have_prev = true;
+                prev_e = e; prev_grow = grow; prev_m = m; have_prev = true;
                 ++m;
             }
         }
@@ -998,19 +772,19 @@ void stage_programs(int HD, int NP, int parts, int group, int nhid, std::vector<
     *w2_bytes = off;
 }
 
-int chunks_per_w2_slot(int HD, int NP, int slot_bytes = W2SLOT) {
-    int cps = slot_bytes / (NP * 128);
+int chunks_per_w2_slot(int HD, int NP) {
+    int cps = W2SLOT / (NP * 128);
     int p2 = 1;
     while (p2 * 2 <= cps) p2 *= 2;
     const int NC = HD / 64;
     return p2 < NC ? p2 : NC;
 }
 
-template <int HD, int FMT, int ACT, int G = 1, bool FUSE = false, int NMID = 0, bool WO = false>
+template <int HD, int FMT, int ACT, int G = 1, int NMID = 0, bool WO = false>
 int launch_tc(cmbpo_ctx* ctx, const TcParams& p) {
-    const int smem = (FUSE ? SMEM_TOTAL_F : SMEM_TOTAL) + 1024;
+    const int smem = SMEM_TOTAL + 1024;
     static_assert(SMEM_TOTAL + 1024 <= 232448, "shared memory budget");
-    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, G, FUSE, NMID, 1, WO>;
+    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, G, NMID, 1, WO>;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const long long units = (long long)p.ntiles * ((p.E + G - 1) / G);
     const int grid = units < ctx->sm_count ? (int)units : ctx->sm_count;
@@ -1025,7 +799,7 @@ int launch_tc(cmbpo_ctx* ctx, const TcParams& p) {
 template <int HD, int FMT, int ACT>
 int launch_tc_pairs(cmbpo_ctx* ctx, const TcParams& p) {
     const int smem = SMEM_TOTAL + 1024;
-    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, 1, false, 0, 2>;
+    auto kern = ens_mlp3_tc_kernel<HD, FMT, ACT, 1, 0, 2>;
     static int max_pairs = -1;
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
@@ -1055,14 +829,6 @@ int launch_tc_pairs(cmbpo_ctx* ctx, const TcParams& p) {
     return 0;
 }
 
-// the fused rollout step: swish dynamics ensembles of any supported width
-template <int FMT>
-int launch_tc_fused(cmbpo_ctx* ctx, const TcParams& p, int hd) {
-    if (hd == 128) return launch_tc<128, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
-    if (hd == 256) return launch_tc<256, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
-    return launch_tc<512, FMT, CMBPO_ACT_SWISH, 1, true>(ctx, p);
-}
-
 template <int HD, int FMT>
 int launch_tc_act(cmbpo_ctx* ctx, const TcParams& p, int act) {
     if (act == 0) return launch_tc<HD, FMT, 0>(ctx, p);
@@ -1073,8 +839,8 @@ int launch_tc_act(cmbpo_ctx* ctx, const TcParams& p, int act) {
 // 3 / 4 hidden layers at (padded) width 256; more than 64 output columns take the wide-output kernel (WO)
 template <int FMT, int ACT, int NMID>
 int launch_tc_deep_out(cmbpo_ctx* ctx, const TcParams& p) {
-    if (p.NP > 64) return launch_tc<256, FMT, ACT, 1, false, NMID, true>(ctx, p);
-    return launch_tc<256, FMT, ACT, 1, false, NMID>(ctx, p);
+    if (p.NP > 64) return launch_tc<256, FMT, ACT, 1, NMID, true>(ctx, p);
+    return launch_tc<256, FMT, ACT, 1, NMID>(ctx, p);
 }
 template <int FMT>
 int launch_tc_deep(cmbpo_ctx* ctx, const TcParams& p, int act, int nmid) {
@@ -1172,23 +938,8 @@ int ens_tc_prepare(cmbpo_ctx* ctx, Net& net) {
     return 0;
 }
 
-// the conditions under which cmbpo_rollout may fuse the step around this ensemble's GEMM chain
-bool ens_tc_fusable(const Net& n) {
-    if (!ens_tc_supported(n) || n.n_layers != 3 || n.tc_group != 1 || n.E != 7 || !n.probabilistic) return false;
-    if (n.acts[0] != CMBPO_ACT_SWISH || n.member_act[0] >= 0) return false;
-    const OutShape os = out_shape(n.dims[3]);
-    return os.NP * 128 <= W2SLOT_F && n.D <= 64;       // one chunk's layer-2 tiles must fit a (shrunk) ring slot
-}
-
-int ens_tc_fused_rp_shift(int O) {
-    // rows per row-math pass: kl + epv staging of [O][RP] floats each within FZ_STAGE
-    int sh = 7;
-    while (sh > 5 && (size_t)(1 << sh) * O * 8 > (size_t)FZ_STAGE) --sh;
-    return ((size_t)(1 << sh) * O * 8 <= (size_t)FZ_STAGE) ? sh : -1;
-}
-
 int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* out_raw, int precision,
-                   const int64_t* n_dev, const FusedStep* fz) {
+                   const int64_t* n_dev) {
     CMBPO_CHECK(precision == CMBPO_PREC_BF16 || precision == CMBPO_PREC_FP16, "bad precision %d", precision);
     CMBPO_CHECK(net.tc_pack[precision], "tcgen05 weights not packed");
     if (N <= 0) return 0;
@@ -1199,7 +950,7 @@ int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* o
     TcParams p;
     p.Nout = net.dims[net.n_layers];
     p.NP = os.NP; p.parts = os.parts;
-    p.cps = chunks_per_w2_slot(HD * net.tc_group, os.NP, fz ? W2SLOT_F : W2SLOT);
+    p.cps = chunks_per_w2_slot(HD * net.tc_group, os.NP);
     p.wmain = (const uint8_t*)net.tc_pack[precision];
     p.main_bytes = net.tc_pack_bytes[precision];
     p.w2 = p.wmain + (size_t)((net.E + net.tc_group - 1) / net.tc_group) * p.main_bytes;
@@ -1213,12 +964,6 @@ int ens_forward_tc(cmbpo_ctx* ctx, Net& net, const float* x, int64_t N, float* o
     p.out = out_raw; p.out_member_stride = (long long)N * p.Nout;
     p.ntiles = (int)((N + 127) / 128);
     for (int i = 0; i < CMBPO_MAX_E; ++i) p.member_act[i] = net.member_act[i];
-    if (fz) {
-        CMBPO_CHECK(ens_tc_fusable(net) && fz->rp_shift >= 5, "this ensemble cannot run the fused rollout step");
-        p.fz = *fz;
-        return precision == CMBPO_PREC_FP16 ? launch_tc_fused<0>(ctx, p, HD) : launch_tc_fused<1>(ctx, p, HD);
-    }
-    memset(&p.fz, 0, sizeof(p.fz));
     const int act_sel = net.member_act[0] >= 0 ? 0 : net.acts[0];
     if (nmid > 0) {
         CMBPO_CHECK(HD == 256 && group == 1 && (nmid == 1 || nmid == 2) && net.member_act[0] < 0, "deep tcgen05 variant: bad shape");

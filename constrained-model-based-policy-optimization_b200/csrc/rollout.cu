@@ -2,8 +2,7 @@
 // ModelBuffer write-out) and the single-step entry points cmbpo_policy_act / cmbpo_fakeenv_step.
 //
 // The GEMM chains go through ens_forward(precision): fp32 CUDA cores (logic reference on the
-// device) or the tcgen05 kernels of ens_tc.cu.  The per-row arithmetic lives in row_math.cuh and
-// is shared with the fully fused kernel.
+// device) or the tcgen05 kernels of ens_tc.cu.  The per-row arithmetic lives in row_math.cuh.
 //
 // Reference: samplers/model_sampler.py:239-375 (sample), 377-416 (_finish_paths),
 //            models/fake_env.py:66-172, buffers/modelbuffer.py:114-135 (store_multiple),
@@ -12,9 +11,26 @@
 #include <cstring>
 #include "common.cuh"
 #include "row_math.cuh"
-#include "step_common.cuh"
 
 namespace {
+
+// one non-probabilistic value ensemble read through PE.predict (cpo_policy.py:801-835, pe.py:343)
+struct ValueHead {
+    const float* raw;         // [E, N, ld], value in column 0
+    int E, ld;
+    const float *mu_out, *sig_out;   // [1] or null
+};
+
+__device__ __forceinline__ float value_of(const ValueHead& h, int64_t N, int64_t p) {
+    // tf.reduce_mean over members of inverse_transform(out) (pe.py:343, pens/utils.py:167)
+    float s = 0.f;
+    for (int e = 0; e < h.E; ++e) {
+        float m = h.raw[((int64_t)e * N + p) * h.ld];
+        if (h.mu_out) m = __fadd_rn(__fmul_rn(h.sig_out[0], m), h.mu_out[0]);
+        s = (e == 0) ? m : __fadd_rn(s, m);
+    }
+    return __fdiv_rn(s, (float)h.E);
+}
 
 struct PolicyRowsArgs {
     int64_t N;                 // rows
@@ -209,6 +225,55 @@ __global__ void __launch_bounds__(ROW_THREADS, 4) env_step_kernel(EnvStepArgs a)
 
 __global__ void finish_mean_kernel(const double* sum, int64_t n, float* out) {
     if (threadIdx.x == 0 && blockIdx.x == 0) out[0] = (float)(sum[0] / (double)n);
+}
+
+// ---- what a step does with one fed row once FakeEnv.step's outputs are known ---------------------
+// sampler rules model_sampler.py:275-367 + ModelBuffer.store_multiple (modelbuffer.py:114-135)
+struct StepRules {
+    int64_t B; int t, last_storable;          // last_storable = T-2: storing it ends the path (horizon)
+    int uncertainty; double dkl_lim;
+    int no_store;                             // CMBPO_ROLLOUT_NO_STORE: per-path results and statistics only
+    uint8_t* alive;                           // [B] by path
+    uint8_t* pending;                         // [B] by path: bit0 last_val, bit1 last_cval wanted from the next policy pass
+    cmbpo_rollout_bufs b;
+};
+
+struct RowCarry { float v, vc, logp; double dkl, ret, cost; };
+
+// returns 1 = the step was stored, 2 = the path was cut as too uncertain BEFORE the store.
+// st[0..3] += rows fed, sum dkl, rows stored, sum ep_var  (the caller reduces them per step)
+__device__ __forceinline__ int step_row_commit(const StepRules& a, int64_t p, const EnvRowOut& o, const RowCarry& pf,
+                                               double& st0, double& st1, double& st2, double& st3) {
+    const float v = pf.v, vc = pf.vc;
+    // uncertainty cut-off BEFORE the step is stored (model_sampler.py:275-290)
+    const double next_dkl = pf.dkl + (double)o.dkl_path;
+    const bool cut = a.uncertainty && next_dkl >= a.dkl_lim;
+    st0 += 1.0; st1 += (double)o.dkl_path;
+    if (cut) {
+        a.alive[p] = 0;
+        a.b.end_reason[p] = CMBPO_END_UNCERTAIN;
+        a.b.last_val[p] = v; a.b.last_cval[p] = vc;      // V(s_t), VC(s_t): model_sampler.py:401-407
+        return 2;
+    }
+    const int t = a.t;
+    if (!a.no_store) {
+        const int64_t row = (int64_t)t * a.B + p;      // ModelBuffer.store_multiple, time-major
+        a.b.rew[row] = o.rew; a.b.val[row] = v; a.b.cost[row] = o.cost; a.b.cval[row] = vc;
+        a.b.logp[row] = pf.logp; a.b.dyn_error[row] = o.ep_var_mean; a.b.dkl[row] = o.dkl_path;
+        a.b.term[row] = o.term ? 1 : 0;
+    }
+    a.b.length[p] = t + 1;
+    a.b.cum_dkl[p] = next_dkl;                        // model_sampler.py:332
+    a.b.path_return[p] = pf.ret + (double)o.rew;      // :317-318
+    a.b.path_cost[p] = pf.cost + (double)o.cost;
+    st2 += 1.0; st3 += (double)o.ep_var_sum;
+    if (t >= a.last_storable) {                       // path_length >= max_path_length-1 (:352)
+        a.alive[p] = 0; a.b.end_reason[p] = CMBPO_END_HORIZON; a.pending[p] = 3;
+    } else if (o.term) {                              // env terminal (:357-364)
+        a.alive[p] = 0; a.b.end_reason[p] = CMBPO_END_TERMINAL;
+        a.b.last_val[p] = 0.f; a.pending[p] = 2;
+    }
+    return 1;
 }
 
 // ---- rollout step ------------------------------------------------------------------------
@@ -588,23 +653,6 @@ extern "C" int cmbpo_rollout(cmbpo_ctx* ctx, const cmbpo_rollout_cfg* cfg, const
                             (cfg->uncertainty_mode || cfg->env.term_id != CMBPO_TERM_NO_DONE);
     int cur_gen = 0;
     const int compact_every = cfg->compact_every > 0 ? cfg->compact_every : 2;    // measured: 2 beats 1 and 4 by 2-6 %
-    // Fused step (tcgen05 precisions, opt-in with CMBPO_ROLLOUT_FUSE): policy head in the dynamics kernel's
-    // input staging, FakeEnv row math / sampler rules / ModelBuffer write-out in its epilogue -> two launches per
-    // step, and the raw [E,B,2D] outputs only exist tile by tile in an L2-resident scratch.  Opt-in because the
-    // row math then runs on the GEMM kernel's epilogue warps with the tensor pipe idle: measured 24.6 ms against
-    // 21.9 ms per 100 k x 34-step rollout for the four-launch step.
-    const int rp_shift = ens_tc_fused_rp_shift(O);
-    const bool fused = cfg->precision != CMBPO_PREC_FP32 && (cfg->flags & CMBPO_ROLLOUT_FUSE) && ctx->polnet.loaded &&
-                       ens_tc_fusable(dyn) && rp_shift >= 5 && dyn.n_elite <= 8 && A <= CMBPO_MAX_ACT;
-    const int64_t ntiles = (B + 127) / 128;
-    int* tile_cnt = nullptr;
-    float* pol_raw = nullptr;
-    if (fused) {
-        if (cmbpo_ws_get(ctx, 7, (size_t)ntiles * sizeof(int), (void**)&tile_cnt)) return 1;
-        CUDA_TRY(cudaMemsetAsync(tile_cnt, 0, (size_t)ntiles * sizeof(int), ctx->stream));
-        if (cmbpo_ws_get(ctx, 2, (size_t)ntiles * 128 * dyn.E * 2 * dyn.D * sizeof(float), (void**)&raw)) return 1;
-        if (cmbpo_ws_get(ctx, 3, (size_t)ctx->polnet.E * B * A * sizeof(float), (void**)&pol_raw)) return 1;
-    } else
     if (cmbpo_ws_get(ctx, 2, (size_t)dyn.E * B * 2 * dyn.D * sizeof(float), (void**)&raw)) return 1;
 
     CUDA_TRY(cudaMemsetAsync(bufs->step_stats, 0, (size_t)T * 4 * sizeof(double), ctx->stream));
@@ -631,35 +679,6 @@ extern "C" int cmbpo_rollout(cmbpo_ctx* ctx, const cmbpo_rollout_cfg* cfg, const
             CUDA_TRY(cudaEventSynchronize(ctx->n_ev[slot]));
             if (ctx->host_n[slot] == 0) break;                 // nothing alive, nothing pending
         }
-        if (fused && !last) {
-            const int64_t* nd = compacting ? n_dev + cur_gen : nullptr;
-            {
-                ProfScope prof(ctx, CMBPO_PROF_POLICY);
-                if (ens_forward(ctx, ctx->polnet, cur, B, false, pol_raw, cfg->precision, nd)) return 1;
-            }
-            FusedStep fz = {};
-            fz.rules.B = B; fz.rules.t = t; fz.rules.last_storable = T - 2;
-            fz.rules.uncertainty = cfg->uncertainty_mode; fz.rules.dkl_lim = cfg->dkl_lim;
-            fz.rules.alive = alive; fz.rules.pending = pending; fz.rules.b = *bufs;
-            fz.rules.no_store = (cfg->flags & CMBPO_ROLLOUT_NO_STORE) ? 1 : 0;
-            fz.O = O; fz.A = A; fz.n_elite = dyn.n_elite;
-            fz.c = make_env_cfg(dyn, cfg->env, O, cfg->precision);
-            fz.path_base = cfg->path_id_base; fz.seed = cfg->seed;
-            fz.cur_obs = cur; fz.pol_raw = pol_raw;
-            fz.v = make_head(ctx->nets[CMBPO_NET_V], pol_raw + (size_t)B * A); fz.v.ld = A;
-            fz.vc = make_head(ctx->nets[CMBPO_NET_VC], pol_raw + (size_t)(1 + ctx->nets[CMBPO_NET_V].E) * B * A); fz.vc.ld = A;
-            fz.log_std = ctx->log_std;
-            fz.pi = pi; fz.mu = mu; fz.logp = logp; fz.vrow = v; fz.vcrow = vc;
-            fz.act_eps = bufs->act_eps ? bufs->act_eps + (size_t)t * B * A : nullptr;
-            fz.elite_pos = bufs->elite_pos ? bufs->elite_pos + (size_t)t * B : nullptr;
-            fz.state_eps = bufs->state_eps ? bufs->state_eps + (size_t)t * B * O : nullptr;
-            fz.row_path = compacting ? row_path[cur_gen] : nullptr;
-            fz.raw_tiles = raw; fz.tile_cnt = tile_cnt; fz.rp_shift = rp_shift;
-            {
-                ProfScope prof(ctx, CMBPO_PROF_DYN);
-                if (ens_forward_tc(ctx, dyn, nullptr, B, nullptr, cfg->precision, nd, &fz)) return 1;
-            }
-        } else {
         PolicyRowsArgs pa = {};
         pa.N = B; pa.O = O; pa.A = A; pa.obs = cur;
         pa.row_path = compacting ? row_path[cur_gen] : nullptr;
@@ -702,7 +721,6 @@ extern "C" int cmbpo_rollout(cmbpo_ctx* ctx, const cmbpo_rollout_cfg* cfg, const
             kern<<<(unsigned)std::min<int64_t>(cdiv(B, step_rows(O)), (int64_t)ctx->sm_count * 64), STEP_THREADS, smem, ctx->stream>>>(sa);
         }
         ctx->launches++;
-        }   // step-wise path
         if (compacting && (t % compact_every) == compact_every - 1 && t + 1 < n_steps) {
             compact_flags_kernel<<<cdiv(B, 256), 256, 0, ctx->stream>>>(B, row_path[cur_gen], n_dev + cur_gen, alive, pending, cflags);
             ctx->launches++;

@@ -1,6 +1,6 @@
-// Per-row arithmetic of the rollout step, shared by the fp32 CUDA-core path and the fused
-// tcgen05 path so that both apply exactly the same logic (the precision of the GEMM chain is
-// the only thing that differs between them).
+// Per-row arithmetic of the rollout step and of the single FakeEnv step (rollout.cu).  The fp32 and
+// the tensor-core precision modes run the same code; the FAST template argument selects the
+// tensor-core modes' approximate divisions and closed-form KL.
 //
 // Everything here follows the reference's op order in float32 without FMA contraction
 // (__fmul_rn / __fadd_rn), because numpy/TF evaluate these expressions one ufunc at a time.
@@ -64,25 +64,23 @@ __device__ inline int philox_elite_pos(uint64_t seed, int64_t path, int step, in
 // numpy's float32 pairwise sum for n < 128 elements (np.mean over the last axis):
 // 8 running partial sums, a fixed combination tree, then the n%8 tail added sequentially.
 // ------------------------------------------------------------------------------------------
-// Element i at a[i * stride]: stride 1 for the row kernels' [row][dim] staging, the rows per pass
-// for the fused step kernel's [dim][row] staging.
-__device__ inline float np_sum_strided(const float* a, int n, int stride) {
+__device__ inline float np_sum(const float* a, int n) {
     if (n < 8) {
         float s = 0.f;
-        for (int i = 0; i < n; ++i) s = __fadd_rn(s, a[i * stride]);
+        for (int i = 0; i < n; ++i) s = __fadd_rn(s, a[i]);
         return s;
     }
     float r[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) r[j] = a[j * stride];
+    for (int j = 0; j < 8; ++j) r[j] = a[j];
     int i = 8;
     for (; i < n - (n & 7); i += 8) {
 #pragma unroll
-        for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], a[(i + j) * stride]);
+        for (int j = 0; j < 8; ++j) r[j] = __fadd_rn(r[j], a[i + j]);
     }
     float s = __fadd_rn(__fadd_rn(__fadd_rn(r[0], r[1]), __fadd_rn(r[2], r[3])),
                         __fadd_rn(__fadd_rn(r[4], r[5]), __fadd_rn(r[6], r[7])));
-    for (; i < n; ++i) s = __fadd_rn(s, a[i * stride]);
+    for (; i < n; ++i) s = __fadd_rn(s, a[i]);
     return s;
 }
 
@@ -137,7 +135,7 @@ struct EnvRowOut {
 // ------------------------------------------------------------------------------------------
 // One action dimension: pi = mu + eps * exp(log_std) (ac_network.py:109) and its log-likelihood term
 // (ac_network.py:47).  FAST (tensor-core precision modes): approximate division (2 ulp) -- the IEEE
-// division is a subroutine call, which the fused tcgen05 kernel cannot afford in its epilogue warps.
+// division is a subroutine call per use.
 template <bool FAST>
 __device__ __forceinline__ float actor_dim(float mu, float ls, float eps, float& pi) {
     const float log2pi = 1.8378770664093453f;   // float32(np.log(2*np.pi))
@@ -261,28 +259,17 @@ __device__ __forceinline__ EnvDimOut env_dim(const EnvRowCfg& c, Raw raw, int o,
     return out;
 }
 
-// next state of ONE dimension from the chosen member only -- the same operations, in the same order,
-// as the `sel` / `nx` values of env_dim (the fused step kernel recomputes it at write-out time instead
-// of staging all of next_obs)
+// row-owner part: ordered reductions over the O dimensions (numpy order), statics, reward
 template <bool FAST, class Raw>
-__device__ __forceinline__ float env_dim_nx(const EnvRowCfg& c, Raw raw, int o, int member, float obs_o, float eps) {
-    const float mean = __fadd_rn(__fmul_rn(c.sig_out[o], raw(member, o)), c.mu_out[o]);
-    float x = mean;
-    if (!c.deterministic) {
-        const float logvar = __fadd_rn(c.l2s_out[o], raw(member, c.D + o));
-        const float var = FAST ? __expf(logvar) : expf(logvar);
-        const float sd = FAST ? ((var > 0.f && !isinf(var)) ? __fmul_rn(var, rsqrtf(var)) : var) : sqrtf(var);
-        x = __fadd_rn(mean, __fmul_rn(sd, eps));
-    }
-    return c.predicts_delta ? __fadd_rn(x, obs_o) : x;
-}
-
-// row-owner part: statics and reward from the reduced sums and the few next-state coordinates the
-// statics read (z = nx[0], q1 = nx[2], q2 = nx[3], last = nx[O-1])
-template <bool FAST, class Raw>
-__device__ __forceinline__ EnvRowOut env_row_core(const EnvRowCfg& c, Raw raw, int member, float ks, float es,
-                                                  bool all_finite, float z, float q1, float q2, float last) {
+__device__ inline EnvRowOut env_row_finish(const EnvRowCfg& c, Raw raw, int member, const float* kl,
+                                           const float* epv, const float* nx, const unsigned char* fin) {
     const int O = c.O;
+    const float ks = np_sum(kl, O);
+    const float es = np_sum(epv, O);
+    bool all_finite = true;
+    for (int o = 0; o < O; ++o) all_finite = all_finite && fin[o];
+    // the next-state coordinates the statics read
+    const float z = nx[0], q1 = O > 2 ? nx[2] : 0.f, q2 = O > 3 ? nx[3] : 0.f, last = nx[O - 1];
     EnvRowOut r;
     r.dkl_path = FAST ? __fdividef(ks, (float)O) : __fdiv_rn(ks, (float)O);      // fake_env.py:113
     r.ep_var_sum = es;
@@ -308,17 +295,4 @@ __device__ __forceinline__ EnvRowOut env_row_core(const EnvRowCfg& c, Raw raw, i
     }
     r.rew = __fadd_rn(__fmul_rn(c.sig_out[rcol], raw(member, rcol)), c.mu_out[rcol]);   // :148-151
     return r;
-}
-
-// ordered reductions over the O dimensions (numpy order) from per-dimension arrays, then the core
-template <bool FAST, class Raw>
-__device__ inline EnvRowOut env_row_finish(const EnvRowCfg& c, Raw raw, int member, const float* kl,
-                                           const float* epv, const float* nx, const unsigned char* fin) {
-    const int O = c.O;
-    const float ks = np_sum_strided(kl, O, 1);
-    const float es = np_sum_strided(epv, O, 1);
-    bool all_finite = true;
-    for (int o = 0; o < O; ++o) all_finite = all_finite && fin[o];
-    return env_row_core<FAST>(c, raw, member, ks, es, all_finite, nx[0], O > 2 ? nx[2] : 0.f, O > 3 ? nx[3] : 0.f,
-                              nx[O - 1]);
 }

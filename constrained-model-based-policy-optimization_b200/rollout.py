@@ -65,7 +65,7 @@ class RolloutBuffers:
     def run(self, env_cfg, uncertainty_mode=False, dkl_lim=0.0, seed=0, path_id_base=0,
             max_steps=0, precision=None, flags=0, compact_every=0):
         """cmbpo_rollout: the speculative per-path rollout.  `flags`: L.ROLLOUT_* bits (results do not
-        depend on NO_COMPACT / FUSE; NO_STORE leaves the per-step fields untouched)."""
+        depend on NO_COMPACT; FUSE is retired and ignored; NO_STORE leaves the per-step fields untouched)."""
         e = self.engine
         if self.lean:
             flags = int(flags) | L.ROLLOUT_NO_STORE

@@ -187,12 +187,7 @@ typedef struct {
 
 /* cmbpo_rollout_cfg.flags.  None of them changes a result bit (tests compare both settings):
  *   NO_COMPACT  keep finished paths' rows in the batch (see below);
- *   FUSE        tensor-core precisions: run the step as TWO launches -- the policy GEMM, and the dynamics
- *               GEMM kernel with the policy head in its input staging and the FakeEnv row math / sampler
- *               rules / ModelBuffer write-out in its epilogue (raw outputs only tile by tile in an
- *               L2-resident scratch) -- instead of the default four (policy GEMM, policy rows, dynamics
- *               GEMM with raw [E,B,2D] outputs in HBM, row kernel).  Bit-identical; opt-in because it is
- *               currently slower (the row math occupies the GEMM kernel's epilogue warps);
+ *   FUSE        retired and ignored: it selected a fused step that gave the same results as the default;
  *   NO_STORE    do not write the per-step ModelBuffer fields (obs .. term may then be NULL): only the
  *               per-path results and step_stats -- ModelSampler.compute_dynamics_dkl
  *               (samplers/model_sampler.py:151-167) = sum_t step_stats[t][1] / sum_t step_stats[t][0]. */

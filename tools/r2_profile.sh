@@ -11,7 +11,6 @@ fi
 timeout 600 python bench.py --steps 20 --warmup 3 > $O/${TAG}_bench.json 2> $O/${TAG}_bench.err; echo "bench rc=$?"
 if [ -z "$SKIP_CONFIGS" ]; then
 timeout 300 python bench.py --steps 10 --warmup 3 --mode injected --cpu-batch 0 --no-e2e > $O/${TAG}_bench_injected.json 2> $O/${TAG}_bench_injected.err; echo "injected rc=$?"
-timeout 300 python bench.py --steps 10 --warmup 3 --fuse --cpu-batch 0 --no-e2e > $O/${TAG}_bench_fused.json 2> $O/${TAG}_bench_fused.err; echo "fused rc=$?"
 timeout 300 python bench.py --config hs_gae --steps 10 --warmup 3 > $O/${TAG}_bench_hs_gae.json 2> $O/${TAG}_bench_hs_gae.err; echo "hs_gae rc=$?"
 timeout 400 python bench.py --config ant1m --steps 5 --warmup 2 > $O/${TAG}_bench_ant1m.json 2> $O/${TAG}_bench_ant1m.err; echo "ant1m rc=$?"
 timeout 900 python bench.py --config sweep --steps 3 --warmup 1 > $O/${TAG}_bench_sweep.json 2> $O/${TAG}_bench_sweep.err; echo "sweep rc=$?"
