@@ -80,6 +80,7 @@ SIGNATURES = {
     "cmbpo_archive_index": (_i, [_vp, _vp, _i64, _i, _vp, _vp, C.POINTER(C.c_int64)]),
     "cmbpo_archive_sample_epochs": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _u64, _u64, _vp]),
     "cmbpo_archive_sample_boltz": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64, _u64, _u64, _vp]),
+    "cmbpo_archive_sample_boltz_range": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64, _i64, _u64, _u64, _vp]),
     "cmbpo_gather_rows": (_i, [_vp, _vp, _i, _vp, _i64, _vp]),
     "cmbpo_policy_kl_epochs": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64, _i, C.POINTER(C.c_double)]),
     "cmbpo_rollout_diagnostics": (_i, [_vp, C.POINTER(RolloutBufs), _i64, _vp, _vp, C.POINTER(C.c_double)]),

@@ -109,6 +109,8 @@ class DeviceArchive:
         src = getattr(self, field)
         flat = idx.reshape(-1)
         dst = e.empty(flat.numel(), src.shape[1])
+        if flat.numel() == 0:                 # an empty shard: nothing to launch (and NULL pointers)
+            return dst
         L.check(e.lib.cmbpo_gather_rows(e.h, e._p(src), src.shape[1], e._p(flat), flat.numel(), e._p(dst)))
         return dst
 
@@ -145,9 +147,13 @@ class DeviceArchive:
         return np.where(ep >= 0, sample_p[ep], 0)
 
     # ---- distributed_batch_from_archive (cpobuffer.py:413-463) -----------------------------------
-    def distributed_batch_indices(self, batch_size, kls, alpha=1):
-        """Row numbers [batch_size]: row r with probability boltz_dist(kls, alpha)[r]."""
+    def distributed_batch_indices(self, batch_size, kls, alpha=1, shard=None):
+        """Row numbers [batch_size]: row r with probability boltz_dist(kls, alpha)[r].  `shard=(lo, hi)`:
+        only entries lo:hi of that batch (the same draw counter advances either way)."""
         e, t = self.engine, self.engine.torch
+        lo, hi = (0, int(batch_size)) if shard is None else (int(shard[0]), int(shard[1]))
+        if not 0 <= lo <= hi <= int(batch_size):
+            raise L.CmbpoError("shard %r is not inside a batch of %d" % (shard, batch_size))
         sorted_idx, offs, _ = self._build_index()
         eps = self.epochs_list
         _, sample_p = self.boltz_epoch_probs(kls, alpha)
@@ -156,18 +162,28 @@ class DeviceArchive:
         mass = sample_p[eps].astype(np.float64) * self.epoch_counts[eps]
         cdf = np.cumsum(mass)
         cdf /= cdf[-1]
-        out = e.zeros(int(batch_size), dtype=t.int32)
+        out = e.zeros(hi - lo, dtype=t.int32)
         eps_d = e.to_device(eps.astype(np.int32), t.int32)      # named: must outlive the launch
         cdf_d = e.to_device(cdf, t.float64)
-        L.check(e.lib.cmbpo_archive_sample_boltz(e.h, e._p(sorted_idx), e._p(offs), e._p(eps_d), e._p(cdf_d),
-                                                 len(eps), int(batch_size), self.seed, self._next_draw(),
-                                                 e._p(out)))
+        L.check(e.lib.cmbpo_archive_sample_boltz_range(e.h, e._p(sorted_idx), e._p(offs), e._p(eps_d), e._p(cdf_d),
+                                                       len(eps), lo, hi - lo, self.seed, self._next_draw(),
+                                                       e._p(out)))
         return out
 
-    def sample_start_states(self, policy, batch_size, alpha=1, precision=None):
+    def sample_start_states(self, policy, batch_size, alpha=1, precision=None, shard=None, group=None):
         """algorithms/cmbpo.py:241-245 in one call.  Returns a dict of DEVICE tensors
-        (observations [B,O], mu, log_std [B,A]) and the clipped per-epoch KLs (numpy)."""
+        (observations [B,O], mu, log_std [B,A]) and the clipped per-epoch KLs (numpy).
+
+        `shard=(lo, hi)`: rows lo:hi of what the call without `shard` returns (`batch_size` stays the
+        whole batch).  Several ranks that hold the same archive and call this in step each get their block
+        of one batch: every rank computes the per-epoch KLs, and when torch.distributed runs more than one
+        rank in `group`, all of them use rank 0's (all-gathered), so that every rank draws from the same
+        distribution bit for bit."""
         kls = np.clip(self.epoch_kls(policy, batch_size, precision=precision), a_min=0, a_max=None)
-        idx = self.distributed_batch_indices(batch_size, kls, alpha)
+        if shard is not None:
+            from .dist import all_gather_host, is_multi_rank
+            if is_multi_rank(group):
+                kls = all_gather_host(kls, group, self.engine.device)[0]
+        idx = self.distributed_batch_indices(batch_size, kls, alpha, shard)
         return dict(observations=self.gather("observations", idx), mu=self.gather("mu", idx),
                     log_std=self.gather("log_std", idx), kls=kls, indices=idx)

@@ -118,12 +118,16 @@ __global__ void archive_sample_epochs_kernel(const int32_t* __restrict__ sorted_
     out[i] = cnt > 0 ? sorted_idx[lo + (int64_t)(((uint64_t)u * (uint64_t)cnt) >> 32)] : -1;
 }
 
-// rows with probability p(epoch) / count(epoch): epoch by inverse CDF, then a uniform row of it
+// rows with probability p(epoch) / count(epoch): epoch by inverse CDF, then a uniform row of it.  Samples
+// [first, first + count) of a batch: sample i depends on (seed, draw, i) only, never on the batch size, so a
+// shard writes exactly the rows the whole batch has at those positions
 __global__ void archive_sample_boltz_kernel(const int32_t* __restrict__ sorted_idx, const int64_t* __restrict__ bin_offsets,
                                             const int32_t* __restrict__ epochs, const double* __restrict__ cdf, int n_ep,
-                                            int64_t B, uint64_t seed, uint64_t draw, int32_t* __restrict__ out) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= B) return;
+                                            int64_t first, int64_t count, uint64_t seed, uint64_t draw,
+                                            int32_t* __restrict__ out) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= count) return;
+    const int64_t i = first + j;
     uint32_t o[4];
     philox4x32_10((uint32_t)i, (uint32_t)((uint64_t)i >> 32), (uint32_t)draw, ((uint32_t)(RNG_STREAM_ARCHIVE + 1) << 16) | (uint32_t)(draw >> 32),
                   (uint32_t)seed, (uint32_t)(seed >> 32), o);
@@ -135,7 +139,7 @@ __global__ void archive_sample_boltz_kernel(const int32_t* __restrict__ sorted_i
         if (cdf[mid] > u) hi = mid; else lo = mid + 1;
     }
     const int64_t start = bin_offsets[epochs[lo]], cnt = bin_offsets[epochs[lo] + 1] - start;
-    out[i] = cnt > 0 ? sorted_idx[start + (int64_t)(((uint64_t)o[2] * (uint64_t)cnt) >> 32)] : -1;
+    out[j] = cnt > 0 ? sorted_idx[start + (int64_t)(((uint64_t)o[2] * (uint64_t)cnt) >> 32)] : -1;
 }
 
 __global__ void gather_rows_kernel(const float* __restrict__ src, int width, const int32_t* __restrict__ idx, int64_t n,
@@ -217,10 +221,19 @@ extern "C" int cmbpo_archive_sample_epochs(cmbpo_ctx* ctx, const int32_t* sorted
 extern "C" int cmbpo_archive_sample_boltz(cmbpo_ctx* ctx, const int32_t* sorted_idx, const int64_t* bin_offsets,
                                           const int32_t* epochs, const double* cdf, int n_ep, int64_t B,
                                           uint64_t seed, uint64_t draw, int32_t* out_idx) {
-    CMBPO_CHECK(ctx && sorted_idx && bin_offsets && epochs && cdf && out_idx, "null argument");
+    return cmbpo_archive_sample_boltz_range(ctx, sorted_idx, bin_offsets, epochs, cdf, n_ep, 0, B, seed, draw, out_idx);
+}
+
+extern "C" int cmbpo_archive_sample_boltz_range(cmbpo_ctx* ctx, const int32_t* sorted_idx, const int64_t* bin_offsets,
+                                                const int32_t* epochs, const double* cdf, int n_ep, int64_t first,
+                                                int64_t count, uint64_t seed, uint64_t draw, int32_t* out_idx) {
+    // an empty shard may pass out_idx = NULL (torch's pointer of an empty tensor)
+    CMBPO_CHECK(ctx && sorted_idx && bin_offsets && epochs && cdf && (out_idx || count == 0), "null argument");
     CMBPO_CHECK(n_ep > 0, "no epochs to sample from");
-    if (B == 0) return 0;
-    archive_sample_boltz_kernel<<<cdiv(B, 256), 256, 0, ctx->stream>>>(sorted_idx, bin_offsets, epochs, cdf, n_ep, B, seed, draw, out_idx);
+    CMBPO_CHECK(first >= 0 && count >= 0, "sample range [%lld, +%lld) out of range", (long long)first, (long long)count);
+    if (count == 0) return 0;
+    archive_sample_boltz_kernel<<<cdiv(count, 256), 256, 0, ctx->stream>>>(sorted_idx, bin_offsets, epochs, cdf, n_ep,
+                                                                         first, count, seed, draw, out_idx);
     ctx->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;

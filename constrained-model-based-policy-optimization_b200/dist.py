@@ -1,11 +1,13 @@
-"""Multi-GPU plumbing of the rollout path: contiguous sharding of start states and the two
-Allreduce steps of `mpi_statistics_scalar` (utilities/mpi_tools.py:71-92).
+"""Multi-GPU plumbing of the rollout path: contiguous sharding of start states, the two
+Allreduce steps of `mpi_statistics_scalar` (utilities/mpi_tools.py:71-92) and the batch-wide
+rules of a sharded rollout block (`ModelSampler.distribute`).
 
-Paths are independent units, so there is no data-path collective: every rank rolls out its own
-block of start states (Philox counters use GLOBAL path ids, so results do not depend on the
-sharding), and only the five running sums (n, sum adv, sum cadv, sum ret, sum cret) and then the
-sum of squared deviations cross ranks.  One process per GPU, `torch.distributed` (NCCL on GPUs,
-gloo in the CPU tests).
+Paths are independent units: every rank rolls out its own block of start states (Philox counters
+use GLOBAL path ids, so results do not depend on the sharding).  Across ranks go the five running
+sums (n, sum adv, sum cadv, sum ret, sum cret) and then the sum of squared deviations; with
+`ModelSampler.distribute`, also small all-gathers of counts and sums (shard sizes, length histograms,
+per-step statistics, diagnostics) and, in `ModelBuffer.get`, the populated rows to one rank.
+One process per GPU, `torch.distributed` (NCCL on GPUs, gloo in the CPU tests).
 """
 import numpy as np
 
@@ -27,6 +29,46 @@ def make_reduce_fn(group=None):
         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
         return t
     return reduce_fn
+
+
+def is_multi_rank(group=None):
+    import torch.distributed as dist
+    return dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+
+
+def all_gather_host(vec, group=None, device=None):
+    """All-gather of a small numpy vector of the same shape on every rank -> numpy [world, ...] in rank
+    order.  `device`: where the collective runs (the rank's GPU for NCCL; the host for gloo)."""
+    import torch
+    import torch.distributed as dist
+    if dist.get_backend(group) != "nccl":
+        device = "cpu"
+    a = np.ascontiguousarray(vec)
+    x = torch.from_numpy(a.reshape(-1)).to(device)
+    out = torch.empty(dist.get_world_size(group) * x.numel(), dtype=x.dtype, device=x.device)
+    dist.all_gather_into_tensor(out, x, group=group)
+    return out.cpu().numpy().reshape((-1,) + a.shape)
+
+
+def rank_order_sum(gathered):
+    """Sum of the rows of an all-gathered [world, ...] array, rank 0 first.  Every rank adds the same
+    numbers in the same order, so float sums are bit-identical on every rank (an all-reduce does not
+    promise that)."""
+    acc = gathered[0].copy()
+    for row in gathered[1:]:
+        acc = acc + row
+    return acc
+
+
+def cap_split(n, survivors):
+    """The max_samples cap of a sharded batch: the reference cuts the first n surviving paths of the whole
+    batch by path index.  Shards are contiguous in path order, so rank r cuts its first
+    clamp(n - sum_{g<r} s_g, 0, s_r) survivors, where s_g = survivors of rank g.  Returns the per-rank cuts."""
+    cuts, before = [], 0
+    for s in survivors:
+        cuts.append(int(min(max(int(n) - before, 0), int(s))))
+        before += int(s)
+    return cuts
 
 
 def combine_pass1(sums):

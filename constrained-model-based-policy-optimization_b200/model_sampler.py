@@ -15,6 +15,7 @@ from collections import OrderedDict
 import numpy as np
 
 from . import _lib as L
+from .dist import all_gather_host, cap_split, rank_order_sum
 from .fake_env import FakeEnv
 from .policy import B200Policy
 
@@ -39,6 +40,9 @@ class ModelSampler:
         self.injected = None          # tests: dict(act_eps=[T,B,A], elite_pos=[T,B], state_eps=...)
         self.path_id_base = 0         # multi-GPU: global id of this rank's first path
         self.return_arrays = False
+        self._dist = None             # distribute(): (group, rank) of a sharded rollout block
+        self._batch_total = batch_size
+        self._global_sums = None
 
     # ---- plumbing identical to the reference ------------------------------------------------
     def initialize(self, env, policy, pool):
@@ -71,10 +75,44 @@ class ModelSampler:
         return (isinstance(self.policy, B200Policy) and isinstance(self.env, FakeEnv)
                 and self.policy.engine is self.env.engine)
 
+    # ---- multi-GPU ---------------------------------------------------------------------------
+    def distribute(self, group=None, root=0):
+        """Run the rollout block sharded over the ranks of `group` (torch.distributed, one process per
+        GPU) with the samples one GPU gives.  Every rank calls reset() with its contiguous block of the
+        start states, in rank order (DeviceArchive.sample_start_states(shard=...)).  The batch-wide
+        rules -- the max_samples cap, the sample count and alive ratio the caller stops on,
+        compute_dynamics_dkl and the finish_all_paths() diagnostics -- then use counts and sums over all
+        ranks and are identical on every rank, and the pool's get() returns the whole batch on rank
+        `root` (zero rows elsewhere).  Fused mode only; call after initialize()."""
+        import torch.distributed as dist
+        if not (dist.is_available() and dist.is_initialized()):
+            raise L.CmbpoError("ModelSampler.distribute needs an initialised torch.distributed process group")
+        if not self.fused:
+            raise L.CmbpoError("a multi-rank ModelSampler needs the fused mode (a B200Policy and a FakeEnv of "
+                               "one Engine); the step-wise mode runs on one rank only")
+        self._dist = dict(group=group, rank=dist.get_rank(group))
+        self._auto_base = self.path_id_base
+        self.pool.distribute(group, root)
+
+    def _gather(self, vec):
+        """[world, ...] all-gather of a small host vector, rank order."""
+        return all_gather_host(vec, self._dist["group"], self.pool.engine.device)
+
+    def _shard_base(self, n):
+        """(global id of this rank's first path, global path count) from the ranks' shard sizes."""
+        sizes = self._gather(np.array([n], np.int64))[:, 0]
+        base = int(sizes[:self._dist["rank"]].sum())
+        if self.path_id_base not in (self._auto_base, base):
+            raise L.CmbpoError("path_id_base %d was set by hand, but the shard sizes put this rank's first path "
+                               "at %d" % (self.path_id_base, base))
+        self.path_id_base = self._auto_base = base
+        return base, int(sizes.sum())
+
     # ---- calibration (model_sampler.py:151-167) ----------------------------------------------
     def compute_dynamics_dkl(self, obs_batch, depth=1):
         if self.fused:
             return self._dynamics_dkl_device(obs_batch, depth)
+        self._require_fused_if_distributed()
         for _ in range(depth):
             outs = self.policy.get_action_outs(obs_batch)
             next_obs, _, terminal, info = self.env.step(obs_batch, outs["pi"])
@@ -100,20 +138,35 @@ class ModelSampler:
         inj = self.injected or {}
         bufs.set_inputs(obs, inj.get("act_eps"), inj.get("elite_pos"), inj.get("state_eps"))
         self._dkl_calls = getattr(self, "_dkl_calls", 0) + 1
+        if self._dist is not None:        # obs_batch is this rank's block of the calibration batch
+            self._shard_base(obs.shape[0])
         bufs.run(env.env_cfg(True), uncertainty_mode=False, seed=(self.seed << 20) + (1 << 19) + self._dkl_calls,
                  path_id_base=self.path_id_base, max_steps=depth)
         st = bufs.step_stats.cpu().numpy()[:depth]
+        if self._dist is not None:
+            st = rank_order_sum(self._gather(np.ascontiguousarray(st[:, 0:2])))
         self._total_dkl += float(st[:, 1].sum())
         self._total_samples += int(st[:, 0].sum())
         return self.dyn_dkl * depth
 
     # ---- reset (model_sampler.py:203-237) ----------------------------------------------------
+    def _require_fused_if_distributed(self):
+        if self._dist is not None and not self.fused:
+            raise L.CmbpoError("a multi-rank ModelSampler runs the fused mode only: the step-wise mode "
+                               "(external policy objects) runs on one rank")
+
     def reset(self, observations):
+        """`observations`: the start states; after distribute(), this rank's contiguous block of them."""
         # a device tensor (DeviceArchive.sample_start_states) stays on the device in fused mode
         on_device = hasattr(observations, "is_cuda") and observations.is_cuda
         if not (on_device and self.fused):
             observations = np.asarray(observations.cpu() if on_device else observations, np.float32)
         self.batch_size = observations.shape[0]
+        self._batch_total = self.batch_size
+        self._global_sums = None
+        self._require_fused_if_distributed()
+        if self._dist is not None:
+            _, self._batch_total = self._shard_base(self.batch_size)
         self._current_observation = observations
         self.policy.reset()
         self.pool.reset(self.batch_size)
@@ -153,18 +206,32 @@ class ModelSampler:
         # (so a caller may prepare / finish another batch while this one runs)
         self._hist = None
         self._step_stats_host = None
-        self._alive_now = self.batch_size
+        self._alive_now = self._batch_total
         self._stopped = False
         self._horizon_steps = steps
 
     def _counts(self, t):
         """(rows alive at the start of step t, of which cut as too uncertain at t, survivors)."""
         if self._hist is None:                      # first use after reset(): waits for the rollout
-            self._hist = self.pool.bufs.histogram()
-            self._step_stats_host = self.pool.bufs.step_stats.cpu().numpy()
+            self._hist = self._histogram()
+            st = self.pool.bufs.step_stats.cpu().numpy()
+            if self._dist is not None:
+                st = rank_order_sum(self._gather(np.ascontiguousarray(st[:, 0:2])))
+            self._step_stats_host = st
         h_len, h_unc = self._hist
         longer = int(h_len[t + 1:].sum())
         return longer + int(h_unc[t]), int(h_unc[t]), longer
+
+    def _histogram(self):
+        """The length histograms of the batch (cmbpo_rollout_histogram); after distribute(), summed over the
+        ranks, with the ranks' own length histograms kept in self._rank_h_len for the cap split."""
+        h_len, h_unc = self.pool.bufs.histogram()
+        if self._dist is None:
+            return h_len, h_unc
+        g = self._gather(np.concatenate([h_len, h_unc]))
+        self._rank_h_len = g[:, :len(h_len)]
+        s = rank_order_sum(g)
+        return s[:len(h_len)], s[len(h_len):]
 
     def _sample_fused(self, max_samples):
         t = self._n_episodes
@@ -175,8 +242,13 @@ class ModelSampler:
             n = max(self._total_samples + alive0 - uncertain - max_samples, 0)
             n = min(n, survivors)
             if n > 0:
-                bufs.truncate(cap_step=t, cap_n=n)
-                self._hist = bufs.histogram()
+                if self._dist is None:
+                    cut = n
+                else:       # the first n survivors of the whole batch: this rank's share of them
+                    cut = cap_split(n, self._rank_h_len[:, t + 1:].sum(axis=1))[self._dist["rank"]]
+                if cut > 0:
+                    bufs.truncate(cap_step=t, cap_n=cut)
+                self._hist = self._histogram()
                 survivors -= n
         self._total_samples += survivors
         self.pool.ptr = t + 1 if survivors > 0 else self.pool.ptr
@@ -189,7 +261,7 @@ class ModelSampler:
         stats = self._step_stats_host[t]
         dkl_mean = stats[1] / stats[0] if stats[0] > 0 else 0.0
         info = {"ensemble_dkl_mean": np.float32(dkl_mean),
-                "alive_ratio": alive_after / self.batch_size if survivors > 0 else 0}
+                "alive_ratio": alive_after / self._batch_total if survivors > 0 else 0}
         self._total_dkl += dkl_mean * survivors
         if self.return_arrays:
             m = (bufs.length > t)
@@ -208,14 +280,25 @@ class ModelSampler:
         # model_sampler.py:314-333 and the sums of get_diagnostics (:89-133)
         B = bufs.B
         d = bufs.diagnostics()
-        self._total_rew, self._total_cost = d["rew"], d["cost"]
-        self._total_Vs, self._total_CVs = d["val"], d["cval"]
         self._path_return = bufs.path_return.cpu().numpy()
         self._path_cost = bufs.path_cost.cpu().numpy()
+        max_len = int(bufs.length.max().item()) if B else 0
+        if self._dist is not None:
+            # sums over the ranks in rank order, maxima over the ranks: the same dict on every rank
+            sums = ("rew", "cost", "val", "cval", "dyn_error", "n")
+            v = np.array([d[k] for k in sums] + [self.pool.size, self._path_return.sum(), self._path_cost.sum(),
+                                                 d["max_dkl"], d["max_path_return"], max_len], np.float64)
+            g = self._gather(v)
+            s, m = rank_order_sum(g), g.max(axis=0)
+            d.update(zip(sums, (float(x) for x in s[:6])))
+            self._global_sums = (int(s[6]), float(s[7]), float(s[8]))
+            d["max_dkl"], d["max_path_return"], max_len = float(m[9]), float(m[10]), int(m[11])
+        self._total_rew, self._total_cost = d["rew"], d["cost"]
+        self._total_Vs, self._total_CVs = d["val"], d["cval"]
         self._total_dyn_ep_var = d["dyn_error"] * bufs.O
         self._max_dkl = d["max_dkl"] if self._total_samples else 0
         self._max_path_return = max(0.0, d["max_path_return"]) if self._total_samples else 0
-        self.pool.ptr = int(bufs.length.max().item()) if B else 0
+        self.pool.ptr = max_len
 
     # ---- sample (model_sampler.py:239-375) ---------------------------------------------------
     def sample(self, max_samples=None):
@@ -224,6 +307,7 @@ class ModelSampler:
         if self.fused:
             assert self._alive_now > 0
             return self._sample_fused(max_samples)
+        self._require_fused_if_distributed()
         return self._sample_stepwise(max_samples)
 
     def _sample_stepwise(self, max_samples):
@@ -318,16 +402,20 @@ class ModelSampler:
     def get_diagnostics(self):
         """model_sampler.py:89-133 (keys and formulas)."""
         n = self._total_samples + EPS
-        d = OrderedDict({"pool-size": self.pool.size})
+        if self._global_sums is None:
+            size, ret_sum, cost_sum = self.pool.size, np.sum(self._path_return), np.sum(self._path_cost)
+        else:
+            size, ret_sum, cost_sum = self._global_sums
+        d = OrderedDict({"pool-size": size})
         d.update({
             "msampler/samples_added": self._total_samples,
             "msampler/rollout_H_max": self._n_episodes,
-            "msampler/rollout_H_mean": self._total_samples / (self.batch_size + EPS),
+            "msampler/rollout_H_mean": self._total_samples / (self._batch_total + EPS),
             "msampler/rew_var_perstep": 0 / n,
             "msampler/cost_var_perstep": 0 / n,
             "msampler/dyn_var_perstep": self._total_dyn_ep_var / n,
-            "msampler/cost_rate": np.sum(self._path_cost) / n,
-            "msampler/rew_rate": np.sum(self._path_return) / n,
+            "msampler/cost_rate": cost_sum / n,
+            "msampler/rew_rate": ret_sum / n,
             "msampler/v_mean": self._total_Vs / n,
             "msampler/cv_mean": self._total_CVs / n,
             "msampler/ens_DKL": self._total_dkl / n,

@@ -23,6 +23,7 @@ class ModelBuffer:
         self.pi_info_shapes = None
         self.gamma, self.lam, self.cost_gamma, self.cost_lam = 0.99, 0.95, 0.99, 0.95
         self.reduce_fn = None        # set by the multi-GPU wrapper: all-reduce of the statistics
+        self._dist = None            # distribute(): get() gathers the whole batch on one rank
         self.scan_mode = L.SCAN_STRICT
         self.reset()
 
@@ -143,6 +144,60 @@ class ModelBuffer:
         self.bufs.gae(self.gamma, self.lam, self.cost_gamma, self.cost_lam, scan=self.scan_mode)
         self.terminated_paths_mask[:] = True
 
+    # ---- multi-GPU ---------------------------------------------------------------------------
+    def distribute(self, group=None, root=0):
+        """Every rank of `group` holds a contiguous block of one batch's paths (rank order = path order):
+        the advantage statistics are all-reduced, and get() / get_device() return the rows of the WHOLE batch,
+        in global path order, on rank `root` (group rank) and arrays with zero rows on the other ranks.  The
+        diagnostics are the batch's on every rank.  Called by ModelSampler.distribute."""
+        import torch.distributed as dist
+        from .dist import make_reduce_fn
+        self.reduce_fn = make_reduce_fn(group)
+        self._dist = dict(group=group, root=int(root), rank=dist.get_rank(group))
+
+    def _gather_rows(self, fields, off, n_rows):
+        """The compacted `fields` ((field, width, vector) as get_device compacts them) of every rank, in rank
+        order, into fresh [N_total, ...] tensors on the root: the root compacts its own rows straight into its
+        slice of them; the other ranks compact into their persistent staging and send it; the root receives
+        straight into the final slices (one batch of point-to-point operations: no padding, no reassembly copy).
+        Over gloo (ranks that share a GPU) the messages are host copies.
+        Returns (the tensors -- zero rows off the root --, the row count of the whole batch)."""
+        import torch.distributed as dist
+        from .dist import all_gather_host
+        e, ds, b = self.engine, self._dist, self.bufs
+        group, root, rank = ds["group"], ds["root"], ds["rank"]
+        nccl = dist.get_backend(group) == "nccl"
+        landed = []                         # gloo: (device slice, host message)
+        counts = all_gather_host(np.array([n_rows], np.int64), group, e.device)[:, 0]
+        starts = np.concatenate([[0], np.cumsum(counts)])
+        n_out = int(starts[-1]) if rank == root else 0
+        out, ops = [], []
+        for i, (f, width, vector) in enumerate(fields):
+            def compact(dst):
+                return e.compact(f, self.batch_size, self.max_path_length, width, b.length, off, n_rows, dst)
+            if rank == root:
+                full = e.empty(n_out, width) if vector else e.empty(n_out)
+                compact(full[starts[rank]:starts[rank + 1]])
+                for g in range(len(counts)):
+                    if g != rank and counts[g]:
+                        dst = full[starts[g]:starts[g + 1]]
+                        msg = dst if nccl else e.torch.empty(dst.shape, dtype=dst.dtype)
+                        ops.append(dist.P2POp(dist.irecv, msg, group=group, group_peer=g))
+                        if not nccl:
+                            landed.append((dst, msg))
+            else:
+                full = e.empty(0, width) if vector else e.empty(0)
+                if n_rows:
+                    msg = compact(self._staging("send", i, n_rows, width, vector))
+                    ops.append(dist.P2POp(dist.isend, msg if nccl else msg.cpu(), group=group, group_peer=root))
+            out.append(full)
+        if ops:
+            for req in dist.batch_isend_irecv(ops):
+                req.wait()
+        for dst, msg in landed:
+            dst.copy_(msg)
+        return out, int(starts[-1])
+
     # ---- get ---------------------------------------------------------------------------------
     def _staging(self, gen, i, n_rows, width, vector):
         """Persistent compaction target (generation `gen`, field `i`), sized for a full buffer: no
@@ -174,17 +229,29 @@ class ModelBuffer:
         n_rows = int(off[-1].item())
         st = e.stats_from_sums(sums.cpu().numpy())
         O, A = self.obs_dim, self.act_dim
-        def tgt(i, width, vector):
-            return None if staging_gen is None else self._staging(staging_gen, i, n_rows, width, vector)
+        if self._dist is not None:
+            if staging_gen is not None:
+                raise L.CmbpoError("the persistent staging of get_async() is for one rank only; after "
+                                   "distribute() use get()")
+            vec, sc = (lambda f, w: (f, w, True)), (lambda f: (f, 1, False))
+            fields = [vec(b.obs, O), vec(b.act, A)] + [sc(f) for f in (b.adv, b.cadv, b.ret, b.cret, b.logp, b.val,
+                                                                       b.cval, b.cost)] + [vec(b.mu, A)]
+            full, n_rows = self._gather_rows(fields, off, n_rows)
+            out, mu = full[:10], full[10]
+            n_out = mu.shape[0]
+        else:
+            def tgt(i, width, vector):
+                return None if staging_gen is None else self._staging(staging_gen, i, n_rows, width, vector)
 
-        out = [e.compact(b.obs, B, T, O, b.length, off, n_rows, tgt(0, O, True)),
-               e.compact(b.act, B, T, A, b.length, off, n_rows, tgt(1, A, True))]
-        for i, f in enumerate((b.adv, b.cadv, b.ret, b.cret, b.logp, b.val, b.cval, b.cost)):
-            out.append(e.compact(f, B, T, 1, b.length, off, n_rows, tgt(2 + i, 1, False)))
-        mu = e.compact(b.mu, B, T, A, b.length, off, n_rows, tgt(11, A, True))
+            out = [e.compact(b.obs, B, T, O, b.length, off, n_rows, tgt(0, O, True)),
+                   e.compact(b.act, B, T, A, b.length, off, n_rows, tgt(1, A, True))]
+            for i, f in enumerate((b.adv, b.cadv, b.ret, b.cret, b.logp, b.val, b.cval, b.cost)):
+                out.append(e.compact(f, B, T, 1, b.length, off, n_rows, tgt(2 + i, 1, False)))
+            mu = e.compact(b.mu, B, T, A, b.length, off, n_rows, tgt(11, A, True))
+            n_out = n_rows
         ls_row = self._log_std_row if self._log_std_row is not None else np.zeros(A, np.float32)
         # every row of log_std is the same [A] variable (ac_network.py:119): a stride-0 view
-        log_std = e.to_device(ls_row, t.float32).reshape(1, A).expand(n_rows, A)
+        log_std = e.to_device(ls_row, t.float32).reshape(1, A).expand(n_out, A)
         out += [log_std, mu]                       # sorted pi_info keys: log_std, mu
         diag = dict(poolm_batch_size=n_rows, poolm_ret_mean=st["ret_mean"],
                     poolm_cret_mean=st["cret_mean"])
@@ -230,7 +297,9 @@ class ModelBuffer:
         concatenates their sample lists): statistics / normalisation / compaction run now on the
         engine's stream, the copies into page-locked buffers are queued on a side stream, the buffer
         resets.  Returns a handle whose `result()` waits for the copies and returns exactly what
-        `get()` returns.  At most two handles may be outstanding (two pinned buffer sets)."""
+        `get()` returns.  At most two handles may be outstanding (two pinned buffer sets).  One rank only."""
+        if self._dist is not None:
+            raise L.CmbpoError("get_async() runs on one rank only; after distribute() use get()")
         self._pin_gen = getattr(self, "_pin_gen", 0) ^ 1
         t, dev = self.engine.torch, self.engine.device
         # the staging / pinned buffers of this generation may still be read by the copy of the handle

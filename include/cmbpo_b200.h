@@ -242,6 +242,9 @@ int cmbpo_rollout_diagnostics(cmbpo_ctx* ctx, const cmbpo_rollout_bufs* bufs, in
  * cmbpo_archive_sample_boltz: distributed_batch_from_archive with a boltz_dist distribution
  *   (cpobuffer.py:385-396, 413-463): epoch k with probability cdf[k] - cdf[k-1] (cdf [n_ep] float64,
  *   device), then a uniform row of it == np.random.choice(N, B, p=dist) in distribution.
+ * cmbpo_archive_sample_boltz_range: samples [first, first + count) of that batch into out_idx[0, count):
+ *   sample i is keyed by (seed, draw, i) alone, so these are exactly the rows a whole-batch call writes at
+ *   those positions, whatever the batch size (one contiguous shard per GPU).
  * cmbpo_gather_rows: dst[i, :] = src[idx[i], :]   (arch_dict[field][indices]).
  * cmbpo_policy_kl_epochs: CPOPolicy.compute_DKL for a 3-D batch (cpo_policy.py:837-845,
  *   network/ac_network.py:50-55): kl_host[k] = mean_b sum_a KL(current || archived) over the B rows of
@@ -255,6 +258,9 @@ int cmbpo_archive_sample_epochs(cmbpo_ctx* ctx, const int32_t* sorted_idx, const
 int cmbpo_archive_sample_boltz(cmbpo_ctx* ctx, const int32_t* sorted_idx, const int64_t* bin_offsets,
                                const int32_t* epochs, const double* cdf, int n_ep, int64_t B,
                                uint64_t seed, uint64_t draw, int32_t* out_idx);
+int cmbpo_archive_sample_boltz_range(cmbpo_ctx* ctx, const int32_t* sorted_idx, const int64_t* bin_offsets,
+                                     const int32_t* epochs, const double* cdf, int n_ep, int64_t first,
+                                     int64_t count, uint64_t seed, uint64_t draw, int32_t* out_idx);
 int cmbpo_gather_rows(cmbpo_ctx* ctx, const float* src, int width, const int32_t* idx, int64_t n, float* dst);
 int cmbpo_policy_kl_epochs(cmbpo_ctx* ctx, const float* cur_mu, const float* cur_log_std, const float* old_mu,
                            const float* old_log_std, int n_ep, int64_t B, int A, double* kl_host);
