@@ -55,7 +55,7 @@ class TrainCfg(C.Structure):
 
 
 # name -> (restype, argtypes); every symbol include/cmbpo_b200.h declares
-_vp, _i, _i64, _d, _f, _u64 = C.c_void_p, C.c_int, C.c_int64, C.c_double, C.c_float, C.c_uint64
+_vp, _i, _i64, _d, _u64 = C.c_void_p, C.c_int, C.c_int64, C.c_double, C.c_uint64
 SIGNATURES = {
     "cmbpo_abi_version": (_i, []),
     "cmbpo_last_error": (C.c_char_p, []),
@@ -85,14 +85,12 @@ SIGNATURES = {
     "cmbpo_policy_kl_epochs": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64, _i, C.POINTER(C.c_double)]),
     "cmbpo_rollout_diagnostics": (_i, [_vp, C.POINTER(RolloutBufs), _i64, _vp, _vp, C.POINTER(C.c_double)]),
     "cmbpo_gae_paths": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _i64, _i64, _vp, _vp, _vp,
-                             _d, _d, _d, _d, _vp, _vp, _vp, _vp, _i]),
-    "cmbpo_gae_flat": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp,
+                             _d, _d, _d, _d, _vp, _vp, _vp, _vp]),
+    "cmbpo_gae_flat": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp,
                             _d, _d, _d, _d, _vp, _vp, _vp, _vp, _i]),
     "cmbpo_adv_stats_pass1": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _i, _i64, _i64, _vp, _vp]),
-    "cmbpo_adv_stats_pass2": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _vp, _f, _vp]),
-    "cmbpo_adv_normalise": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _i64, _vp, _f, _f, _f]),
-    "cmbpo_adv_stats_pass2_dev": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _vp, _vp, _vp]),
-    "cmbpo_adv_normalise_dev": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _i64, _vp, _vp]),
+    "cmbpo_adv_stats_pass2": (_i, [_vp, _vp, _i64, _i, _i64, _i64, _vp, _vp, _vp]),
+    "cmbpo_adv_normalise": (_i, [_vp, _vp, _vp, _i64, _i, _i64, _i64, _vp, _vp]),
     "cmbpo_ens_train_begin": (_i, [_vp, _i]),
     "cmbpo_ens_train_step": (_i, [_vp, _i, _vp, _vp, _i64, C.POINTER(TrainCfg), _vp]),
     "cmbpo_ens_train_loss": (_i, [_vp, _i, _vp, _vp, _i64, _vp]),
@@ -106,7 +104,7 @@ SIGNATURES = {
 }
 
 _lib = None
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 
 class CmbpoError(RuntimeError):

@@ -105,8 +105,9 @@ class CPOBuffer:
         if n > 0:
             adv, cadv = e.to_device(self.adv_buf[:n]), e.to_device(self.cadv_buf[:n])
             ret, cret = e.to_device(self.ret_buf[:n]), e.to_device(self.cret_buf[:n])
-            st = e.adv_statistics(adv, cadv, ret, cret, 1, n, n, 1, None)
-            e.adv_normalise(adv, cadv, 1, n, n, 1, None, st)
+            sums = e.adv_statistics_device(adv, cadv, ret, cret, 1, n, n, 1, None)
+            e.adv_normalise_device(adv, cadv, 1, n, n, 1, None, sums)
+            st = e.stats_from_sums(sums.cpu().numpy())
             self.adv_buf[:n], self.cadv_buf[:n] = adv.cpu().numpy(), cadv.cpu().numpy()
             ret_mean, cret_mean = st["ret_mean"], st["cret_mean"]
         else:

@@ -88,7 +88,6 @@ struct cmbpo_ctx {
     int64_t launches = 0;
     // per-context (= per-device) records of cudaFuncSetAttribute calls already made
     size_t step_smem_max[2] = {0, 0};
-    bool gae_rows_attr_set = false;
     // rollout: page-locked mirror of the live row count + events (early exit once every path ended)
     int64_t* host_n = nullptr;      // [4]
     cudaEvent_t n_ev[4] = {nullptr, nullptr, nullptr, nullptr};

@@ -71,66 +71,10 @@ __global__ void gae_paths_strict_kernel(const float* __restrict__ rew, const flo
     }
 }
 
-// ---- STRICT, row-major [B, T] (the reference ModelBuffer layout): each warp stages its 32
-// rows (one contiguous 32*T-float block per field) through shared memory so that global
-// traffic is coalesced float4; lane i then scans row i (row pitch T|1 words -> conflict free).
-template <int WARPS>
-__global__ void gae_rows_strict_kernel(const float* __restrict__ rew, const float* __restrict__ val,
-                                       const float* __restrict__ cost, const float* __restrict__ cval,
-                                       int64_t n_paths, int T, const int32_t* __restrict__ length,
-                                       const float* __restrict__ last_val,
-                                       const float* __restrict__ last_cval, GaeK k,
-                                       float* __restrict__ adv, float* __restrict__ ret,
-                                       float* __restrict__ cadv, float* __restrict__ cret) {
-    extern __shared__ float smem[];
-    const int pitch = T | 1;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    float* s_r = smem + (size_t)warp * 4 * 32 * pitch;
-    float* s_v = s_r + 32 * pitch;
-    float* s_c = s_v + 32 * pitch;
-    float* s_cv = s_c + 32 * pitch;
-    const int64_t p0 = ((int64_t)blockIdx.x * WARPS + warp) * 32;
-    if (p0 >= n_paths) return;
-    const int rows = (int)min((int64_t)32, n_paths - p0);
-    const int64_t g0 = p0 * T;
-    const int n = rows * T;
-    for (int i = lane; i < n; i += 32) {
-        int rr = i / T, tt = i - rr * T;
-        int s = rr * pitch + tt;
-        s_r[s] = rew[g0 + i]; s_v[s] = val[g0 + i]; s_c[s] = cost[g0 + i]; s_cv[s] = cval[g0 + i];
-    }
-    __syncwarp();
-    int len = 0;
-    if (lane < rows) {
-        len = length ? length[p0 + lane] : T;
-        double y = 0.0, cy = 0.0;
-        float vn = last_val[p0 + lane], cvn = last_cval[p0 + lane];
-        float* rr = s_r + lane * pitch; float* vv = s_v + lane * pitch;
-        float* cc = s_c + lane * pitch; float* cvv = s_cv + lane * pitch;
-        for (int t = len - 1; t >= 0; --t) {
-            float r = rr[t], v = vv[t], c = cc[t], cv = cvv[t];
-            float a, rt, ca, crt;
-            gae_step(r, v, vn, k.g32, k.d, y, a, rt);
-            gae_step(c, cv, cvn, k.cg32, k.cd, cy, ca, crt);
-            rr[t] = a; vv[t] = rt; cc[t] = ca; cvv[t] = crt;   // results overwrite the inputs
-            vn = v; cvn = cv;
-        }
-    }
-    __syncwarp();
-    // write back only t < length (unpopulated cells keep their zeros, modelbuffer.py:53-98)
-    for (int i = lane; i < n; i += 32) {
-        int rr = i / T, tt = i - rr * T;
-        int l = __shfl_sync(0xffffffffu, len, rr);
-        if (tt < l) {
-            int s = rr * pitch + tt;
-            adv[g0 + i] = s_r[s]; ret[g0 + i] = s_v[s]; cadv[g0 + i] = s_c[s]; cret[g0 + i] = s_cv[s];
-        }
-    }
-}
-
-// ---- WARP: one warp per segment, 32-element chunks walked from the end of the segment to
-// its start; inside a chunk the recurrence y_t = x_t + d*y_{t+1} is a Hillis-Steele scan over
-// lanes with powers of d (5 shuffle rounds, float64), the carry enters as d^(k+1)*carry.
+// ---- WARP, flat CPOBuffer layout: one warp per segment, 32-element chunks walked from the end
+// of the segment to its start; inside a chunk the recurrence y_t = x_t + d*y_{t+1} is a
+// Hillis-Steele scan over lanes with powers of d (5 shuffle rounds, float64), the carry enters
+// as d^(k+1)*carry.
 __device__ __forceinline__ double shfl_down_f64(double x, int delta) {
     return __shfl_down_sync(0xffffffffu, x, delta);
 }
@@ -138,21 +82,15 @@ __device__ __forceinline__ double shfl_down_f64(double x, int delta) {
 __global__ void gae_segments_warp_kernel(const float* __restrict__ rew, const float* __restrict__ val,
                                          const float* __restrict__ cost, const float* __restrict__ cval,
                                          int64_t n_seg, const int64_t* __restrict__ seg_offsets,
-                                         int64_t ps, int64_t ts, const int32_t* __restrict__ length,
-                                         int max_len, const float* __restrict__ last_val,
+                                         const float* __restrict__ last_val,
                                          const float* __restrict__ last_cval, GaeK k,
                                          float* __restrict__ adv, float* __restrict__ ret,
                                          float* __restrict__ cadv, float* __restrict__ cret) {
     const int lane = threadIdx.x & 31;
     const int64_t seg = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (seg >= n_seg) return;
-    int64_t base, stride;
-    int len;
-    if (seg_offsets) {            // flat CPOBuffer layout
-        base = seg_offsets[seg]; stride = 1; len = (int)(seg_offsets[seg + 1] - base);
-    } else {                      // path layout
-        base = seg * ps; stride = ts; len = length ? length[seg] : max_len;
-    }
+    const int64_t base = seg_offsets[seg];
+    const int len = (int)(seg_offsets[seg + 1] - base);
     if (len <= 0) return;
     // powers of d for the in-chunk scan
     double dp[5], cdp[5];
@@ -167,12 +105,12 @@ __global__ void gae_segments_warp_kernel(const float* __restrict__ rew, const fl
         const bool ok = t < hi;
         double x = 0.0, cx = 0.0;
         float v = 0.f, cv = 0.f;
-        int64_t i = base + (int64_t)t * stride;
+        const int64_t i = base + t;
         if (ok) {
             float r = rew[i], c = cost[i];
             v = val[i]; cv = cval[i];
-            float vn = (t + 1 < len) ? val[i + stride] : lv;
-            float cvn = (t + 1 < len) ? cval[i + stride] : lcv;
+            float vn = (t + 1 < len) ? val[i + 1] : lv;
+            float cvn = (t + 1 < len) ? cval[i + 1] : lcv;
             x = (double)__fsub_rn(__fadd_rn(r, __fmul_rn(k.g32, vn)), v);
             cx = (double)__fsub_rn(__fadd_rn(c, __fmul_rn(k.cg32, cvn)), cv);
         }
@@ -272,11 +210,11 @@ __global__ void stats_pass1_kernel(const float* __restrict__ adv, const float* _
 
 __global__ void stats_pass2_kernel(const float* __restrict__ adv, int64_t n_paths, int max_len,
                                    int64_t ps, int64_t ts, const int32_t* __restrict__ length,
-                                   float mean, const double* __restrict__ sums_dev, double* __restrict__ partial) {
+                                   const double* __restrict__ sums, double* __restrict__ partial) {
     __shared__ double sh[32];
     double ss = 0;
-    // device-resident statistics (no host round trip): mean = float32(sum) / float32(n) as mpi_tools.py:82-83
-    if (sums_dev) mean = (sums_dev[0] > 0.0) ? __fdiv_rn((float)sums_dev[1], (float)sums_dev[0]) : 0.f;
+    // mean = float32(sum) / float32(n) as mpi_tools.py:82-83, from the (all-reduced) sums of pass 1
+    const float mean = (sums[0] > 0.0) ? __fdiv_rn((float)sums[1], (float)sums[0]) : 0.f;
     const int64_t total = n_paths * (int64_t)max_len;
     const bool path_fast = ps <= ts;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -314,15 +252,13 @@ __global__ void __launch_bounds__(256) stats_final_kernel(const double* __restri
 
 __global__ void normalise_kernel(float* __restrict__ adv, float* __restrict__ cadv, int64_t n_paths,
                                  int max_len, int64_t ps, int64_t ts,
-                                 const int32_t* __restrict__ length, float mean, float denom,
-                                 float cmean, const double* __restrict__ sums_dev) {
-    if (sums_dev) {                     // sums = (n, sum adv, sum cadv, sum ret, sum cret, sum (adv-mean)^2), all-reduced
-        if (!(sums_dev[0] > 0.0)) return;
-        const float n = (float)sums_dev[0];
-        mean = __fdiv_rn((float)sums_dev[1], n);
-        cmean = __fdiv_rn((float)sums_dev[2], n);
-        denom = __fadd_rn(__fsqrt_rn(__fdiv_rn((float)sums_dev[5], n)), 1e-8f);     // mpi_tools.py:85-86, modelbuffer.py:199
-    }
+                                 const int32_t* __restrict__ length, const double* __restrict__ sums) {
+    // sums = (n, sum adv, sum cadv, sum ret, sum cret, sum (adv-mean)^2), all-reduced
+    if (!(sums[0] > 0.0)) return;
+    const float n = (float)sums[0];
+    const float mean = __fdiv_rn((float)sums[1], n);
+    const float cmean = __fdiv_rn((float)sums[2], n);
+    const float denom = __fadd_rn(__fsqrt_rn(__fdiv_rn((float)sums[5], n)), 1e-8f);     // mpi_tools.py:85-86, modelbuffer.py:199
     const int64_t total = n_paths * (int64_t)max_len;
     const bool path_fast = ps <= ts;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -427,49 +363,27 @@ extern "C" int cmbpo_gae_paths(cmbpo_ctx* ctx, const float* rew, const float* va
                                const float* cval, int64_t n_paths, int max_len, int64_t path_stride,
                                int64_t time_stride, const int32_t* length, const float* last_val,
                                const float* last_cval, double gamma, double lam, double cgamma,
-                               double clam, float* adv, float* ret, float* cadv, float* cret,
-                               int scan_mode) {
+                               double clam, float* adv, float* ret, float* cadv, float* cret) {
     CMBPO_CHECK(ctx, "null context");
     if (n_paths <= 0 || max_len <= 0) return 0;
     GaeK k = make_k(gamma, lam, cgamma, clam);
     ProfScope prof(ctx, CMBPO_PROF_GAE);
-    if (scan_mode == CMBPO_SCAN_WARP) {
-        int threads = 256;
-        int64_t blocks = (n_paths * 32 + threads - 1) / threads;
-        gae_segments_warp_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>(
-            rew, val, cost, cval, n_paths, nullptr, path_stride, time_stride, length, max_len,
-            last_val, last_cval, k, adv, ret, cadv, cret);
-    } else if (time_stride == 1 && path_stride == max_len && max_len <= 96) {
-        constexpr int WARPS = 4;
-        size_t smem = (size_t)WARPS * 4 * 32 * (max_len | 1) * sizeof(float);
-        if (!ctx->gae_rows_attr_set) {
-            CUDA_TRY(cudaFuncSetAttribute(gae_rows_strict_kernel<WARPS>,
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            ctx->gae_rows_attr_set = true;
-        }
-        int64_t blocks = (n_paths + WARPS * 32 - 1) / (WARPS * 32);
-        gae_rows_strict_kernel<WARPS><<<(unsigned)blocks, WARPS * 32, smem, ctx->stream>>>(
-            rew, val, cost, cval, n_paths, max_len, length, last_val, last_cval, k, adv, ret, cadv,
-            cret);
-    } else {
-        int threads = 128;
-        int64_t blocks = (n_paths + threads - 1) / threads;
-        gae_paths_strict_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>(
-            rew, val, cost, cval, n_paths, max_len, path_stride, time_stride, length, last_val,
-            last_cval, k, adv, ret, cadv, cret);
-    }
+    int threads = 128;
+    int64_t blocks = (n_paths + threads - 1) / threads;
+    gae_paths_strict_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>(
+        rew, val, cost, cval, n_paths, max_len, path_stride, time_stride, length, last_val,
+        last_cval, k, adv, ret, cadv, cret);
     ctx->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
 extern "C" int cmbpo_gae_flat(cmbpo_ctx* ctx, const float* rew, const float* val, const float* cost,
-                              const float* cval, int64_t n, const int64_t* seg_offsets, int64_t n_seg,
+                              const float* cval, const int64_t* seg_offsets, int64_t n_seg,
                               const float* last_val, const float* last_cval, double gamma, double lam,
                               double cgamma, double clam, float* adv, float* ret, float* cadv,
                               float* cret, int scan_mode) {
     CMBPO_CHECK(ctx, "null context");
-    (void)n;
     if (n_seg <= 0) return 0;
     GaeK k = make_k(gamma, lam, cgamma, clam);
     ProfScope prof(ctx, CMBPO_PROF_GAE);
@@ -477,8 +391,7 @@ extern "C" int cmbpo_gae_flat(cmbpo_ctx* ctx, const float* rew, const float* val
     if (scan_mode == CMBPO_SCAN_WARP) {
         int64_t blocks = (n_seg * 32 + threads - 1) / threads;
         gae_segments_warp_kernel<<<(unsigned)blocks, threads, 0, ctx->stream>>>(
-            rew, val, cost, cval, n_seg, seg_offsets, 0, 1, nullptr, 0, last_val, last_cval, k, adv,
-            ret, cadv, cret);
+            rew, val, cost, cval, n_seg, seg_offsets, last_val, last_cval, k, adv, ret, cadv, cret);
     } else {
         int64_t blocks = (n_seg + 63) / 64;
         gae_flat_strict_kernel<<<(unsigned)blocks, 64, 0, ctx->stream>>>(
@@ -508,60 +421,28 @@ extern "C" int cmbpo_adv_stats_pass1(cmbpo_ctx* ctx, const float* adv, const flo
 
 extern "C" int cmbpo_adv_stats_pass2(cmbpo_ctx* ctx, const float* adv, int64_t n_paths, int max_len,
                                      int64_t path_stride, int64_t time_stride, const int32_t* length,
-                                     float adv_mean, double* sums_out) {
-    CMBPO_CHECK(ctx, "null context");
+                                     const double* sums, double* sums_out) {
+    CMBPO_CHECK(ctx && sums && sums_out, "null argument");
     int threads = 256;
     int blocks = grid_for(ctx, n_paths * (int64_t)max_len, threads);
     double* partial;
     if (cmbpo_ws_get(ctx, 7, (size_t)blocks * 8 * sizeof(double), (void**)&partial)) return 1;
     stats_pass2_kernel<<<blocks, threads, 0, ctx->stream>>>(adv, n_paths, max_len, path_stride,
-                                                          time_stride, length, adv_mean, nullptr, partial);
+                                                          time_stride, length, sums, partial);
     stats_final_kernel<<<1, 256, 0, ctx->stream>>>(partial, blocks, 1, 1, sums_out, 5);
     ctx->launches += 2;
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-}
-
-extern "C" int cmbpo_adv_stats_pass2_dev(cmbpo_ctx* ctx, const float* adv, int64_t n_paths, int max_len,
-                                         int64_t path_stride, int64_t time_stride, const int32_t* length,
-                                         const double* sums_dev, double* sums_out) {
-    CMBPO_CHECK(ctx && sums_dev && sums_out, "null argument");
-    int threads = 256;
-    int blocks = grid_for(ctx, n_paths * (int64_t)max_len, threads);
-    double* partial;
-    if (cmbpo_ws_get(ctx, 7, (size_t)blocks * 8 * sizeof(double), (void**)&partial)) return 1;
-    stats_pass2_kernel<<<blocks, threads, 0, ctx->stream>>>(adv, n_paths, max_len, path_stride,
-                                                          time_stride, length, 0.f, sums_dev, partial);
-    stats_final_kernel<<<1, 256, 0, ctx->stream>>>(partial, blocks, 1, 1, sums_out, 5);
-    ctx->launches += 2;
-    CUDA_TRY(cudaGetLastError());
-    return 0;
-}
-
-extern "C" int cmbpo_adv_normalise_dev(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths,
-                                       int max_len, int64_t path_stride, int64_t time_stride,
-                                       const int32_t* length, const double* sums_dev) {
-    CMBPO_CHECK(ctx && sums_dev, "null argument");
-    int threads = 256;
-    int blocks = grid_for(ctx, n_paths * (int64_t)max_len, threads);
-    normalise_kernel<<<blocks, threads, 0, ctx->stream>>>(adv, cadv, n_paths, max_len, path_stride,
-                                                         time_stride, length, 0.f, 1.f, 0.f, sums_dev);
-    ctx->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
 extern "C" int cmbpo_adv_normalise(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths,
                                    int max_len, int64_t path_stride, int64_t time_stride,
-                                   const int32_t* length, float adv_mean, float adv_std,
-                                   float cadv_mean) {
-    CMBPO_CHECK(ctx, "null context");
+                                   const int32_t* length, const double* sums) {
+    CMBPO_CHECK(ctx && sums, "null argument");
     int threads = 256;
     int blocks = grid_for(ctx, n_paths * (int64_t)max_len, threads);
-    float denom = adv_std + 1e-8f;   // float32(std) + EPS, modelbuffer.py:199
     normalise_kernel<<<blocks, threads, 0, ctx->stream>>>(adv, cadv, n_paths, max_len, path_stride,
-                                                         time_stride, length, adv_mean, denom,
-                                                         cadv_mean, nullptr);
+                                                         time_stride, length, sums);
     ctx->launches++;
     CUDA_TRY(cudaGetLastError());
     return 0;

@@ -280,7 +280,7 @@ class Engine:
 
     # ------------------------------------------------------------------ GAE
     def gae_paths(self, rew, val, cost, cval, length, last_val, last_cval, gamma, lam, cgamma, clam,
-                  n_paths, max_len, path_stride, time_stride, out=None, scan=L.SCAN_STRICT):
+                  n_paths, max_len, path_stride, time_stride, out=None):
         t = self.torch
         if out is None:
             out = tuple(t.zeros_like(rew) for _ in range(4))
@@ -289,7 +289,7 @@ class Engine:
             self.h, self._p(rew), self._p(val), self._p(cost), self._p(cval), n_paths, max_len,
             path_stride, time_stride, self._p(length), self._p(last_val), self._p(last_cval),
             float(gamma), float(lam), float(cgamma), float(clam), self._p(adv), self._p(ret),
-            self._p(cadv), self._p(cret), int(scan)))
+            self._p(cadv), self._p(cret)))
         return adv, ret, cadv, cret
 
     def gae_flat(self, rew, val, cost, cval, seg_offsets, last_val, last_cval, gamma, lam, cgamma,
@@ -300,45 +300,19 @@ class Engine:
         adv, ret, cadv, cret = out
         n_seg = seg_offsets.shape[0] - 1
         L.check(self.lib.cmbpo_gae_flat(
-            self.h, self._p(rew), self._p(val), self._p(cost), self._p(cval), rew.shape[0],
+            self.h, self._p(rew), self._p(val), self._p(cost), self._p(cval),
             self._p(seg_offsets, t.int64), n_seg, self._p(last_val), self._p(last_cval),
             float(gamma), float(lam), float(cgamma), float(clam), self._p(adv), self._p(ret),
             self._p(cadv), self._p(cret), int(scan)))
         return adv, ret, cadv, cret
 
-    def adv_statistics(self, adv, cadv, ret, cret, n_paths, max_len, path_stride, time_stride,
-                       length, reduce_fn=None):
-        """Two-pass float32 statistics of mpi_statistics_scalar (mpi_tools.py:71-92).
-        `reduce_fn(tensor)` all-reduces a small float64 tensor in place (multi-GPU)."""
-        t = self.torch
-        sums = self.zeros(8, dtype=t.float64)
-        L.check(self.lib.cmbpo_adv_stats_pass1(self.h, self._p(adv), self._p(cadv), self._p(ret),
-                                               self._p(cret), n_paths, max_len, path_stride,
-                                               time_stride, self._p(length), self._p(sums)))
-        if reduce_fn is not None:
-            reduce_fn(sums)
-        s = sums.cpu().numpy()
-        st = combine_pass1(s)
-        if st["n"] == 0:
-            st["adv_std"] = np.float32(0)
-            return st
-        L.check(self.lib.cmbpo_adv_stats_pass2(self.h, self._p(adv), n_paths, max_len, path_stride,
-                                               time_stride, self._p(length), float(st["adv_mean"]),
-                                               self._p(sums)))
-        if reduce_fn is not None:
-            ss = sums[5:6].clone()
-            reduce_fn(ss)
-            ssq = float(ss.item())
-        else:
-            ssq = float(sums[5].item())
-        st["adv_std"] = np.float32(combine_pass2(ssq, st["n"]))
-        return st
-
     def adv_statistics_device(self, adv, cadv, ret, cret, n_paths, max_len, path_stride, time_stride,
                               length, reduce_fn=None):
-        """The same two passes with the sums kept on the device: no host synchronisation, so the host can queue
-        the normalisation and whatever follows without waiting for the scans; with N > 1 the ranks meet only in the
-        two all-reduces.  Returns the device tensor of 8 float64 sums (see `stats_from_sums`)."""
+        """Two-pass float32 statistics of mpi_statistics_scalar (mpi_tools.py:71-92) with the sums kept on the
+        device: no host synchronisation, so the host can queue the normalisation and whatever follows without
+        waiting for the scans; with N > 1 the ranks meet only in the two all-reduces.  `reduce_fn(tensor)`
+        all-reduces a small float64 tensor in place (multi-GPU).  Returns the device tensor of 8 float64 sums
+        (see `stats_from_sums`)."""
         t = self.torch
         sums = self.zeros(8, dtype=t.float64)
         L.check(self.lib.cmbpo_adv_stats_pass1(self.h, self._p(adv), self._p(cadv), self._p(ret),
@@ -346,28 +320,25 @@ class Engine:
                                                time_stride, self._p(length), self._p(sums)))
         if reduce_fn is not None:
             reduce_fn(sums)
-        L.check(self.lib.cmbpo_adv_stats_pass2_dev(self.h, self._p(adv), n_paths, max_len, path_stride,
-                                                   time_stride, self._p(length), self._p(sums), self._p(sums)))
+        L.check(self.lib.cmbpo_adv_stats_pass2(self.h, self._p(adv), n_paths, max_len, path_stride,
+                                               time_stride, self._p(length), self._p(sums), self._p(sums)))
         if reduce_fn is not None:
             reduce_fn(sums[5:6])                 # in place: a one-element view of the same memory
         return sums
 
     def adv_normalise_device(self, adv, cadv, n_paths, max_len, path_stride, time_stride, length, sums):
-        L.check(self.lib.cmbpo_adv_normalise_dev(self.h, self._p(adv), self._p(cadv), n_paths, max_len,
-                                                 path_stride, time_stride, self._p(length), self._p(sums)))
+        """adv <- (adv - mean) / (std + 1e-8), cadv <- cadv - cmean from the device sums of
+        `adv_statistics_device` (modelbuffer.py:196-204)."""
+        L.check(self.lib.cmbpo_adv_normalise(self.h, self._p(adv), self._p(cadv), n_paths, max_len,
+                                             path_stride, time_stride, self._p(length), self._p(sums)))
 
     @staticmethod
     def stats_from_sums(s):
-        """dict of adv_statistics() from a HOST copy of the 8 sums of adv_statistics_device()."""
+        """dict of n, adv_mean, adv_std, cadv_mean, ret_mean, cret_mean (float32) from a HOST copy of the 8
+        sums of adv_statistics_device()."""
         st = combine_pass1(s)
         st["adv_std"] = np.float32(combine_pass2(float(s[5]), st["n"])) if st["n"] else np.float32(0)
         return st
-
-    def adv_normalise(self, adv, cadv, n_paths, max_len, path_stride, time_stride, length, st):
-        L.check(self.lib.cmbpo_adv_normalise(self.h, self._p(adv), self._p(cadv), n_paths, max_len,
-                                             path_stride, time_stride, self._p(length),
-                                             float(st["adv_mean"]), float(st["adv_std"]),
-                                             float(st["cadv_mean"])))
 
     def path_offsets(self, length):
         t = self.torch

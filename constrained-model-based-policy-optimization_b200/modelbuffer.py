@@ -24,7 +24,6 @@ class ModelBuffer:
         self.gamma, self.lam, self.cost_gamma, self.cost_lam = 0.99, 0.95, 0.99, 0.95
         self.reduce_fn = None        # set by the multi-GPU wrapper: all-reduce of the statistics
         self._dist = None            # distribute(): get() gathers the whole batch on one rank
-        self.scan_mode = L.SCAN_STRICT
         self.reset()
 
     def initialize(self, pi_info_shapes, gamma=0.99, lam=0.95, cost_gamma=0.99, cost_lam=0.95):
@@ -129,7 +128,7 @@ class ModelBuffer:
             e.gae_paths(b.rew, b.val, b.cost, b.cval, e.to_device(len_now, t.int32),
                         e.to_device(lv), e.to_device(lc), self.gamma, self.lam, self.cost_gamma,
                         self.cost_lam, self.batch_size, self.max_path_length, 1, self.batch_size,
-                        out=(b.adv, b.ret, b.cadv, b.cret), scan=self.scan_mode)
+                        out=(b.adv, b.ret, b.cadv, b.cret))
         # a path closed before its first store contributes nothing (modelbuffer.py:160)
         self.terminated_paths_mask[fin] = True
 
@@ -141,7 +140,7 @@ class ModelBuffer:
 
     def finish_all_device(self):
         """GAE for every path from the device-resident (length, last_val, last_cval)."""
-        self.bufs.gae(self.gamma, self.lam, self.cost_gamma, self.cost_lam, scan=self.scan_mode)
+        self.bufs.gae(self.gamma, self.lam, self.cost_gamma, self.cost_lam)
         self.terminated_paths_mask[:] = True
 
     # ---- multi-GPU ---------------------------------------------------------------------------

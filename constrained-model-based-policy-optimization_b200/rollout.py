@@ -101,12 +101,12 @@ class RolloutBuffers:
         keys = ("rew", "cost", "val", "cval", "dyn_error", "max_dkl", "max_path_return", "n")
         return dict(zip(keys, (float(x) for x in st)))
 
-    def gae(self, gamma, lam, cgamma, clam, scan=L.SCAN_STRICT):
+    def gae(self, gamma, lam, cgamma, clam):
         """adv/ret/cadv/cret for every path from (length, last_val, last_cval)."""
         self.engine.gae_paths(self.rew, self.val, self.cost, self.cval, self.length, self.last_val,
                               self.last_cval, gamma, lam, cgamma, clam, self.B, self.T,
                               path_stride=1, time_stride=self.B,
-                              out=(self.adv, self.ret, self.cadv, self.cret), scan=scan)
+                              out=(self.adv, self.ret, self.cadv, self.cret))
 
     # ---- reference-layout views (host) -------------------------------------------------
     def host(self, name):

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define CMBPO_ABI_VERSION 2
+#define CMBPO_ABI_VERSION 3
 
 typedef struct cmbpo_ctx cmbpo_ctx;
 
@@ -58,9 +58,10 @@ enum { CMBPO_END_ALIVE = 0, CMBPO_END_UNCERTAIN = 1, CMBPO_END_HORIZON = 2, CMBP
        CMBPO_END_CAPPED = 4,  /* max_samples cap, model_sampler.py:282-287 */
        CMBPO_END_STOPPED = 5  /* finish_all_paths after the caller stopped, model_sampler.py:418-444 */ };
 
-/* GAE scan flavour */
+/* GAE scan flavour of cmbpo_gae_flat (the path layout of cmbpo_gae_paths always scans STRICT) */
 enum { CMBPO_SCAN_STRICT = 0, /* float64, strictly sequential: bit-identical to scipy.signal.lfilter */
-       CMBPO_SCAN_WARP = 1 }; /* float64 warp-shuffle segmented scan (re-associated; <= 1 ulp after the fp32 round) */
+       CMBPO_SCAN_WARP = 1 }; /* flat layout only: float64 warp-shuffle segmented scan (re-associated;
+                                 <= 1 ulp after the fp32 round) */
 
 int cmbpo_abi_version(void);
 const char* cmbpo_last_error(void);
@@ -276,44 +277,37 @@ int cmbpo_gae_paths(cmbpo_ctx* ctx, const float* rew, const float* val, const fl
                     const float* cval, int64_t n_paths, int max_len, int64_t path_stride,
                     int64_t time_stride, const int32_t* length, const float* last_val,
                     const float* last_cval, double gamma, double lam, double cgamma, double clam,
-                    float* adv, float* ret, float* cadv, float* cret, int scan_mode);
+                    float* adv, float* ret, float* cadv, float* cret);
 /* flat CPOBuffer layout: segment i = [seg_offsets[i], seg_offsets[i+1]) (cpobuffer.py:180, 206) */
 int cmbpo_gae_flat(cmbpo_ctx* ctx, const float* rew, const float* val, const float* cost,
-                   const float* cval, int64_t n, const int64_t* seg_offsets, int64_t n_seg,
+                   const float* cval, const int64_t* seg_offsets, int64_t n_seg,
                    const float* last_val, const float* last_cval, double gamma, double lam,
                    double cgamma, double clam, float* adv, float* ret, float* cadv, float* cret,
                    int scan_mode);
 
 /*
- * mpi_statistics_scalar (utilities/mpi_tools.py:71-92) pass 1 and 2 over the valid entries
- * (valid = t < length[p] for the path layout; all n for the flat layout when length == NULL).
- *   sums_out (device, 8 doubles): {n, sum_adv, sum_cadv, sum_ret, sum_cret, sumsq_adv(after pass 2), 0, 0}.
- *   Multi-GPU: the caller all-reduces sums_out[0..4] between pass 1 and pass 2 and sums_out[5]
- *   after pass 2 (the two Allreduce calls of mpi_tools.py:82-86).
+ * mpi_statistics_scalar (utilities/mpi_tools.py:71-92) and the normalisation of ModelBuffer.get
+ * (modelbuffer.py:196-204) over the valid entries (valid = t < length[p]; every t < max_len when
+ * length == NULL).  The statistics stay in DEVICE memory: no host round trip between the calls, so a
+ * multi-GPU job's ranks are only coupled by the two all-reduces.
+ *   sums (device, 8 doubles): {n, sum_adv, sum_cadv, sum_ret, sum_cret, sumsq_adv, 0, 0}.
+ *   pass1 writes sums_out[0..4] (and zeroes [5..7]).  Multi-GPU: the caller all-reduces [0..4] here.
+ *   pass2 forms mean = float32(sum_adv)/float32(n) from `sums` on the device (mpi_tools.py:82-83) and
+ *     writes the local sum of (adv - mean)^2 to sums_out[5] (sums_out may equal sums).  Multi-GPU: the
+ *     caller all-reduces [5] here (the two Allreduce calls of mpi_tools.py:82-86).
+ *   normalise forms mean, cmean = float32(sum)/float32(n) and std = sqrt(float32(sumsq)/float32(n)) from
+ *     the all-reduced sums and sets adv <- (adv-mean)/(std+1e-8), cadv <- cadv-cmean on valid entries.
+ *   n == 0: pass2 writes 0, normalise touches nothing.
  */
 int cmbpo_adv_stats_pass1(cmbpo_ctx* ctx, const float* adv, const float* cadv, const float* ret,
                           const float* cret, int64_t n_paths, int max_len, int64_t path_stride,
                           int64_t time_stride, const int32_t* length, double* sums_out);
 int cmbpo_adv_stats_pass2(cmbpo_ctx* ctx, const float* adv, int64_t n_paths, int max_len,
                           int64_t path_stride, int64_t time_stride, const int32_t* length,
-                          float adv_mean, double* sums_out);
-/* adv <- (adv-mean)/(std+1e-8), cadv <- cadv-cmean on valid entries (modelbuffer.py:198-204) */
+                          const double* sums, double* sums_out);
 int cmbpo_adv_normalise(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths, int max_len,
                         int64_t path_stride, int64_t time_stride, const int32_t* length,
-                        float adv_mean, float adv_std, float cadv_mean);
-/*
- * The same two steps with the statistics kept in DEVICE memory (no host round trip between the passes, so a
- * multi-GPU job's ranks are only coupled by the two NCCL all-reduces, not by host synchronisations):
- * sums_dev = the 8 doubles of pass 1 (all-reduced); pass2_dev forms mean = float32(sum)/float32(n) on the device
- * (mpi_tools.py:82-83) and writes the local sum of squares to sums_out[5]; normalise_dev forms mean, cmean and
- * std = sqrt(float32(sumsq)/float32(n)) from the (all-reduced) sums (mpi_tools.py:85-86).  n == 0: no-ops.
- */
-int cmbpo_adv_stats_pass2_dev(cmbpo_ctx* ctx, const float* adv, int64_t n_paths, int max_len,
-                              int64_t path_stride, int64_t time_stride, const int32_t* length,
-                              const double* sums_dev, double* sums_out);
-int cmbpo_adv_normalise_dev(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths, int max_len,
-                            int64_t path_stride, int64_t time_stride, const int32_t* length,
-                            const double* sums_dev);
+                        const double* sums);
 
 /*
  * SURVEY.md 8f-4: the ensemble training step -- the body of the batch loop of PE.train (models/pens/pe.py:547-567).

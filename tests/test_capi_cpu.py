@@ -25,7 +25,7 @@ def test_every_declared_symbol_is_exported_and_bound():
         assert hasattr(lib, n), "missing export %s" % n
         assert n in _lib.SIGNATURES, "no ctypes prototype for %s" % n
     assert sorted(_lib.SIGNATURES) == names
-    assert _lib.load().cmbpo_abi_version() == 2
+    assert _lib.load().cmbpo_abi_version() == 3
 
 
 def test_struct_layouts_match_header():

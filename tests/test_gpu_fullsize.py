@@ -121,11 +121,12 @@ def test_fullsize_normalise_and_compaction(hcs_full, engine):
     b, B, T, O = (hcs_full[k] for k in ("bufs", "B", "T", "O"))
     t = engine.torch
     adv, cadv = b.adv.clone(), b.cadv.clone()
-    st = engine.adv_statistics(adv, cadv, b.ret, b.cret, B, T, 1, B, b.length)
+    sums = engine.adv_statistics_device(adv, cadv, b.ret, b.cret, B, T, 1, B, b.length)
+    st = engine.stats_from_sums(sums.cpu().numpy())
     assert st["n"] == B * (T - 1)
     ref_mean = float(b.adv[:T - 1].double().mean())
     assert abs(st["adv_mean"] - ref_mean) <= 1e-6 * max(1.0, abs(ref_mean)) + 1e-6
-    engine.adv_normalise(adv, cadv, B, T, 1, B, b.length, st)
+    engine.adv_normalise_device(adv, cadv, B, T, 1, B, b.length, sums)
     a = adv[:T - 1].double()
     assert abs(float(a.mean())) < 1e-4 and abs(float(a.std(unbiased=False)) - 1.0) < 1e-3
     assert abs(float(cadv[:T - 1].double().mean())) < 1e-4

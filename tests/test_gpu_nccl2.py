@@ -32,8 +32,9 @@ def _run_shard(eng, cb, L, wl, torch, nets, obs, lo, hi, reduce_fn, precision):
     # uncertainty mode with a finite limit: ragged path lengths, so the gathered order matters
     bufs.run(cfg, uncertainty_mode=True, dkl_lim=_run_shard.dkl_lim, seed=77, path_id_base=lo, precision=precision)
     bufs.gae(GAE["gamma"], GAE["lam"], GAE["cost_gamma"], GAE["cost_lam"])
-    st = eng.adv_statistics(bufs.adv, bufs.cadv, bufs.ret, bufs.cret, n, T, 1, n, bufs.length, reduce_fn)
-    eng.adv_normalise(bufs.adv, bufs.cadv, n, T, 1, n, bufs.length, st)
+    sums = eng.adv_statistics_device(bufs.adv, bufs.cadv, bufs.ret, bufs.cret, n, T, 1, n, bufs.length, reduce_fn)
+    eng.adv_normalise_device(bufs.adv, bufs.cadv, n, T, 1, n, bufs.length, sums)
+    st = eng.stats_from_sums(sums.cpu().numpy())
     torch.cuda.synchronize()
     out = {k: bufs.host(k) for k in ("obs", "act", "nextobs", "rew", "val", "cval", "cost", "logp", "adv", "cadv", "ret", "cret")}
     out["length"] = bufs.length.cpu().numpy()
