@@ -8,7 +8,12 @@ sums (n, sum adv, sum cadv, sum ret, sum cret) and then the sum of squared devia
 `ModelSampler.distribute`, also small all-gathers of counts and sums (shard sizes, length histograms,
 per-step statistics, diagnostics) and, in `ModelBuffer.get`, the populated rows to one rank.
 One process per GPU, `torch.distributed` (NCCL on GPUs, gloo in the CPU tests).
+
+The rollout block has one code path for any number of ranks: a process on its own is the one-rank case
+(`Ranks()`), whose gathers return its own vector without touching `torch.distributed`.
 """
+from typing import Any, NamedTuple
+
 import numpy as np
 
 
@@ -48,6 +53,28 @@ def all_gather_host(vec, group=None, device=None):
     out = torch.empty(dist.get_world_size(group) * x.numel(), dtype=x.dtype, device=x.device)
     dist.all_gather_into_tensor(out, x, group=group)
     return out.cpu().numpy().reshape((-1,) + a.shape)
+
+
+class Ranks(NamedTuple):
+    """The ranks of a rollout block and this process's place among them.  `Ranks()` is a process on its own:
+    one rank, no group.  `sharded` marks a block that `ModelSampler.distribute` set up (its `group` None is the
+    default process group), even one of world size 1."""
+    group: Any = None
+    rank: int = 0
+    world: int = 1
+    root: int = 0
+    sharded: bool = False
+
+    @classmethod
+    def of(cls, group=None, root=0):
+        import torch.distributed as dist
+        return cls(group, dist.get_rank(group), dist.get_world_size(group), int(root), True)
+
+    def gather(self, vec, device=None):
+        """all_gather_host over these ranks; one rank gathers its own vector and issues no collective."""
+        if self.world == 1:
+            return np.asarray(vec)[None]
+        return all_gather_host(vec, self.group, device)
 
 
 def rank_order_sum(gathered):

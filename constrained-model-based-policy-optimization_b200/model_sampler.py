@@ -15,7 +15,7 @@ from collections import OrderedDict
 import numpy as np
 
 from . import _lib as L
-from .dist import all_gather_host, cap_split, rank_order_sum
+from .dist import Ranks, cap_split, rank_order_sum
 from .fake_env import FakeEnv
 from .policy import B200Policy
 
@@ -40,7 +40,7 @@ class ModelSampler:
         self.injected = None          # tests: dict(act_eps=[T,B,A], elite_pos=[T,B], state_eps=...)
         self.path_id_base = 0         # multi-GPU: global id of this rank's first path
         self.return_arrays = False
-        self._dist = None             # distribute(): (group, rank) of a sharded rollout block
+        self._ranks = Ranks()         # the rollout block's ranks: this process alone until distribute()
         self._batch_total = batch_size
         self._global_sums = None
 
@@ -81,32 +81,35 @@ class ModelSampler:
         GPU) with the samples one GPU gives.  Every rank calls reset() with its contiguous block of the
         start states, in rank order (DeviceArchive.sample_start_states(shard=...)).  The batch-wide
         rules -- the max_samples cap, the sample count and alive ratio the caller stops on,
-        compute_dynamics_dkl and the finish_all_paths() diagnostics -- then use counts and sums over all
-        ranks and are identical on every rank, and the pool's get() returns the whole batch on rank
-        `root` (zero rows elsewhere).  Fused mode only; call after initialize()."""
+        compute_dynamics_dkl and the finish_all_paths() diagnostics -- use counts and sums over all ranks
+        and are identical on every rank, and the pool's get() returns the whole batch on rank `root` (zero
+        rows elsewhere).  Without distribute() the same code runs with this process as the only rank.
+        Fused mode only; call after initialize()."""
         import torch.distributed as dist
         if not (dist.is_available() and dist.is_initialized()):
             raise L.CmbpoError("ModelSampler.distribute needs an initialised torch.distributed process group")
         if not self.fused:
             raise L.CmbpoError("a multi-rank ModelSampler needs the fused mode (a B200Policy and a FakeEnv of "
                                "one Engine); the step-wise mode runs on one rank only")
-        self._dist = dict(group=group, rank=dist.get_rank(group))
+        self._ranks = Ranks.of(group, root)
         self._auto_base = self.path_id_base
         self.pool.distribute(group, root)
 
     def _gather(self, vec):
         """[world, ...] all-gather of a small host vector, rank order."""
-        return all_gather_host(vec, self._dist["group"], self.pool.engine.device)
+        return self._ranks.gather(vec, self.pool.engine.device)
 
     def _shard_base(self, n):
-        """(global id of this rank's first path, global path count) from the ranks' shard sizes."""
+        """The global path count from the ranks' shard sizes.  After distribute(), also sets path_id_base (global
+        id of this rank's first path); a single process keeps the caller's path_id_base."""
         sizes = self._gather(np.array([n], np.int64))[:, 0]
-        base = int(sizes[:self._dist["rank"]].sum())
-        if self.path_id_base not in (self._auto_base, base):
-            raise L.CmbpoError("path_id_base %d was set by hand, but the shard sizes put this rank's first path "
-                               "at %d" % (self.path_id_base, base))
-        self.path_id_base = self._auto_base = base
-        return base, int(sizes.sum())
+        if self._ranks.sharded:
+            base = int(sizes[:self._ranks.rank].sum())
+            if self.path_id_base not in (self._auto_base, base):
+                raise L.CmbpoError("path_id_base %d was set by hand, but the shard sizes put this rank's first "
+                                   "path at %d" % (self.path_id_base, base))
+            self.path_id_base = self._auto_base = base
+        return int(sizes.sum())
 
     # ---- calibration (model_sampler.py:151-167) ----------------------------------------------
     def compute_dynamics_dkl(self, obs_batch, depth=1):
@@ -138,20 +141,17 @@ class ModelSampler:
         inj = self.injected or {}
         bufs.set_inputs(obs, inj.get("act_eps"), inj.get("elite_pos"), inj.get("state_eps"))
         self._dkl_calls = getattr(self, "_dkl_calls", 0) + 1
-        if self._dist is not None:        # obs_batch is this rank's block of the calibration batch
-            self._shard_base(obs.shape[0])
+        self._shard_base(obs.shape[0])    # obs_batch is this rank's block of the calibration batch
         bufs.run(env.env_cfg(True), uncertainty_mode=False, seed=(self.seed << 20) + (1 << 19) + self._dkl_calls,
                  path_id_base=self.path_id_base, max_steps=depth)
-        st = bufs.step_stats.cpu().numpy()[:depth]
-        if self._dist is not None:
-            st = rank_order_sum(self._gather(np.ascontiguousarray(st[:, 0:2])))
+        st = self._step_stats(bufs, depth)
         self._total_dkl += float(st[:, 1].sum())
         self._total_samples += int(st[:, 0].sum())
         return self.dyn_dkl * depth
 
     # ---- reset (model_sampler.py:203-237) ----------------------------------------------------
     def _require_fused_if_distributed(self):
-        if self._dist is not None and not self.fused:
+        if self._ranks.sharded and not self.fused:
             raise L.CmbpoError("a multi-rank ModelSampler runs the fused mode only: the step-wise mode "
                                "(external policy objects) runs on one rank")
 
@@ -162,11 +162,9 @@ class ModelSampler:
         if not (on_device and self.fused):
             observations = np.asarray(observations.cpu() if on_device else observations, np.float32)
         self.batch_size = observations.shape[0]
-        self._batch_total = self.batch_size
         self._global_sums = None
         self._require_fused_if_distributed()
-        if self._dist is not None:
-            _, self._batch_total = self._shard_base(self.batch_size)
+        self._batch_total = self._shard_base(self.batch_size)
         self._current_observation = observations
         self.policy.reset()
         self.pool.reset(self.batch_size)
@@ -214,20 +212,20 @@ class ModelSampler:
         """(rows alive at the start of step t, of which cut as too uncertain at t, survivors)."""
         if self._hist is None:                      # first use after reset(): waits for the rollout
             self._hist = self._histogram()
-            st = self.pool.bufs.step_stats.cpu().numpy()
-            if self._dist is not None:
-                st = rank_order_sum(self._gather(np.ascontiguousarray(st[:, 0:2])))
-            self._step_stats_host = st
+            self._step_stats_host = self._step_stats(self.pool.bufs)
         h_len, h_unc = self._hist
         longer = int(h_len[t + 1:].sum())
         return longer + int(h_unc[t]), int(h_unc[t]), longer
 
+    def _step_stats(self, bufs, steps=None):
+        """(rows fed, sum of their disagreement) of each step (step_stats[:, 0:2]), summed over the ranks."""
+        st = bufs.step_stats.cpu().numpy()[:steps]
+        return rank_order_sum(self._gather(np.ascontiguousarray(st[:, 0:2])))
+
     def _histogram(self):
-        """The length histograms of the batch (cmbpo_rollout_histogram); after distribute(), summed over the
-        ranks, with the ranks' own length histograms kept in self._rank_h_len for the cap split."""
+        """The length histograms of the batch (cmbpo_rollout_histogram), summed over the ranks, with the ranks'
+        own length histograms kept in self._rank_h_len for the cap split."""
         h_len, h_unc = self.pool.bufs.histogram()
-        if self._dist is None:
-            return h_len, h_unc
         g = self._gather(np.concatenate([h_len, h_unc]))
         self._rank_h_len = g[:, :len(h_len)]
         s = rank_order_sum(g)
@@ -241,11 +239,8 @@ class ModelSampler:
         if max_samples:                                           # model_sampler.py:282-287
             n = max(self._total_samples + alive0 - uncertain - max_samples, 0)
             n = min(n, survivors)
-            if n > 0:
-                if self._dist is None:
-                    cut = n
-                else:       # the first n survivors of the whole batch: this rank's share of them
-                    cut = cap_split(n, self._rank_h_len[:, t + 1:].sum(axis=1))[self._dist["rank"]]
+            if n > 0:       # the first n survivors of the whole batch: this rank's share of them
+                cut = cap_split(n, self._rank_h_len[:, t + 1:].sum(axis=1))[self._ranks.rank]
                 if cut > 0:
                     bufs.truncate(cap_step=t, cap_n=cut)
                 self._hist = self._histogram()
@@ -283,16 +278,15 @@ class ModelSampler:
         self._path_return = bufs.path_return.cpu().numpy()
         self._path_cost = bufs.path_cost.cpu().numpy()
         max_len = int(bufs.length.max().item()) if B else 0
-        if self._dist is not None:
-            # sums over the ranks in rank order, maxima over the ranks: the same dict on every rank
-            sums = ("rew", "cost", "val", "cval", "dyn_error", "n")
-            v = np.array([d[k] for k in sums] + [self.pool.size, self._path_return.sum(), self._path_cost.sum(),
-                                                 d["max_dkl"], d["max_path_return"], max_len], np.float64)
-            g = self._gather(v)
-            s, m = rank_order_sum(g), g.max(axis=0)
-            d.update(zip(sums, (float(x) for x in s[:6])))
-            self._global_sums = (int(s[6]), float(s[7]), float(s[8]))
-            d["max_dkl"], d["max_path_return"], max_len = float(m[9]), float(m[10]), int(m[11])
+        # sums over the ranks in rank order, maxima over the ranks: the same dict on every rank
+        sums = ("rew", "cost", "val", "cval", "dyn_error", "n")
+        v = np.array([d[k] for k in sums] + [self.pool.size, self._path_return.sum(), self._path_cost.sum(),
+                                             d["max_dkl"], d["max_path_return"], max_len], np.float64)
+        g = self._gather(v)
+        s, m = rank_order_sum(g), g.max(axis=0)
+        d.update(zip(sums, (float(x) for x in s[:6])))
+        self._global_sums = (int(s[6]), float(s[7]), float(s[8]))
+        d["max_dkl"], d["max_path_return"], max_len = float(m[9]), float(m[10]), int(m[11])
         self._total_rew, self._total_cost = d["rew"], d["cost"]
         self._total_Vs, self._total_CVs = d["val"], d["cval"]
         self._total_dyn_ep_var = d["dyn_error"] * bufs.O

@@ -5,9 +5,17 @@ normalisation and the populated-mask flatten of get() in cmbpo_adv_* / cmbpo_com
 import numpy as np
 
 from . import _lib as L
+from .dist import Ranks
 from .rollout import RolloutBuffers
 
 EPS = 1e-8
+
+# The 12 arrays of get() in the reference's order (modelbuffer.py:184-226; log_std and mu are the sorted pi_info
+# keys): the RolloutBuffers field and the ModelBuffer attribute that gives its row width, None for one scalar
+# per row (a 1-D array).
+FIELDS = (("obs", "obs_dim"), ("act", "act_dim"), ("adv", None), ("cadv", None), ("ret", None), ("cret", None),
+          ("logp", None), ("val", None), ("cval", None), ("cost", None), ("log_std", "act_dim"), ("mu", "act_dim"))
+LOG_STD = [name for name, _ in FIELDS].index("log_std")
 
 
 class ModelBuffer:
@@ -23,7 +31,7 @@ class ModelBuffer:
         self.pi_info_shapes = None
         self.gamma, self.lam, self.cost_gamma, self.cost_lam = 0.99, 0.95, 0.99, 0.95
         self.reduce_fn = None        # set by the multi-GPU wrapper: all-reduce of the statistics
-        self._dist = None            # distribute(): get() gathers the whole batch on one rank
+        self._ranks = Ranks()        # the ranks get() gathers the batch from: this process alone until distribute()
         self.reset()
 
     def initialize(self, pi_info_shapes, gamma=0.99, lam=0.95, cost_gamma=0.99, cost_lam=0.95):
@@ -44,8 +52,6 @@ class ModelBuffer:
         self.max_size = np.ones(self.batch_size) * self.max_path_length
         self.terminated_paths_mask = np.zeros(self.batch_size, dtype=bool)
         self._length = np.zeros(self.batch_size, dtype=np.int32)   # host mirror (step-wise mode)
-        self._last_val = np.zeros(self.batch_size, dtype=np.float32)
-        self._last_cval = np.zeros(self.batch_size, dtype=np.float32)
         self._device_lengths = False     # True once a fused rollout owns length/last_val on device
         self._log_std_row = None
 
@@ -123,7 +129,6 @@ class ModelBuffer:
             lc = np.zeros(self.batch_size, np.float32)
             lv[fin] = np.asarray(last_val, np.float32)
             lc[fin] = np.asarray(last_cval, np.float32)
-            self._last_val[fin], self._last_cval[fin] = lv[fin], lc[fin]
             b = self.bufs
             e.gae_paths(b.rew, b.val, b.cost, b.cval, e.to_device(len_now, t.int32),
                         e.to_device(lv), e.to_device(lc), self.gamma, self.lam, self.cost_gamma,
@@ -148,47 +153,53 @@ class ModelBuffer:
         """Every rank of `group` holds a contiguous block of one batch's paths (rank order = path order):
         the advantage statistics are all-reduced, and get() / get_device() return the rows of the WHOLE batch,
         in global path order, on rank `root` (group rank) and arrays with zero rows on the other ranks.  The
-        diagnostics are the batch's on every rank.  Called by ModelSampler.distribute."""
-        import torch.distributed as dist
+        diagnostics are the batch's on every rank.  Without distribute() the same code gathers from this
+        process alone.  Called by ModelSampler.distribute."""
         from .dist import make_reduce_fn
         self.reduce_fn = make_reduce_fn(group)
-        self._dist = dict(group=group, root=int(root), rank=dist.get_rank(group))
+        self._ranks = Ranks.of(group, root)
 
-    def _gather_rows(self, fields, off, n_rows):
-        """The compacted `fields` ((field, width, vector) as get_device compacts them) of every rank, in rank
-        order, into fresh [N_total, ...] tensors on the root: the root compacts its own rows straight into its
-        slice of them; the other ranks compact into their persistent staging and send it; the root receives
-        straight into the final slices (one batch of point-to-point operations: no padding, no reassembly copy).
-        Over gloo (ranks that share a GPU) the messages are host copies.
-        Returns (the tensors -- zero rows off the root --, the row count of the whole batch)."""
+    def _gather_rows(self, off, n_rows, staging_gen):
+        """The compacted rows of the FIELDS (log_std aside) of every rank, in rank order, as [N_total, ...] tensors
+        on the root: persistent staging of generation `staging_gen` when given, else fresh tensors.  The root
+        compacts its own rows straight into its slice of them; the other ranks compact into their persistent
+        staging and send it; the root receives straight into the final slices (one batch of point-to-point
+        operations: no padding, no reassembly copy).  Over gloo (ranks that share a GPU) the messages are host
+        copies.  A single rank compacts its rows and exchanges nothing.
+        Returns (the tensors -- zero rows off the root, None at LOG_STD --, the row count of the whole batch)."""
         import torch.distributed as dist
-        from .dist import all_gather_host
-        e, ds, b = self.engine, self._dist, self.bufs
-        group, root, rank = ds["group"], ds["root"], ds["rank"]
-        nccl = dist.get_backend(group) == "nccl"
-        landed = []                         # gloo: (device slice, host message)
-        counts = all_gather_host(np.array([n_rows], np.int64), group, e.device)[:, 0]
+        e, b, r = self.engine, self.bufs, self._ranks
+        counts = r.gather(np.array([n_rows], np.int64), e.device)[:, 0]
         starts = np.concatenate([[0], np.cumsum(counts)])
-        n_out = int(starts[-1]) if rank == root else 0
-        out, ops = [], []
-        for i, (f, width, vector) in enumerate(fields):
+        root = r.rank == r.root
+        n_out = int(starts[-1]) if root else 0
+        nccl = r.world > 1 and dist.get_backend(r.group) == "nccl"
+        out, ops, landed = [], [], []       # landed (gloo): (device slice, host message)
+        for i, (name, dim) in enumerate(FIELDS):
+            if i == LOG_STD:
+                out.append(None)
+                continue
+            width, vector = (getattr(self, dim), True) if dim else (1, False)
+
             def compact(dst):
-                return e.compact(f, self.batch_size, self.max_path_length, width, b.length, off, n_rows, dst)
-            if rank == root:
+                return e.compact(getattr(b, name), self.batch_size, self.max_path_length, width, b.length, off,
+                                 n_rows, dst)
+            if staging_gen is not None:
+                full = self._staging(staging_gen, i, n_out, width, vector)
+            else:
                 full = e.empty(n_out, width) if vector else e.empty(n_out)
-                compact(full[starts[rank]:starts[rank + 1]])
-                for g in range(len(counts)):
-                    if g != rank and counts[g]:
+            if root:
+                compact(full[starts[r.rank]:starts[r.rank + 1]])
+                for g in range(r.world):
+                    if g != r.rank and counts[g]:
                         dst = full[starts[g]:starts[g + 1]]
                         msg = dst if nccl else e.torch.empty(dst.shape, dtype=dst.dtype)
-                        ops.append(dist.P2POp(dist.irecv, msg, group=group, group_peer=g))
+                        ops.append(dist.P2POp(dist.irecv, msg, group=r.group, group_peer=g))
                         if not nccl:
                             landed.append((dst, msg))
-            else:
-                full = e.empty(0, width) if vector else e.empty(0)
-                if n_rows:
-                    msg = compact(self._staging("send", i, n_rows, width, vector))
-                    ops.append(dist.P2POp(dist.isend, msg if nccl else msg.cpu(), group=group, group_peer=root))
+            elif n_rows:
+                msg = compact(self._staging("send", i, n_rows, width, vector))
+                ops.append(dist.P2POp(dist.isend, msg if nccl else msg.cpu(), group=r.group, group_peer=r.root))
             out.append(full)
         if ops:
             for req in dist.batch_isend_irecv(ops):
@@ -211,11 +222,20 @@ class ModelBuffer:
         flat = buf[:n_rows * width]
         return flat.view(n_rows, width) if vector else flat
 
+    def _log_std_host(self):
+        """A [1, A] float32 copy of the row every row of log_std repeats (one variable, ac_network.py:119):
+        this batch's policy row, zeros before anything was stored."""
+        row = self._log_std_row if self._log_std_row is not None else np.zeros(self.act_dim, np.float32)
+        return np.array(row, np.float32).reshape(1, self.act_dim)
+
     def get_device(self, staging_gen=None):
-        """get() without the device->host copy: (list of 12 device tensors, diagnostics).  With
+        """get() without the device->host copy: (list of the 12 device tensors of FIELDS, diagnostics).  With
         `staging_gen` (0 | 1) the tensors are views of persistent buffers of that generation, valid
         until the second next call with the same generation."""
         assert self.terminated_paths_mask.all()
+        if staging_gen is not None and self._ranks.sharded:
+            raise L.CmbpoError("the persistent staging of get_async() is for one rank only; after "
+                               "distribute() use get()")
         e, t, b = self.engine, self.engine.torch, self.bufs
         B, T = self.batch_size, self.max_path_length
         if not self._device_lengths:
@@ -227,31 +247,10 @@ class ModelBuffer:
         off = e.path_offsets(b.length)
         n_rows = int(off[-1].item())
         st = e.stats_from_sums(sums.cpu().numpy())
-        O, A = self.obs_dim, self.act_dim
-        if self._dist is not None:
-            if staging_gen is not None:
-                raise L.CmbpoError("the persistent staging of get_async() is for one rank only; after "
-                                   "distribute() use get()")
-            vec, sc = (lambda f, w: (f, w, True)), (lambda f: (f, 1, False))
-            fields = [vec(b.obs, O), vec(b.act, A)] + [sc(f) for f in (b.adv, b.cadv, b.ret, b.cret, b.logp, b.val,
-                                                                       b.cval, b.cost)] + [vec(b.mu, A)]
-            full, n_rows = self._gather_rows(fields, off, n_rows)
-            out, mu = full[:10], full[10]
-            n_out = mu.shape[0]
-        else:
-            def tgt(i, width, vector):
-                return None if staging_gen is None else self._staging(staging_gen, i, n_rows, width, vector)
-
-            out = [e.compact(b.obs, B, T, O, b.length, off, n_rows, tgt(0, O, True)),
-                   e.compact(b.act, B, T, A, b.length, off, n_rows, tgt(1, A, True))]
-            for i, f in enumerate((b.adv, b.cadv, b.ret, b.cret, b.logp, b.val, b.cval, b.cost)):
-                out.append(e.compact(f, B, T, 1, b.length, off, n_rows, tgt(2 + i, 1, False)))
-            mu = e.compact(b.mu, B, T, A, b.length, off, n_rows, tgt(11, A, True))
-            n_out = n_rows
-        ls_row = self._log_std_row if self._log_std_row is not None else np.zeros(A, np.float32)
-        # every row of log_std is the same [A] variable (ac_network.py:119): a stride-0 view
-        log_std = e.to_device(ls_row, t.float32).reshape(1, A).expand(n_out, A)
-        out += [log_std, mu]                       # sorted pi_info keys: log_std, mu
+        out, n_rows = self._gather_rows(off, n_rows, staging_gen)
+        n_out = out[0].shape[0]
+        # every row of log_std is the same [A] variable: a stride-0 view
+        out[LOG_STD] = e.to_device(self._log_std_host(), t.float32).expand(n_out, self.act_dim)
         diag = dict(poolm_batch_size=n_rows, poolm_ret_mean=st["ret_mean"],
                     poolm_cret_mean=st["cret_mean"])
         return out, diag
@@ -264,31 +263,19 @@ class ModelBuffer:
         recycled under the caller.  When the caller drops an array its block goes back to torch's caching host
         allocator, so in steady state (cmbpo.py:270 concatenates the arrays and drops them) no page is pinned or
         faulted again: ~50 GB/s instead of the ~3 GB/s of fresh pageable arrays.  `pinned=False`: plain pageable
-        `.cpu()` copies."""
+        host tensors."""
         out, diag = self.get_device()
         res = self.to_host(out, pinned)
         self.reset()
         return res, diag
 
     def to_host(self, out, pinned=True):
-        """The device->host half of get(): the 12 device tensors of get_device() as numpy arrays."""
-        # log_std (index 10) is one [A] row repeated: it crosses PCIe once and is returned as a
-        # read-only broadcast view (values, shape and dtype as the reference's array)
-        ls_host = np.broadcast_to(out[10][:1].cpu().numpy().reshape(1, -1) if out[10].shape[0] else
-                                  np.zeros((1, self.act_dim), np.float32), tuple(out[10].shape))
-        if not pinned:
-            return [ls_host if i == 10 else x.cpu().numpy() for i, x in enumerate(out)]
+        """The device->host half of get(): the 12 device tensors of get_device() as numpy arrays.  Call it
+        before the next reset(): log_std comes from this batch's host row."""
         t = self.engine.torch
-        host = []
-        for i, x in enumerate(out):
-            if i == 10:
-                host.append(None)
-                continue
-            h = t.empty(tuple(x.shape), dtype=x.dtype, pin_memory=True)
-            h.copy_(x, non_blocking=True)
-            host.append(h)
+        host = _copy_to_host(out, lambda i, x: t.empty(tuple(x.shape), dtype=x.dtype, pin_memory=pinned))
         t.cuda.current_stream(self.engine.device).synchronize()
-        return [ls_host if h is None else h.numpy() for h in host]
+        return _numpy_arrays(host, self._log_std_host())
 
     def get_async(self):
         """`get()` split in two so that the device->host copy of this batch overlaps the NEXT
@@ -297,7 +284,7 @@ class ModelBuffer:
         engine's stream, the copies into page-locked buffers are queued on a side stream, the buffer
         resets.  Returns a handle whose `result()` waits for the copies and returns exactly what
         `get()` returns.  At most two handles may be outstanding (two pinned buffer sets).  One rank only."""
-        if self._dist is not None:
+        if self._ranks.sharded:
             raise L.CmbpoError("get_async() runs on one rank only; after distribute() use get()")
         self._pin_gen = getattr(self, "_pin_gen", 0) ^ 1
         t, dev = self.engine.torch, self.engine.device
@@ -307,43 +294,58 @@ class ModelBuffer:
         if prev is not None:
             t.cuda.current_stream(dev).wait_event(prev)
         out, diag = self.get_device(staging_gen=self._pin_gen)
-        ls_row = out[10][:1].cpu().numpy().reshape(1, -1) if out[10].shape[0] else np.zeros((1, self.act_dim), np.float32)
-        ls_host = np.broadcast_to(ls_row, tuple(out[10].shape))
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = t.cuda.Stream(device=dev)
         pool = self.__dict__.setdefault("_pin_pool", {})
+
+        def pinned(i, x):                           # the page-locked buffer of this generation and field
+            key = (self._pin_gen, i)
+            buf = pool.get(key)
+            if buf is None or buf.numel() < x.numel() or buf.dtype != x.dtype:
+                buf = t.empty(max(x.numel(), 1), dtype=x.dtype, pin_memory=True)
+                pool[key] = buf
+            return buf[:x.numel()].view(x.shape)
+
         main = t.cuda.current_stream(dev)
         ready = t.cuda.Event()
         ready.record(main)                          # compaction kernels of this batch are queued
-        host = []
         with t.cuda.stream(self._copy_stream):
             self._copy_stream.wait_event(ready)
-            for i, x in enumerate(out):
-                if i == 10:
-                    host.append(None)
-                    continue
-                key = (self._pin_gen, i)
-                buf = pool.get(key)
-                if buf is None or buf.numel() < x.numel() or buf.dtype != x.dtype:
-                    buf = t.empty(max(x.numel(), 1), dtype=x.dtype, pin_memory=True)
-                    pool[key] = buf
-                h = buf[:x.numel()].view(x.shape)
-                h.copy_(x, non_blocking=True)       # x: persistent staging buffer of this generation
-                host.append(h)
+            host = _copy_to_host(out, pinned)       # out: persistent staging buffers of this generation
             done = t.cuda.Event()
             done.record(self._copy_stream)
         self._gen_done[self._pin_gen] = done
+        res = PendingGet(done, host, self._log_std_host(), diag, out)
         self.reset()
-        return PendingGet(done, host, ls_host, diag, out)
+        return res
+
+
+def _copy_to_host(out, host_like):
+    """Queue on the current stream one device->host copy of each of get_device()'s tensors but log_std, into
+    `host_like(i, x)` (a host tensor of x's shape and dtype).  Returns the host tensors, None at LOG_STD."""
+    host = [None] * len(out)
+    for i, x in enumerate(out):
+        if i != LOG_STD:
+            host[i] = host_like(i, x)
+            host[i].copy_(x, non_blocking=True)
+    return host
+
+
+def _numpy_arrays(host, log_std_row):
+    """get()'s 12 numpy arrays from the host tensors of _copy_to_host: log_std is the [1, A] row as a read-only
+    broadcast view (values, shape and dtype as the reference's array; it crossed PCIe once, as an upload)."""
+    rows = host[0].shape[0]
+    return [np.broadcast_to(log_std_row, (rows, log_std_row.shape[1])) if i == LOG_STD else h.numpy()
+            for i, h in enumerate(host)]
 
 
 class PendingGet:
     """Handle of `ModelBuffer.get_async()`."""
 
-    def __init__(self, done, host, ls_host, diag, keep_alive):
-        self._done, self._host, self._ls, self._diag, self._keep = done, host, ls_host, diag, keep_alive
+    def __init__(self, done, host, log_std_row, diag, keep_alive):
+        self._done, self._host, self._ls, self._diag, self._keep = done, host, log_std_row, diag, keep_alive
 
     def result(self):
         self._done.synchronize()
         self._keep = None
-        return [self._ls if h is None else h.numpy() for h in self._host], self._diag
+        return _numpy_arrays(self._host, self._ls), self._diag
