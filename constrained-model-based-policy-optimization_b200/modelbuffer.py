@@ -151,10 +151,10 @@ class ModelBuffer:
     # ---- multi-GPU ---------------------------------------------------------------------------
     def distribute(self, group=None, root=0):
         """Every rank of `group` holds a contiguous block of one batch's paths (rank order = path order):
-        the advantage statistics are all-reduced, and get() / get_device() return the rows of the WHOLE batch,
-        in global path order, on rank `root` (group rank) and arrays with zero rows on the other ranks.  The
-        diagnostics are the batch's on every rank.  Without distribute() the same code gathers from this
-        process alone.  Called by ModelSampler.distribute."""
+        the advantage statistics are all-reduced, and get() / get_device() / get_async() return the rows of the
+        WHOLE batch, in global path order, on rank `root` (group rank) and arrays with zero rows on the other
+        ranks.  The diagnostics are the batch's on every rank.  Without distribute() the same code gathers from
+        this process alone.  Called by ModelSampler.distribute."""
         from .dist import make_reduce_fn
         self.reduce_fn = make_reduce_fn(group)
         self._ranks = Ranks.of(group, root)
@@ -166,6 +166,12 @@ class ModelBuffer:
         staging and send it; the root receives straight into the final slices (one batch of point-to-point
         operations: no padding, no reassembly copy).  Over gloo (ranks that share a GPU) the messages are host
         copies.  A single rank compacts its rows and exchanges nothing.
+        Every write into the returned tensors is ordered before what the caller queues next on the current
+        stream: the compaction runs on it, req.wait() of an NCCL receive makes it wait for NCCL's stream, and the
+        gloo messages land through copies on it.  The NCCL operations themselves start only after what the
+        current stream had queued before this call.  A non-root rank reuses its single "send" staging in its
+        next compaction, which is ordered after the send: by req.wait() over NCCL, and over gloo because the
+        message is a synchronous host copy of it.
         Returns (the tensors -- zero rows off the root, None at LOG_STD --, the row count of the whole batch)."""
         import torch.distributed as dist
         e, b, r = self.engine, self.bufs, self._ranks
@@ -184,7 +190,7 @@ class ModelBuffer:
             def compact(dst):
                 return e.compact(getattr(b, name), self.batch_size, self.max_path_length, width, b.length, off,
                                  n_rows, dst)
-            if staging_gen is not None:
+            if staging_gen is not None and root:
                 full = self._staging(staging_gen, i, n_out, width, vector)
             else:
                 full = e.empty(n_out, width) if vector else e.empty(n_out)
@@ -210,14 +216,15 @@ class ModelBuffer:
 
     # ---- get ---------------------------------------------------------------------------------
     def _staging(self, gen, i, n_rows, width, vector):
-        """Persistent compaction target (generation `gen`, field `i`), sized for a full buffer: no
-        allocator traffic per batch (a fresh 500 MB of tensors per batch makes the caching allocator
-        call cudaMalloc / cudaFree, which synchronise the device at unpredictable moments)."""
+        """Persistent compaction target (generation `gen`, field `i`), sized for a full buffer of this rank and
+        grown when `n_rows` is more (the root of a sharded block holds the rows of every rank): no allocator
+        traffic per batch (a fresh 500 MB of tensors per batch makes the caching allocator call cudaMalloc /
+        cudaFree, which synchronise the device at unpredictable moments)."""
         pool = self.__dict__.setdefault("_compact_pool", {})
-        cap = self.batch_size * self.max_path_length
+        need = max(self.batch_size * self.max_path_length, n_rows) * width
         buf = pool.get((gen, i))
-        if buf is None or buf.numel() < cap * width:
-            buf = self.engine.empty(cap * width)
+        if buf is None or buf.numel() < need:
+            buf = self.engine.empty(need)
             pool[(gen, i)] = buf
         flat = buf[:n_rows * width]
         return flat.view(n_rows, width) if vector else flat
@@ -231,11 +238,9 @@ class ModelBuffer:
     def get_device(self, staging_gen=None):
         """get() without the device->host copy: (list of the 12 device tensors of FIELDS, diagnostics).  With
         `staging_gen` (0 | 1) the tensors are views of persistent buffers of that generation, valid
-        until the second next call with the same generation."""
+        until the second next call with the same generation.  After distribute(), the root's tensors hold the
+        whole batch and the other ranks' have zero rows (never staging)."""
         assert self.terminated_paths_mask.all()
-        if staging_gen is not None and self._ranks.sharded:
-            raise L.CmbpoError("the persistent staging of get_async() is for one rank only; after "
-                               "distribute() use get()")
         e, t, b = self.engine, self.engine.torch, self.bufs
         B, T = self.batch_size, self.max_path_length
         if not self._device_lengths:
@@ -283,17 +288,27 @@ class ModelBuffer:
         concatenates their sample lists): statistics / normalisation / compaction run now on the
         engine's stream, the copies into page-locked buffers are queued on a side stream, the buffer
         resets.  Returns a handle whose `result()` waits for the copies and returns exactly what
-        `get()` returns.  At most two handles may be outstanding (two pinned buffer sets).  One rank only."""
-        if self._ranks.sharded:
-            raise L.CmbpoError("get_async() runs on one rank only; after distribute() use get()")
+        `get()` returns.  At most two handles may be outstanding (two pinned buffer sets).
+
+        After distribute() the root's handle returns the whole batch in global path order, the other ranks' return
+        zero-row arrays at once (they copy nothing and wait for nothing of the root), and the diagnostics are the
+        same on every rank.  Like get(), this is a sequence of collectives (the statistics all-reduces, the row
+        count gather, the point-to-point batch): every rank calls get_async() and the rest of the block in the same
+        order."""
         self._pin_gen = getattr(self, "_pin_gen", 0) ^ 1
         t, dev = self.engine.torch, self.engine.device
         # the staging / pinned buffers of this generation may still be read by the copy of the handle
-        # issued two calls ago: the compaction kernels below must not start before that copy finished
+        # issued two calls ago: the compaction kernels and the receives below (NCCL's stream waits for the
+        # current stream when they are queued) must not start before that copy finished
         prev = self.__dict__.setdefault("_gen_done", {}).get(self._pin_gen)
         if prev is not None:
             t.cuda.current_stream(dev).wait_event(prev)
         out, diag = self.get_device(staging_gen=self._pin_gen)
+        if self._ranks.rank != self._ranks.root:
+            host = [None if i == LOG_STD else t.empty(tuple(x.shape), dtype=x.dtype) for i, x in enumerate(out)]
+            res = PendingGet(None, host, self._log_std_host(), diag, None)
+            self.reset()
+            return res
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = t.cuda.Stream(device=dev)
         pool = self.__dict__.setdefault("_pin_pool", {})
@@ -307,15 +322,18 @@ class ModelBuffer:
             return buf[:x.numel()].view(x.shape)
 
         main = t.cuda.current_stream(dev)
-        ready = t.cuda.Event()
-        ready.record(main)                          # compaction kernels of this batch are queued
+        # recorded after get_device() returned: behind this batch's compaction kernels and, on the root of a
+        # sharded block, behind the receives of the other ranks' rows (NCCL: req.wait() made the current stream
+        # wait for them; gloo: they landed through copies on it), so the copies below read complete rows
+        ready = t.cuda.Event(enable_timing=True)
+        ready.record(main)
         with t.cuda.stream(self._copy_stream):
             self._copy_stream.wait_event(ready)
             host = _copy_to_host(out, pinned)       # out: persistent staging buffers of this generation
-            done = t.cuda.Event()
+            done = t.cuda.Event(enable_timing=True)
             done.record(self._copy_stream)
         self._gen_done[self._pin_gen] = done
-        res = PendingGet(done, host, self._log_std_host(), diag, out)
+        res = PendingGet(done, host, self._log_std_host(), diag, out, ready)
         self.reset()
         return res
 
@@ -340,12 +358,21 @@ def _numpy_arrays(host, log_std_row):
 
 
 class PendingGet:
-    """Handle of `ModelBuffer.get_async()`."""
+    """Handle of `ModelBuffer.get_async()`.  `done` None: nothing was copied (a non-root rank of a sharded block)."""
 
-    def __init__(self, done, host, log_std_row, diag, keep_alive):
+    def __init__(self, done, host, log_std_row, diag, keep_alive, ready=None):
         self._done, self._host, self._ls, self._diag, self._keep = done, host, log_std_row, diag, keep_alive
+        self._ready = ready
 
     def result(self):
-        self._done.synchronize()
+        if self._done is not None:
+            self._done.synchronize()
         self._keep = None
         return _numpy_arrays(self._host, self._ls), self._diag
+
+    def copy_ms(self):
+        """Device time (ms) from the end of the batch's compaction and receives to the end of its device->host
+        copy, None when nothing was copied.  Call after result()."""
+        if self._done is None:
+            return None
+        return self._ready.elapsed_time(self._done)
