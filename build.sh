@@ -9,7 +9,7 @@ NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -Wall --expt-relaxed-constexpr"
 mkdir -p build
 objs=""
-for f in capi gae ens_f32 ens_tc rollout policy_pack archive train; do
+for f in capi gae ens_f32 ens_tc rollout policy_pack archive train train_tc; do
   if [ ! -f build/$f.o ] || [ $SRC/$f.cu -nt build/$f.o ] || [ -n "$(find $SRC include -name '*.cuh' -newer build/$f.o -o -name '*.h' -newer build/$f.o)" ]; then
     echo "nvcc $f.cu"
     $NVCC $FLAGS ${PTXAS_V:+-Xptxas -v} -c $SRC/$f.cu -o build/$f.o

@@ -47,6 +47,8 @@ class RolloutCfg(C.Structure):
 
 ROLLOUT_NO_COMPACT, ROLLOUT_FUSE, ROLLOUT_NO_STORE = 1, 2, 4
 LOSS_MSPE, LOSS_MSE = 0, 1
+TRAIN_FP32, TRAIN_TF32, TRAIN_BF16 = 0, 1, 2
+TRAIN_MATHS = {"fp32": TRAIN_FP32, "tf32": TRAIN_TF32, "bf16": TRAIN_BF16}
 
 
 class TrainCfg(C.Structure):

@@ -93,6 +93,7 @@ struct cmbpo_ctx {
     cudaEvent_t n_ev[4] = {nullptr, nullptr, nullptr, nullptr};
     // ensemble training (train.cu): optimiser state, activations and the cuBLAS handle per network slot
     void* train[CMBPO_NET_COUNT] = {nullptr};
+    bool train_tc_smem_set[3] = {false, false, false};   // cudaFuncSetAttribute made for the bf16 GEMM kernels
 };
 
 // grow-only scratch

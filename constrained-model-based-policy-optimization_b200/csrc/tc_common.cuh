@@ -210,6 +210,18 @@ __host__ __device__ constexpr uint32_t idesc_f16(int fmt, int n) {
            ((uint32_t)(128 >> 4) << 24);
 }
 
+// the same panel bytes read MN-major: a panel row is then 64 consecutive M (or N) elements at one K index,
+// 8 K rows form one 1024-byte swizzle atom (SBO = 1024 B between 8-K groups), and the next 64 M / N elements
+// sit `lbo_bytes` further on (canonical layout ((8,8,m),(8,k)) : ((1,8,LBO),(64,SBO)) in 16-bit elements)
+__device__ __forceinline__ uint64_t smem_desc_sw128_mn(uint32_t smem_addr, uint32_t lbo_bytes) {
+    return (uint64_t)((smem_addr & 0x3FFFFu) >> 4) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) | (64ull << 32) |
+           (1ull << 46) | (2ull << 61);
+}
+// idesc_f16 with the operand majors chosen: a_mn / b_mn = 1 reads A / B MN-major (bits 15 / 16)
+__host__ __device__ constexpr uint32_t idesc_f16_major(int fmt, int n, int a_mn, int b_mn) {
+    return idesc_f16(fmt, n) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16);
+}
+
 // byte offset of 16-byte chunk `c` (elements 8c..8c+7) of row `r` inside a swizzled panel
 __host__ __device__ constexpr uint32_t panel_off(int r, int c) {
     return (uint32_t)((r >> 3) * 1024 + (r & 7) * 128 + ((c ^ (r & 7)) << 4));

@@ -5,14 +5,14 @@
 // and tf.train.AdamOptimizer's update.
 //
 // The dense contractions (forward, dW = A^T dZ, dA = dZ W^T; batched over the E members) are plain library GEMMs:
-// cublasSgemmStridedBatched, on the tensor cores when `math` = 1 (TF32) -- this row is a consumer-side widening,
-// not the rollout hot path, and has no fusion a library GEMM would prevent.  Everything around them is fused into
+// cublasSgemmStridedBatched, on the tensor cores when `math` = 1 (TF32).  Everything around them is fused into
 // a few element-wise kernels of our own: input scaling, bias + activation (keeping the pre-activations), the loss
 // and its output gradient (two passes: the loss couples all members through one scalar ratio), activation
-// backward, bias gradients (column sums), decay + Adam.
+// backward, bias gradients (column sums), decay + Adam.  `math` = 2 (bf16) runs the same step on the tcgen05
+// GEMMs of train_tc.cu, which fuse that element-wise work into their prologues and epilogues (step_bf16 below).
 #include <cublas_v2.h>
 
-#include "common.cuh"
+#include "train.cuh"
 
 namespace {
 
@@ -29,6 +29,16 @@ struct TrainState {
     double* sums = nullptr;               // [E][3] loss sums + scratch
     float* loss = nullptr;                // [E]
     cublasHandle_t blas = nullptr;
+    // bf16 step (train_tc.cu): panel images of the operands, sized for cap_bs16 rows
+    uint8_t* w16[ML] = {};                // bf16 copy of W_l
+    bool w16_fresh = false;               // w16 equals the master weights rounded (only bf16 steps keep it so)
+    int64_t cap_bs16 = 0;
+    uint8_t* xs16 = nullptr;              // scaled inputs
+    uint8_t* h16[ML] = {};                // hidden activations
+    uint8_t* g16[2] = {};                 // pre-activation gradients, ping-pong
+    float* part[2] = {};                  // per-row-tile column sums of g16 [E, row tiles, width], ping-pong
+    float* z16[ML] = {};                  // fp32 pre-activations [E, bs, width] (the fp32 path's z is not shared)
+    double* lpart = nullptr;              // loss pass 1's per-block sums [E, loss blocks, 3]
 };
 
 #define BLAS_TRY(expr)                                                                     \
@@ -36,28 +46,6 @@ struct TrainState {
         cublasStatus_t st_ = (expr);                                                       \
         if (st_ != CUBLAS_STATUS_SUCCESS) { cmbpo_set_error("cuBLAS error %d at %s:%d", (int)st_, __FILE__, __LINE__); return 1; } \
     } while (0)
-
-__device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
-
-__device__ __forceinline__ float act_fwd(int act, float x) {
-    switch (act) {
-        case CMBPO_ACT_SWISH: return x * sigmoidf_(x);          // fc.py:19
-        case CMBPO_ACT_TANH: return tanhf(x);
-        case CMBPO_ACT_RELU: return fmaxf(x, 0.f);
-        case CMBPO_ACT_SIGMOID: return sigmoidf_(x);
-        default: return x;
-    }
-}
-
-__device__ __forceinline__ float act_bwd(int act, float x) {
-    switch (act) {
-        case CMBPO_ACT_SWISH: { const float s = sigmoidf_(x); return s * (1.0f + x * (1.0f - s)); }
-        case CMBPO_ACT_TANH: { const float t = tanhf(x); return 1.0f - t * t; }
-        case CMBPO_ACT_RELU: return x > 0.f ? 1.0f : 0.f;
-        case CMBPO_ACT_SIGMOID: { const float s = sigmoidf_(x); return s * (1.0f - s); }
-        default: return 1.0f;
-    }
-}
 
 // pens/utils.py:156 on [E, bs, in]
 __global__ void scale_in_kernel(const float* __restrict__ x, const float* __restrict__ mu, const float* __restrict__ sig,
@@ -78,22 +66,6 @@ __global__ void bias_act_kernel(float* __restrict__ z, const float* __restrict__
         z[i] = v;
         if (h) h[i] = act_fwd(act, v);
     }
-}
-
-__device__ __forceinline__ double block_sum_d(double v, double* sh) {
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-    const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-    __syncthreads();
-    if (l == 0) sh[w] = v;
-    __syncthreads();
-    double s = 0;
-    if (threadIdx.x < 32) {
-        s = (threadIdx.x < (blockDim.x >> 5)) ? sh[threadIdx.x] : 0.0;
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
-    }
-    return s;       // valid in thread 0
 }
 
 // Loss pass 1, grid.y = member.  MSPE (pe.py:945-971): s = (mean - y~)^2, q = (exp(logvar) - s)^2, logvar^2;
@@ -218,6 +190,36 @@ int ensure_buffers(cmbpo_ctx* ctx, Net& n, TrainState* st, int64_t bs) {
     return 0;
 }
 
+int ensure_buffers_bf16(cmbpo_ctx* ctx, Net& n, TrainState* st, int64_t bs) {
+    using namespace train_tc;
+    if (!st->w16[0]) {
+        for (int l = 0; l < n.n_layers; ++l) CUDA_TRY(cudaMalloc(&st->w16[l], w16_bytes(n.E, n.dims[l], n.dims[l + 1])));
+        CUDA_TRY(cudaMalloc(&st->lpart, (size_t)n.E * MAX_LOSS_BLOCKS * 3 * sizeof(double)));
+        st->w16_fresh = false;
+    }
+    if (rows_pad(bs) <= st->cap_bs16) return 0;
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    auto re = [&](void** p, size_t bytes) -> int {
+        if (*p) cudaFree(*p);
+        *p = nullptr;
+        CUDA_TRY(cudaMalloc(p, bytes));
+        return 0;
+    };
+    int maxw = 0;
+    for (int l = 0; l < n.n_layers; ++l) maxw = std::max(maxw, n.dims[l + 1]);
+    if (re((void**)&st->xs16, act_bytes(n.E, bs, n.dims[0]))) return 1;
+    for (int l = 0; l < n.n_layers; ++l) {
+        if (l + 1 < n.n_layers && re((void**)&st->h16[l], act_bytes(n.E, bs, n.dims[l + 1]))) return 1;
+        if (re((void**)&st->z16[l], (size_t)n.E * rows_pad(bs) * n.dims[l + 1] * sizeof(float))) return 1;
+    }
+    for (int i = 0; i < 2; ++i) {
+        if (re((void**)&st->g16[i], act_bytes(n.E, bs, maxw))) return 1;
+        if (re((void**)&st->part[i], (size_t)n.E * row_tiles(bs) * maxw * sizeof(float))) return 1;
+    }
+    st->cap_bs16 = rows_pad(bs);
+    return 0;
+}
+
 // C[e] (m x n, row-major) = op(A[e]) op(B[e]); row-major operands handed to column-major cuBLAS as transposes
 int gemm_nn(TrainState* st, int E, int m, int n, int k, const float* A, const float* B, float* C) {       // C = A[m,k] B[k,n]
     const float one = 1.f, zero = 0.f;
@@ -267,6 +269,43 @@ int check_net(cmbpo_ctx* ctx, int which, int64_t bs) {
     return 0;
 }
 
+// the bf16 step (train_tc.cu header): 3L + 2 launches, L more when W16 has to be rebuilt first
+int step_bf16(cmbpo_ctx* ctx, Net& n, TrainState* st, const float* x, const float* y, int64_t bs,
+              const cmbpo_train_cfg* cfg, float* loss_out) {
+    if (ensure_buffers_bf16(ctx, n, st, bs)) return 1;
+    const int L = n.n_layers, W = n.dims[L], prob = n.probabilistic ? 1 : 0;
+    if (!st->w16_fresh) {
+        for (int l = 0; l < L; ++l)
+            if (train_tc::pack_w16(ctx, n.W[l], n.E, n.dims[l], n.dims[l + 1], st->w16[l])) return 1;
+        st->w16_fresh = true;
+    }
+    if (train_tc::scale_in(ctx, x, n.has_in ? n.mu_in : nullptr, n.sig_in, n.E, bs, n.dims[0], st->xs16)) return 1;
+    for (int l = 0; l < L; ++l) {
+        const uint8_t* a = l == 0 ? st->xs16 : st->h16[l - 1];
+        if (train_tc::forward(ctx, n.E, bs, n.dims[l], n.dims[l + 1], a, st->w16[l], n.b[l], n.acts[l], st->z16[l],
+                              l + 1 < L ? st->h16[l] : nullptr)) return 1;
+    }
+    const float* mu_o = n.has_out ? n.mu_out : nullptr;
+    int gi = 0;
+    if (train_tc::loss_grad(ctx, st->z16[L - 1], y, mu_o, n.sig_out, bs, n.D, W, prob, n.E, st->lpart,
+                            loss_out ? loss_out : st->loss, st->g16[gi], st->part[gi])) return 1;
+    st->step += 1;
+    const double t = (double)st->step;
+    const float lr_t = (float)((double)cfg->lr * sqrt(1.0 - pow((double)cfg->beta2, t)) / (1.0 - pow((double)cfg->beta1, t)));
+    for (int l = L - 1; l >= 0; --l) {
+        const int K = n.dims[l], H = n.dims[l + 1];
+        if (l > 0 && train_tc::data_grad(ctx, n.E, bs, K, H, st->g16[gi], st->w16[l], st->z16[l - 1], n.acts[l - 1],
+                                         st->g16[gi ^ 1], st->part[gi ^ 1])) return 1;
+        const train_tc::Adam opt = {lr_t, cfg->beta1, cfg->beta2, cfg->eps, cfg->weight_decay[l]};
+        if (train_tc::weight_grad_adam(ctx, n.E, bs, K, H, l == 0 ? st->xs16 : st->h16[l - 1], st->g16[gi], st->part[gi],
+                                       n.W[l], st->mW[l], st->vW[l], st->gW[l], n.b[l], st->mb[l], st->vb[l], st->gb[l],
+                                       st->w16[l], opt)) return 1;
+        gi ^= 1;
+    }
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace
 
 void train_free(cmbpo_ctx* ctx, int which) {
@@ -275,10 +314,16 @@ void train_free(cmbpo_ctx* ctx, int which) {
     for (int l = 0; l < ML; ++l) {
         float* p[] = {st->mW[l], st->vW[l], st->mb[l], st->vb[l], st->gW[l], st->gb[l], st->z[l], st->h[l]};
         for (float* q : p) if (q) cudaFree(q);
+        if (st->w16[l]) cudaFree(st->w16[l]);
+        if (st->h16[l]) cudaFree(st->h16[l]);
+        if (st->z16[l]) cudaFree(st->z16[l]);
     }
-    float* p[] = {st->xs, st->da, st->db_, st->loss};
+    float* p[] = {st->xs, st->da, st->db_, st->loss, st->part[0], st->part[1]};
     for (float* q : p) if (q) cudaFree(q);
+    uint8_t* p16[] = {st->xs16, st->g16[0], st->g16[1]};
+    for (uint8_t* q : p16) if (q) cudaFree(q);
     if (st->sums) cudaFree(st->sums);
+    if (st->lpart) cudaFree(st->lpart);
     if (st->blas) cublasDestroy(st->blas);
     delete st;
     ctx->train[which] = nullptr;
@@ -336,6 +381,10 @@ extern "C" int cmbpo_ens_train_step(cmbpo_ctx* ctx, int which, const float* x, c
     const int prob = n.probabilistic ? 1 : 0;
     CMBPO_CHECK((cfg->loss == CMBPO_LOSS_MSPE && prob) || (cfg->loss == CMBPO_LOSS_MSE && !prob),
                 "loss %d does not fit this network (MSPE: probabilistic, MSE: not)", cfg->loss);
+    CMBPO_CHECK(cfg->math == CMBPO_TRAIN_FP32 || cfg->math == CMBPO_TRAIN_TF32 || cfg->math == CMBPO_TRAIN_BF16,
+                "math %d is not one of 0 (fp32), 1 (TF32), 2 (bf16)", cfg->math);
+    if (cfg->math == CMBPO_TRAIN_BF16) return step_bf16(ctx, n, st, x, y, bs, cfg, loss_out);
+    st->w16_fresh = false;                           // this step moves the master weights away from W16
     if (ensure_buffers(ctx, n, st, bs)) return 1;
     BLAS_TRY(cublasSetStream(st->blas, ctx->stream));
     BLAS_TRY(cublasSetMathMode(st->blas, cfg->math ? CUBLAS_TF32_TENSOR_OP_MATH : CUBLAS_DEFAULT_MATH));

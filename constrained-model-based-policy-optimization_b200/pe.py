@@ -104,7 +104,9 @@ class B200PE:
         """What `build_PE` fixes at construction (pe_factory.py:9-60): loss type ('MSPE' for the probabilistic
         dynamics ensemble, 'MSE' for value ensembles), Adam learning rate, weight decay (first layer decay/4,
         hidden layers decay/2, last layer decay), which scalers `train` re-fits.  `math`: 'fp32' | 'tf32'
-        (tensor-core GEMMs)."""
+        (tensor-core GEMMs) | 'bf16' (tcgen05 GEMMs on bf16 operands, fp32 accumulation and optimiser state)."""
+        if math not in L.TRAIN_MATHS:
+            raise ValueError("math must be one of %s, not %r" % (", ".join(L.TRAIN_MATHS), math))
         if loss is None:
             loss = "MSPE" if self._probabilistic else "MSE"
         assert loss in ("MSPE", "MSE"), "losses of the CMBPO configs: MSPE (dynamics), MSE (V / VC)"
@@ -114,7 +116,7 @@ class B200PE:
         cfg.lr, cfg.beta1, cfg.beta2, cfg.eps = float(lr), 0.9, 0.999, 1e-8
         for l in range(nl):
             cfg.weight_decay[l] = float(decay / 4 if l == 0 else (decay if l == nl - 1 else decay / 2))
-        cfg.math = 1 if math == "tf32" else 0
+        cfg.math = L.TRAIN_MATHS[math]
         self._train_cfg = cfg
         self._use_scaler_in, self._use_scaler_out = bool(use_scaler_in), bool(use_scaler_out)
         self._scaler_cache = {"in": (0, None, None), "out": (0, None, None)}

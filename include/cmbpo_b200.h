@@ -319,7 +319,10 @@ int cmbpo_adv_normalise(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths
  *                inc_var_loss=False); weight_decay[l] multiplies tf.nn.l2_loss(W_l) (fc.py:168-169;
  *                pe_factory.py:50-55: decay/4, decay/2 ..., decay).  loss_out (device, [E], may be NULL): the
  *                per-member loss vector the reference's loss function returns (before decay).
- *                math: 0 = fp32 GEMMs, 1 = TF32 tensor-core GEMMs (cuBLAS).
+ *                math: CMBPO_TRAIN_FP32 = fp32 GEMMs, CMBPO_TRAIN_TF32 = TF32 tensor-core GEMMs (cuBLAS),
+ *                CMBPO_TRAIN_BF16 = tcgen05 GEMMs on bf16 operands (xs, W, hidden activations and pre-activation
+ *                gradients rounded to bf16; fp32 accumulation, loss, gradients, master weights and Adam state;
+ *                csrc/train_tc.cu).  Any other value is an error.
  *   train_loss   `self.loss` of the reference (pe.py:264): mean 0.5 (mean - transform(y))^2 per member, no update.
  *   train_grads  device copies of the last step's gradients of one layer (before decay): dW [E,in,out], db [E,out].
  *   train_end    installs new elites (NULL keeps them) and re-packs the tcgen05 weight streams: predictions and
@@ -328,6 +331,7 @@ int cmbpo_adv_normalise(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths
  *                (TensorStandardScaler.fit, pens/utils.py:119-138; host pointers).
  */
 enum { CMBPO_LOSS_MSPE = 0, CMBPO_LOSS_MSE = 1 };
+enum { CMBPO_TRAIN_FP32 = 0, CMBPO_TRAIN_TF32 = 1, CMBPO_TRAIN_BF16 = 2 };
 typedef struct {
     int loss;
     float lr, beta1, beta2, eps;       /* tf.train.AdamOptimizer: 1e-3 (cmbpo.py:51), 0.9, 0.999, 1e-8 */
