@@ -24,8 +24,8 @@ from . import statics
 from . import dist
 from . import checkpoint
 from .archive import DeviceArchive
-from .checkpoint import load_pe, load_policy
+from .checkpoint import load_pe, load_policy, load_state, save_state, write_pe_checkpoint
 from . import tf_bundle
 
-__all__ = ["load_pe", "load_policy", "DeviceArchive", "Engine", "B200PE", "B200Policy", "FakeEnv", "ModelBuffer", "CPOBuffer", "ModelSampler",
+__all__ = ["load_pe", "load_policy", "load_state", "save_state", "write_pe_checkpoint", "DeviceArchive", "Engine", "B200PE", "B200Policy", "FakeEnv", "ModelBuffer", "CPOBuffer", "ModelSampler",
            "RolloutBuffers", "CmbpoError", "LIB_PATH", "statics"]

@@ -98,6 +98,8 @@ SIGNATURES = {
     "cmbpo_ens_train_loss": (_i, [_vp, _i, _vp, _vp, _i64, _vp]),
     "cmbpo_ens_train_grads": (_i, [_vp, _i, _i, _vp, _vp]),
     "cmbpo_ens_train_end": (_i, [_vp, _i, _vp, _i]),
+    "cmbpo_ens_train_state_get": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, C.POINTER(_i64)]),
+    "cmbpo_ens_train_state_set": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, _i64]),
     "cmbpo_net_get_weights": (_i, [_vp, _i, _i, _vp, _vp]),
     "cmbpo_net_set_scalers": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "cmbpo_path_offsets": (_i, [_vp, _vp, _i64, _vp]),

@@ -53,6 +53,36 @@ class DeviceArchive:
         self.max_pointer = max(self.archive_ptr, self.max_pointer)
         self._index = None
 
+    # ---- checkpoint and resume (checkpoint.save_state / load_state) ----------------------------
+    def state_dict(self):
+        """Rows [0, max_pointer) of the four columns (the rows past it were never written), the ring pointer, the seed
+        and the draw counter that key the Philox draws."""
+        n = self.max_pointer
+        return {"precision": self.engine.precision_name, "archive_size": self.archive_size, "obs_dim": self.obs_dim,
+                "act_dim": self.act_dim, "observations": self.observations[:n].cpu().numpy(),
+                "mu": self.mu[:n].cpu().numpy(), "log_std": self.log_std[:n].cpu().numpy(),
+                "epoch_archive": self.epoch_archive[:n].cpu().numpy(), "archive_ptr": self.archive_ptr,
+                "max_pointer": n, "seed": self.seed, "draw": self._draw}
+
+    @classmethod
+    def from_state_dict(cls, engine, sd):
+        """The inverse of state_dict(); the epoch index is rebuilt at the first draw."""
+        engine.check_precision(sd["precision"])
+        self = cls(engine, sd["archive_size"], sd["obs_dim"], sd["act_dim"], seed=sd["seed"])
+        n, t = int(sd["max_pointer"]), engine.torch
+        if not 0 <= int(sd["archive_ptr"]) <= n <= self.archive_size:
+            raise ValueError("archive pointers %s / %s in an archive of %d rows"
+                             % (sd["archive_ptr"], n, self.archive_size))
+        for name, width in (("observations", self.obs_dim), ("mu", self.act_dim), ("log_std", self.act_dim),
+                            ("epoch_archive", None)):
+            shape = (n,) if width is None else (n, width)
+            if tuple(sd[name].shape) != shape:
+                raise ValueError("archive column %s is %s, want %s" % (name, tuple(sd[name].shape), shape))
+            if n:
+                getattr(self, name)[:n] = engine.to_device(sd[name], t.int32 if width is None else t.float32)
+        self.archive_ptr, self.max_pointer, self._draw = int(sd["archive_ptr"]), n, int(sd["draw"])
+        return self
+
     # ---- index by epoch ----------------------------------------------------------------------
     def _build_index(self):
         if self._index is not None:

@@ -1,5 +1,10 @@
-"""Loader for the reference's PE checkpoints (SURVEY.md section 8f-3), so ensembles trained by the
-TF code base can drive the B200 rollout.
+"""Checkpoints: the native state file that resumes a run, and the reference's PE checkpoints (SURVEY.md
+section 8f-3) in both directions, so that ensembles trained by the TF code base can drive the B200 rollout
+and ensembles trained here can go back to it.
+
+`save_state` / `load_state` write and read one `.npz` holding a nested dict of numpy arrays and plain values:
+the `state_dict()` of B200PE, B200Policy, DeviceArchive and ModelSampler, and whatever else the caller adds
+(the numpy random state its training loop draws from, say).  See INTEGRATION.md, "Checkpoint and resume".
 
 `PE.save` (models/pens/pe.py:736-764) writes two files per model:
   * `<name>_<timestep>.nns`  -- one `repr(FC)` per layer (models/pens/fc.py:46-50), the last one with
@@ -9,15 +14,115 @@ TF code base can drive the B200 rollout.
     (pe.py:203-213, pens/utils.py:189-194); optvars = per layer (weights [E,in,out], biases
     [E,1,out]) (fc.py:172-175), then (max_logvar, min_logvar) only for the NLL loss.
 Elite indices are not part of the checkpoint (they are recomputed by `PE.train`, pe.py:396-399):
-pass them in.
+pass them in.  `write_pe_checkpoint` writes the same two files (PE.save does not write the Adam slots
+either).
 """
+import json
 import os
 import re
+import zipfile
 
 import numpy as np
 
-from .pe import B200PE
+from .pe import B200PE, layer_decays
 
+# ---- the native state file --------------------------------------------------------------------------------------
+STATE_FORMAT = 1
+_VERSION_KEY, _META_KEY = "format_version", "meta"
+
+
+def _encode(node, arrays, path):
+    """The JSON description of `node`; its arrays (numpy scalars as 0-d arrays) go to `arrays` as (entry, array)."""
+    if isinstance(node, dict):
+        for k in node:
+            if not isinstance(k, str):
+                raise TypeError("%s: key %r is not a string" % (path or "state", k))
+        return {"dict": {k: _encode(v, arrays, path + "/" + k) for k, v in node.items()}}
+    if isinstance(node, list):
+        return {"list": [_encode(v, arrays, "%s/%d" % (path, i)) for i, v in enumerate(node)]}
+    if isinstance(node, (np.ndarray, np.generic)):
+        a = np.asarray(node)
+        arrays.append(("a%d" % len(arrays), a))
+        return {"array": arrays[-1][0], "shape": list(a.shape), "dtype": a.dtype.str,
+                "scalar": isinstance(node, np.generic)}
+    if node is None or isinstance(node, (bool, int, float, str)):
+        return {"value": node}
+    raise TypeError("%s: cannot save a %s" % (path or "state", type(node).__name__))
+
+
+def _decode(node, z, path):
+    if not isinstance(node, dict):
+        raise ValueError("%s: malformed metadata" % (path or "state"))
+    if "dict" in node:
+        return {k: _decode(v, z, path + "/" + k) for k, v in node["dict"].items()}
+    if "list" in node:
+        return [_decode(v, z, "%s/%d" % (path, i)) for i, v in enumerate(node["list"])]
+    if "value" in node:
+        return node["value"]
+    if not {"array", "shape", "dtype", "scalar"} <= set(node):
+        raise ValueError("%s: malformed metadata" % (path or "state"))
+    if node["array"] not in z.files:
+        raise ValueError("%s: the array is missing from the file" % path)
+    a = z[node["array"]]
+    if list(a.shape) != node["shape"] or a.dtype.str != node["dtype"]:
+        raise ValueError("%s: array of shape %s / %s, recorded %s / %s"
+                         % (path, list(a.shape), a.dtype.str, node["shape"], node["dtype"]))
+    return a[()] if node["scalar"] else a
+
+
+def save_state(path, state):
+    """Write the nested dict `state` to `path` (.npz): dicts with string keys, lists, numpy arrays and scalars, and
+    None / bool / int / float / str leaves.  Arrays are stored bit for bit and read back without pickle; the other
+    leaves and the tree go to a JSON entry.  The file is written beside `path` and moved over it with os.replace
+    once complete, so an interrupted save leaves the previous checkpoint intact."""
+    if not isinstance(state, dict):
+        raise TypeError("the state is a dict, not a %s" % type(state).__name__)
+    arrays = []
+    meta = json.dumps(_encode(state, arrays, ""))
+    entries = [(_VERSION_KEY, np.array(STATE_FORMAT, np.int64)),
+               (_META_KEY, np.frombuffer(meta.encode("utf-8"), np.uint8))] + arrays
+    tmp = "%s.tmp%d" % (path, os.getpid())
+    try:
+        with open(tmp, "wb") as f:
+            with zipfile.ZipFile(f, "w", zipfile.ZIP_STORED, allowZip64=True) as zf:
+                for name, a in entries:
+                    with zf.open(name + ".npy", "w", force_zip64=True) as fh:
+                        np.lib.format.write_array(fh, a, allow_pickle=False)
+            f.flush()
+            os.fsync(f.fileno())
+        os.replace(tmp, path)
+    except BaseException:
+        if os.path.exists(tmp):
+            os.unlink(tmp)
+        raise
+    try:                                     # make the rename itself durable
+        fd = os.open(os.path.dirname(os.path.abspath(path)), os.O_RDONLY)
+    except OSError:
+        return
+    try:
+        os.fsync(fd)
+    except OSError:
+        pass
+    finally:
+        os.close(fd)
+
+
+def load_state(path):
+    """The nested dict save_state() wrote.  Raises ValueError on an unknown format version, an array the metadata
+    names that is missing, or an array whose shape or dtype differs from the recorded one."""
+    with np.load(path, allow_pickle=False) as z:
+        if _VERSION_KEY not in z.files or _META_KEY not in z.files:
+            raise ValueError("%s is not a state file (no %s / %s entry)" % (path, _VERSION_KEY, _META_KEY))
+        version = z[_VERSION_KEY]
+        if version.shape != () or int(version) != STATE_FORMAT:
+            raise ValueError("%s: unknown state format version %s (this code reads %d)" % (path, version, STATE_FORMAT))
+        tree = json.loads(z[_META_KEY].tobytes().decode("utf-8"))
+        if "dict" not in tree:
+            raise ValueError("%s: malformed metadata" % path)
+        return _decode(tree, z, "")
+
+
+# ---- the reference's PE checkpoint ------------------------------------------------------------------------------
 _FC = re.compile(r"FC\(output_dim=(?P<out>\d+), input_dim=(?P<inp>None|\d+), activation=(?P<act>None|'[^']*'|\"[^\"]*\"), "
                  r"weight_decay=(?P<wd>[^,]+), ensemble_size=(?P<E>\d+)\)")
 
@@ -102,6 +207,40 @@ def read_pe_checkpoint(model_dir, name, timestep):
         raise ValueError("%s.mat: %d leading arrays are not a set of scalers" % (stem, n_scal))
     return dict(W=W, b=b, acts=acts, probabilistic=probabilistic, mu_in=mu_in, var_in=var_in,
                 mu_out=mu_out, var_out=var_out, max_logvar=bounds[0], min_logvar=bounds[1])
+
+
+def _fc_repr(output_dim, input_dim, activation, weight_decay, ensemble_size):
+    """FC.__repr__ (models/pens/fc.py:46-50)."""
+    return "FC(output_dim=%r, input_dim=%r, activation=%r, weight_decay=%r, ensemble_size=%r)" % (
+        output_dim, input_dim, activation, weight_decay, ensemble_size)
+
+
+def write_pe_checkpoint(model_dir, name, timestep, pe):
+    """`PE.save` (pe.py:736-764) of a B200PE (or of the dict its state_dict() returns), readable by the reference's
+    `PE(load_model=True)` and by read_pe_checkpoint / load_pe: `<name>_<timestep>.nns` with one FC line per layer
+    (weight decay from configure_training's `decay`, None when training was never configured) and
+    `<name>_<timestep>.mat` with the scalers in use, then W [E,in,out] and b [E,1,out] per layer."""
+    from scipy.io import savemat
+
+    sd = pe.state_dict() if hasattr(pe, "state_dict") else pe
+    layers = sd["layers"]
+    n_l, E = len(layers), int(layers[0]["W"].shape[0])
+    decays = layer_decays(sd["train"]["decay"], n_l) if sd.get("train") else [None] * n_l
+    lines = []
+    for l, (x, act, wd) in enumerate(zip(layers, sd["acts"], decays)):
+        out = int(x["W"].shape[2])
+        if l == n_l - 1 and sd["probabilistic"]:
+            out //= 2                                  # pe.py:179-180: the layer was declared with the mean width
+        lines.append(_fc_repr(out, int(x["W"].shape[1]), act, wd, E) + "\n")
+    sc = sd["scalers"]
+    arrs = [np.asarray(sc[k], np.float32).reshape(1, -1)
+            for pair in (("mu_in", "var_in"), ("mu_out", "var_out")) if sc[pair[0]] is not None for k in pair]
+    for x in layers:
+        arrs += [np.asarray(x["W"], np.float32), np.asarray(x["b"], np.float32).reshape(E, 1, -1)]
+    stem = os.path.join(model_dir, "%s_%s" % (name, timestep))
+    with open(stem + ".nns", "w") as f:
+        f.writelines(lines)
+    savemat(stem + ".mat", {str(i): a for i, a in enumerate(arrs)})
 
 
 def load_pe(engine, which, model_dir, name, timestep, elite_inds=None):

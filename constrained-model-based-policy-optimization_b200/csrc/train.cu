@@ -441,6 +441,46 @@ extern "C" int cmbpo_ens_train_grads(cmbpo_ctx* ctx, int which, int layer, float
     return 0;
 }
 
+// checkpointing: one layer's Adam moments and the slot's step counter (the bias correction of lr_t depends on it)
+extern "C" int cmbpo_ens_train_state_get(cmbpo_ctx* ctx, int which, int layer, float* mW, float* vW, float* mb, float* vb,
+                                         int64_t* step_host) {
+    CMBPO_CHECK(ctx && which >= 0 && which < CMBPO_NET_COUNT, "bad arguments");
+    Net& n = ctx->nets[which];
+    CMBPO_CHECK(n.loaded, "network %d not loaded", which);
+    CMBPO_CHECK(layer >= 0 && layer < n.n_layers, "bad layer");
+    TrainState* st = state_of(ctx, which);
+    if (!st) {
+        if (step_host) *step_host = -1;
+        return 0;
+    }
+    const size_t nw = (size_t)n.E * n.dims[layer] * n.dims[layer + 1] * sizeof(float), nb = (size_t)n.E * n.dims[layer + 1] * sizeof(float);
+    if (mW) CUDA_TRY(cudaMemcpyAsync(mW, st->mW[layer], nw, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (vW) CUDA_TRY(cudaMemcpyAsync(vW, st->vW[layer], nw, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (mb) CUDA_TRY(cudaMemcpyAsync(mb, st->mb[layer], nb, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (vb) CUDA_TRY(cudaMemcpyAsync(vb, st->vb[layer], nb, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (step_host) *step_host = st->step;
+    return 0;
+}
+
+extern "C" int cmbpo_ens_train_state_set(cmbpo_ctx* ctx, int which, int layer, const float* mW, const float* vW,
+                                         const float* mb, const float* vb, int64_t step) {
+    CMBPO_CHECK(ctx && which >= 0 && which < CMBPO_NET_COUNT, "bad arguments");
+    Net& n = ctx->nets[which];
+    CMBPO_CHECK(n.loaded, "network %d not loaded", which);
+    CMBPO_CHECK(layer >= 0 && layer < n.n_layers, "bad layer");
+    CMBPO_CHECK(step >= 0, "bad step count %lld", (long long)step);
+    if (cmbpo_ens_train_begin(ctx, which)) return 1;
+    TrainState* st = state_of(ctx, which);
+    const size_t nw = (size_t)n.E * n.dims[layer] * n.dims[layer + 1] * sizeof(float), nb = (size_t)n.E * n.dims[layer + 1] * sizeof(float);
+    if (mW) CUDA_TRY(cudaMemcpyAsync(st->mW[layer], mW, nw, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (vW) CUDA_TRY(cudaMemcpyAsync(st->vW[layer], vW, nw, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (mb) CUDA_TRY(cudaMemcpyAsync(st->mb[layer], mb, nb, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (vb) CUDA_TRY(cudaMemcpyAsync(st->vb[layer], vb, nb, cudaMemcpyDeviceToDevice, ctx->stream));
+    st->step = step;
+    st->w16_fresh = false;                           // the next bf16 step re-packs W16 from the master weights
+    return 0;
+}
+
 extern "C" int cmbpo_net_get_weights(cmbpo_ctx* ctx, int which, int layer, float* W, float* b) {
     CMBPO_CHECK(ctx && which >= 0 && which < CMBPO_NET_COUNT, "bad arguments");
     Net& n = ctx->nets[which];

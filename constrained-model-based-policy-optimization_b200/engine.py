@@ -14,6 +14,15 @@ def _as_f32(a):
     return np.ascontiguousarray(np.asarray(a, dtype=np.float32))
 
 
+def _host_row(a):
+    """A [1, n] float32 host copy of a scaler vector (numpy array or tensor), None for None."""
+    if a is None:
+        return None
+    if hasattr(a, "is_cuda"):
+        a = a.detach().cpu().numpy()
+    return _as_f32(a).reshape(1, -1).copy()
+
+
 class Engine:
     def __init__(self, device=0, precision="fp32"):
         import torch
@@ -94,6 +103,17 @@ class Engine:
         L.check(self.lib.cmbpo_ctx_synchronize(self.h))
 
     @property
+    def precision_name(self):
+        return {v: k for k, v in L.PRECISIONS.items()}[self.precision]
+
+    def check_precision(self, recorded):
+        """Refuse state saved from an Engine of another rollout precision: resumed on this one, the run would not
+        continue the rollouts it was doing."""
+        if recorded != self.precision_name:
+            raise ValueError("the state was saved at rollout precision %r, this Engine runs %r"
+                             % (recorded, self.precision_name))
+
+    @property
     def launch_count(self):
         return int(self.lib.cmbpo_ctx_launch_count(self.h))
 
@@ -142,8 +162,13 @@ class Engine:
             C.c_void_p(sc[0]), C.c_void_p(sc[1]), C.c_void_p(sc[2]), C.c_void_p(sc[3]),
             int(bool(probabilistic)), elp, len(elite), int(on_device)))
         last = dims[-1]
+        # the scalers as uploaded (the library keeps sigma = max(sqrt(var), 1e-2), not the variance): checkpoints
+        # write these
+        scalers = {k: _host_row(a) for k, a in zip(("mu_in", "var_in", "mu_out", "var_out"),
+                                                   (mu_in, var_in, mu_out, var_out))}
         self.nets[which] = dict(E=E, dims=dims, D=last // 2 if probabilistic else last,
-                                probabilistic=bool(probabilistic), elite_inds=elite)
+                                probabilistic=bool(probabilistic), elite_inds=elite, acts=list(acts),
+                                scalers=scalers)
 
     # ------------------------------------------------------------------ ensemble training (SURVEY.md 8f-4)
     def train_begin(self, which):
@@ -185,6 +210,32 @@ class Engine:
         keep = [None if a is None else _as_f32(np.asarray(a).reshape(-1)) for a in (mu_in, var_in, mu_out, var_out)]
         p = [C.c_void_p(None if a is None else a.ctypes.data) for a in keep]
         L.check(self.lib.cmbpo_net_set_scalers(self.h, which, *p))
+        sc = self.nets[which]["scalers"]
+        for k, a in zip(("mu_in", "var_in", "mu_out", "var_out"), (mu_in, var_in, mu_out, var_out)):
+            if a is not None:
+                sc[k] = _host_row(a)
+
+    def train_state_get(self, which, layer):
+        """Checkpointing: ((mW, vW, mb, vb) device tensors, step count) of one layer of slot `which`'s optimiser
+        state, or (None, -1) when the slot has none."""
+        m = self.nets[which]
+        E, K, H = m["E"], m["dims"][layer], m["dims"][layer + 1]
+        mom = (self.empty(E, K, H), self.empty(E, K, H), self.empty(E, H), self.empty(E, H))
+        step = C.c_int64()
+        L.check(self.lib.cmbpo_ens_train_state_get(self.h, which, layer, *(self._p(x) for x in mom), C.byref(step)))
+        return (mom if step.value >= 0 else None), step.value
+
+    def train_state_set(self, which, layer, mW, vW, mb, vb, step):
+        """Restore one layer's Adam moments and the slot's step count (creating the optimiser state if absent).
+        Call after set_network, which drops the optimiser state."""
+        t = self.torch
+        m = self.nets[which]
+        E, K, H = m["E"], m["dims"][layer], m["dims"][layer + 1]
+        mom = [self.to_device(x, t.float32) for x in (mW, vW, mb, vb)]
+        for x, shape in zip(mom, ((E, K, H), (E, K, H), (E, H), (E, H))):
+            if tuple(x.shape) != shape:
+                raise ValueError("Adam moment of shape %s for layer %d of shape %s" % (tuple(x.shape), layer, shape))
+        L.check(self.lib.cmbpo_ens_train_state_set(self.h, which, layer, *(self._p(x) for x in mom), int(step)))
 
     def train_end(self, which, elite_inds=None):
         el = None if elite_inds is None else [int(i) for i in elite_inds]

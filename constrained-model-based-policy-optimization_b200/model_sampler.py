@@ -95,6 +95,29 @@ class ModelSampler:
         self._auto_base = self.path_id_base
         self.pool.distribute(group, root)
 
+    # ---- checkpoint and resume (checkpoint.save_state / load_state) ----------------------------
+    def state_dict(self):
+        """The counters that key the rollouts' Philox draws (seed, resets, calibration calls) and the settings of the
+        sampler.  Take it between batches: it raises while reset() has started a batch that get() has not returned.
+        The sample and disagreement totals are kept too: compute_dynamics_dkl adds to them until the next reset().
+        The ranks of distribute() are a runtime object and are not saved: call distribute() again after loading."""
+        if self.pool is not None and self.pool.holds_batch:
+            raise L.CmbpoError("a rollout batch is in flight: take the state after the pool's get()")
+        return {"seed": self.seed, "resets": self._resets, "dkl_calls": getattr(self, "_dkl_calls", 0),
+                "max_path_length": self._max_path_length,
+                "dkl_lim": None if self.dkl_lim is None else float(self.dkl_lim), "batch_size": self.batch_size,
+                "rollout_mode": self.rollout_mode, "total_samples": int(self._total_samples),
+                "total_dkl": float(self._total_dkl)}
+
+    @classmethod
+    def from_state_dict(cls, sd):
+        """The inverse of state_dict(); then initialize() (and distribute()) as for a new sampler."""
+        self = cls(sd["max_path_length"], sd["batch_size"], sd["rollout_mode"], seed=sd["seed"])
+        self._resets, self._dkl_calls = int(sd["resets"]), int(sd["dkl_calls"])
+        self.dkl_lim = sd["dkl_lim"]
+        self._total_samples, self._total_dkl = int(sd["total_samples"]), float(sd["total_dkl"])
+        return self
+
     def _gather(self, vec):
         """[world, ...] all-gather of a small host vector, rank order."""
         return self._ranks.gather(vec, self.pool.engine.device)

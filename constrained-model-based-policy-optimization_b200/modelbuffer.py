@@ -77,6 +77,11 @@ class ModelBuffer:
     def alive_paths(self):
         return np.logical_not(self.terminated_paths_mask)
 
+    @property
+    def holds_batch(self):
+        """True from a rollout into this buffer until get() / get_async() returns it and resets."""
+        return self._device_lengths or self.ptr > 0
+
     def __getattr__(self, name):
         # reference attribute names, e.g. obs_buf / adv_buf / term_buf, as [B, T, ...] numpy copies
         table = {"obs_buf": "obs", "act_buf": "act", "nextobs_buf": "nextobs", "rew_buf": "rew",

@@ -9,6 +9,14 @@ import numpy as np
 
 from . import _lib as L
 
+_MOMENTS = ("mW", "vW", "mb", "vb")
+
+
+def layer_decays(decay, n_layers):
+    """Per-layer weight decay of build_PE (pe_factory.py:50-55): decay/4 on the first layer, decay on the last,
+    decay/2 in between."""
+    return [float(decay / 4 if l == 0 else (decay if l == n_layers - 1 else decay / 2)) for l in range(n_layers)]
+
 
 class B200PE:
     """One ensemble living in an `Engine` slot (dynamics / V / VC).
@@ -46,6 +54,62 @@ class B200PE:
         self.num_nets, self._in_dim, self._d = meta["E"], meta["dims"][0], meta["D"]
         self._model_inds = list(meta["elite_inds"])
         self.num_elites = len(self._model_inds)
+        return self
+
+    # --- checkpoint and resume (checkpoint.save_state / load_state) ---
+    def state_dict(self):
+        """Everything a resumed run needs to continue this ensemble's training bit for bit, as numpy arrays and plain
+        values: per layer W [E,in,out], b [E,out] and the Adam moments (absent before the first train()), the step
+        count (-1: no optimiser state), the scalers as last uploaded, the elites and the training configuration
+        with the running scaler statistics."""
+        e = self.engine
+        meta = e.nets[self.which]
+        layers, step = [], -1
+        for l in range(len(meta["dims"]) - 1):
+            W, b = e.get_weights(self.which, l)
+            mom, step = e.train_state_get(self.which, l)
+            layer = {"W": W.cpu().numpy(), "b": b.cpu().numpy()}
+            if mom is not None:
+                layer.update(zip(_MOMENTS, (x.cpu().numpy() for x in mom)))
+            layers.append(layer)
+        train = None
+        if hasattr(self, "_train_args"):
+            train = dict(self._train_args)
+            train["scaler_cache"] = {k: {"count": int(c), "mean": mu, "var": var}
+                                     for k, (c, mu, var) in self._scaler_cache.items()}
+        return {"name": self.name, "precision": e.precision_name, "dims": list(meta["dims"]),
+                "acts": list(meta["acts"]), "probabilistic": self._probabilistic, "elite_inds": list(self._model_inds),
+                "scalers": dict(meta["scalers"]), "layers": layers, "step": int(step), "train": train}
+
+    @classmethod
+    def from_state_dict(cls, engine, which, sd):
+        """The inverse of state_dict() into slot `which` of `engine`: the weights first (a new set of weights drops the
+        slot's optimiser state), then the optimiser state and the training configuration."""
+        engine.check_precision(sd["precision"])
+        dims, layers = [int(d) for d in sd["dims"]], sd["layers"]
+        E = int(layers[0]["W"].shape[0]) if layers else 0
+        if len(layers) != len(dims) - 1:
+            raise ValueError("%d layers for dims %s" % (len(layers), dims))
+        step = int(sd["step"])
+        for l, layer in enumerate(layers):
+            want = {"W": (E, dims[l], dims[l + 1]), "b": (E, dims[l + 1])}
+            if step >= 0:
+                want.update(mW=want["W"], vW=want["W"], mb=want["b"], vb=want["b"])
+            for k, shape in want.items():
+                if k not in layer or tuple(layer[k].shape) != shape:
+                    raise ValueError("layer %d: %s is %s, dims %s want %s"
+                                     % (l, k, None if k not in layer else tuple(layer[k].shape), dims, shape))
+        sc = sd["scalers"]
+        self = cls(engine, which, [x["W"] for x in layers], [x["b"] for x in layers], sd["acts"], sd["probabilistic"],
+                   sd["elite_inds"], sc["mu_in"], sc["var_in"], sc["mu_out"], sc["var_out"], name=sd["name"])
+        if sd["train"] is not None:
+            args = dict(sd["train"])
+            cache = args.pop("scaler_cache")
+            self.configure_training(**args)
+            self._scaler_cache = {k: (int(c["count"]), c["mean"], c["var"]) for k, c in cache.items()}
+        if step >= 0:
+            for l, x in enumerate(layers):
+                engine.train_state_set(which, l, *(x[k] for k in _MOMENTS), step)
         return self
 
     # --- contract properties (pe.py:401-434) ---
@@ -114,10 +178,12 @@ class B200PE:
         cfg = L.TrainCfg()
         cfg.loss = L.LOSS_MSPE if loss == "MSPE" else L.LOSS_MSE
         cfg.lr, cfg.beta1, cfg.beta2, cfg.eps = float(lr), 0.9, 0.999, 1e-8
-        for l in range(nl):
-            cfg.weight_decay[l] = float(decay / 4 if l == 0 else (decay if l == nl - 1 else decay / 2))
+        for l, wd in enumerate(layer_decays(decay, nl)):
+            cfg.weight_decay[l] = wd
         cfg.math = L.TRAIN_MATHS[math]
         self._train_cfg = cfg
+        self._train_args = dict(loss=loss, lr=float(lr), decay=float(decay), use_scaler_in=bool(use_scaler_in),
+                                use_scaler_out=bool(use_scaler_out), math=math, n_layers=nl)
         self._use_scaler_in, self._use_scaler_out = bool(use_scaler_in), bool(use_scaler_out)
         self._scaler_cache = {"in": (0, None, None), "out": (0, None, None)}
         return self

@@ -44,6 +44,33 @@ class B200Policy:
         self.v = B200PE.from_arrays(self.engine, L.NET_V, v_ens, name="VEnsemble")
         self.vc = B200PE.from_arrays(self.engine, L.NET_VC, vc_ens, name="VCEnsemble")
 
+    # ---- checkpoint and resume (checkpoint.save_state / load_state) ----------------------------
+    def state_dict(self):
+        """The actor (W [in,out], b [out] per layer, log_std), the seed and the call counter that key the actions'
+        Philox draws.  V and VC are not part of it: save them with their own B200PE.state_dict()."""
+        e = self.engine
+        W, b = [], []
+        for l in range(len(e.nets[L.NET_ACTOR]["dims"]) - 1):
+            w, bb = e.get_weights(L.NET_ACTOR, l)
+            W.append(w[0].cpu().numpy())
+            b.append(bb[0].cpu().numpy())
+        return {"precision": e.precision_name, "actor_W": W, "actor_b": b, "log_std": self.log_std.copy(),
+                "seed": self.seed, "calls": self._calls}
+
+    @classmethod
+    def from_state_dict(cls, engine, sd, v=None, vc=None):
+        """The inverse of state_dict().  Restore V and VC first (B200PE.from_state_dict into NET_V / NET_VC) and pass
+        the objects that returns, or leave `v` / `vc` None to attach views of those slots, as attach_loaded does."""
+        engine.check_precision(sd["precision"])
+        if L.NET_V not in engine.nets or L.NET_VC not in engine.nets:
+            raise L.CmbpoError("restore V and VC into the Engine before the policy")
+        self = cls(engine, seed=sd["seed"])
+        self.load_actor(sd["actor_W"], sd["actor_b"], sd["log_std"])
+        self._calls = int(sd["calls"])
+        self.v = v if v is not None else B200PE.view(engine, L.NET_V, name="VEnsemble")
+        self.vc = vc if vc is not None else B200PE.view(engine, L.NET_VC, name="VCEnsemble")
+        return self
+
     def reset(self):
         pass
 

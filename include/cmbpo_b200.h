@@ -329,6 +329,12 @@ int cmbpo_adv_normalise(cmbpo_ctx* ctx, float* adv, float* cadv, int64_t n_paths
  *                rollouts after it see the trained weights (pe.py:396-399, 601-607).
  *   cmbpo_net_get_weights / cmbpo_net_set_scalers: device copies of one layer's variables; new scaler statistics
  *                (TensorStandardScaler.fit, pens/utils.py:119-138; host pointers).
+ *   train_state_get / _set  checkpoint and resume the optimiser state: device copies of one layer's Adam moments
+ *                mW, vW [E,in,out] and mb, vb [E,out] (any pointer may be NULL), and the slot's step count (host).
+ *                _get on a slot without optimiser state sets *step_host = -1 and copies nothing.  _set creates
+ *                the state as train_begin does when it is absent, copies the moments in and sets the step count
+ *                (>= 0); the next bf16 step rebuilds its bf16 weight copy from the master weights.  Restore the
+ *                weights (cmbpo_net_set_weights, which drops the optimiser state) before the state.
  */
 enum { CMBPO_LOSS_MSPE = 0, CMBPO_LOSS_MSE = 1 };
 enum { CMBPO_TRAIN_FP32 = 0, CMBPO_TRAIN_TF32 = 1, CMBPO_TRAIN_BF16 = 2 };
@@ -344,6 +350,10 @@ int cmbpo_ens_train_step(cmbpo_ctx* ctx, int which, const float* x, const float*
 int cmbpo_ens_train_loss(cmbpo_ctx* ctx, int which, const float* x, const float* y, int64_t bs, float* loss_out);
 int cmbpo_ens_train_grads(cmbpo_ctx* ctx, int which, int layer, float* dW, float* db);
 int cmbpo_ens_train_end(cmbpo_ctx* ctx, int which, const int* elite_inds, int n_elite);
+int cmbpo_ens_train_state_get(cmbpo_ctx* ctx, int which, int layer, float* mW, float* vW, float* mb,
+                              float* vb, int64_t* step_host);
+int cmbpo_ens_train_state_set(cmbpo_ctx* ctx, int which, int layer, const float* mW, const float* vW,
+                              const float* mb, const float* vb, int64_t step);
 int cmbpo_net_get_weights(cmbpo_ctx* ctx, int which, int layer, float* W, float* b);
 int cmbpo_net_set_scalers(cmbpo_ctx* ctx, int which, const float* mu_in, const float* var_in,
                           const float* mu_out, const float* var_out);
