@@ -80,9 +80,13 @@ __device__ __forceinline__ void epi_bar() {      // named barrier 1: the 512 epi
     asm volatile("bar.sync 1, 512;" ::: "memory");
 }
 
-// 32 accumulator columns of this thread's row -> (+bias), act -> 16-bit pairs -> 16 TMEM columns.
-// The accumulator buffer is released (`d_empty`) as soon as the values sit in registers; the
-// destination is only waited for (`dst_free`, 0 = none) right before the store.
+// 32 accumulator columns of this thread's row -> (+bias), act -> 16-bit pairs -> 16 TMEM columns, once the
+// accumulator hand-off (`d_full`) has completed.  The columns are loaded as two 16-column halves: the first half's
+// bias adds and MUFUs run while the second half's tcgen05.ld is in flight, and the accumulator buffer is released
+// (`d_empty`) as soon as both halves sit in registers.  The destination is only waited for (`dst_free`, 0 = none)
+// right before the store.  The biases are loaded where they are added: loaded earlier (before the hand-off wait, or
+// between one tcgen05.ld of all 32 columns and its wait) they are 32 more live registers, ptxas spills the drain's
+// state at 112 registers, and K1 / the policy pass measured 5 % / 14-17 % slower.
 //
 // Swish members are packed with their hidden-layer weights and biases HALVED (exact in 16 bits), so the
 // accumulator already holds t = x/2 and swish(x) = t + t tanh t needs one MUFU and one FFMA.  `bias`
@@ -91,38 +95,46 @@ __device__ __forceinline__ void epi_bar() {      // named barrier 1: the 512 epi
 // the MUFU instructions) or is null when the bias rides in the GEMM (layer 0, see `fold`).  ACT == 0: the
 // activation is a per-member runtime value (merged policy ensemble), swish when `rt_swish`, else tanh.
 template <int FMT, int ACT>
-__device__ __forceinline__ void drain32(uint32_t d_addr, const float* bias, uint32_t dst_addr,
-                                        uint32_t d_empty, uint32_t dst_free, uint32_t dst_parity,
+__device__ __forceinline__ void drain32(uint32_t d_full, uint32_t d_parity, uint32_t d_addr, const float* bias,
+                                        uint32_t dst_addr, uint32_t d_empty, uint32_t dst_free, uint32_t dst_parity,
                                         bool rt_swish = false) {
+    mbar_wait_a(d_full, d_parity);
+    tc_fence_after();
     uint32_t r[32];
-    tmem_ld32(d_addr, r);
+    float v[32];
+    auto convert16 = [&](int h) {          // columns h .. h+15: (+bias), activation, in place in v
+#pragma unroll
+        for (int i = h; i < h + 16; i += 4) {
+            if (bias) {
+                const float4 b = *reinterpret_cast<const float4*>(bias + i);
+                v[i] = __uint_as_float(r[i]) + b.x; v[i + 1] = __uint_as_float(r[i + 1]) + b.y;
+                v[i + 2] = __uint_as_float(r[i + 2]) + b.z; v[i + 3] = __uint_as_float(r[i + 3]) + b.w;
+            } else {
+                v[i] = __uint_as_float(r[i]); v[i + 1] = __uint_as_float(r[i + 1]);
+                v[i + 2] = __uint_as_float(r[i + 2]); v[i + 3] = __uint_as_float(r[i + 3]);
+            }
+        }
+#pragma unroll
+        for (int i = h; i < h + 16; ++i) {
+            if (ACT == 0) {      // per-member run-time activation, ONE copy of the code: both forms from one MUFU, then a select
+                const float t = tanh_approx(v[i]);
+                const float sw = fmaf(v[i], t, v[i]);
+                v[i] = rt_swish ? sw : t;
+            } else {
+                v[i] = (ACT == CMBPO_ACT_SWISH) ? swish_half(v[i]) : tanh_approx(v[i]);
+            }
+        }
+    };
+    tmem_ld16(d_addr, *reinterpret_cast<uint32_t(*)[16]>(&r[0]));
+    tmem_ld_wait();
+    tmem_ld16(d_addr + 16, *reinterpret_cast<uint32_t(*)[16]>(&r[16]));
+    convert16(0);
     tmem_ld_wait();
     tc_fence_before();
     __syncwarp();
     if ((threadIdx.x & 31) == 0) mbar_arrive_a(d_empty);
+    convert16(16);
     uint32_t q[16];
-    float v[32];
-    if (bias) {
-#pragma unroll
-        for (int i = 0; i < 32; i += 4) {
-            const float4 b = *reinterpret_cast<const float4*>(bias + i);
-            v[i] = __uint_as_float(r[i]) + b.x; v[i + 1] = __uint_as_float(r[i + 1]) + b.y;
-            v[i + 2] = __uint_as_float(r[i + 2]) + b.z; v[i + 3] = __uint_as_float(r[i + 3]) + b.w;
-        }
-    } else {
-#pragma unroll
-        for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-    }
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-        if (ACT == 0) {          // per-member run-time activation, ONE copy of the code: both forms from one MUFU, then a select
-            const float r = tanh_approx(v[i]);
-            const float sw = fmaf(v[i], r, v[i]);
-            v[i] = rt_swish ? sw : r;
-        } else {
-            v[i] = (ACT == CMBPO_ACT_SWISH) ? swish_half(v[i]) : tanh_approx(v[i]);
-        }
-    }
 #pragma unroll
     for (int c = 0; c < 16; ++c) q[c] = Cvt<FMT>::pack(v[2 * c], v[2 * c + 1]);
     if (dst_free) { mbar_wait_a(dst_free, dst_parity); tc_fence_after(); }
@@ -179,7 +191,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     constexpr int NHID = 1 + NMID;                 // HD x HD layers: NMID middle ones + the last hidden layer
     constexpr uint32_t COL_LAST = ((NMID + 1) & 1) ? COL_HB : COL_H1;     // WO: the last hidden layer's output
     extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+    // 1024-byte aligned base, as an OFFSET from the shared array: a pointer rebuilt from an integer loses the shared
+    // state space, and every access through it becomes a generic, long-scoreboard LD.E instead of an LDS
+    const uint32_t raw_s = smem_u32(smem_raw);
+    uint8_t* smem = smem_raw + (((raw_s + 1023u) & ~1023u) - raw_s);
     uint8_t* sXA = smem;
     uint8_t* sW = smem + XA_BYTES;
     uint8_t* sW2 = smem + SMEM_W2;
@@ -215,7 +230,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     __syncthreads();
     tc_fence_after();
     if (CL == 2) cluster_sync_all();      // the peer's barriers are initialised before anything is sent to them
-    const uint32_t cta_rank = (CL == 2) ? cluster_ctarank() : 0u;
     // The CTA owns all 512 columns, so the allocation can only start at lane 0 / column 0.  Treating
     // the base as the constant 0 keeps every MMA operand address in uniform registers (a base read
     // back from shared memory forces a per-instruction R2UR waterfall, ~100 cycles per MMA).
@@ -225,15 +239,21 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     // per CTA, so the last wave is balanced to within one member (a tile-granular split leaves the
     // last of ceil(782/148) = 6 rounds 72% empty), and neighbouring CTAs start on different members,
     // which spreads the weight streaming over E x more L2 addresses.
+    // Every role computes the unit range, its cluster rank and the live row count itself, after the register
+    // re-balancing below: values kept live across it were spilled by the 32-register control warps and reloaded from
+    // local memory at every unit boundary of the MMA issuer.
     const int n_groups = (p.E + G - 1) / G;         // E itself when G == 1
     // the live row count may sit in device memory (alive-row compaction of the rollout): rows beyond
     // it are not computed; strides still use the allocated N
-    const long long n_rows = p.n_dev ? *p.n_dev : p.N;
+    auto live_rows = [&]() -> long long { return p.n_dev ? *p.n_dev : p.N; };
     // CL == 2: a unit is (PAIR of row tiles, member), split over the cluster pairs; CTA r of a pair takes tile 2 tp + r
     // (an odd tile count leaves the last pair one tile without rows: it runs the protocol and stores nothing)
-    const long long n_units = ((n_rows + 128 * CL - 1) / (128 * CL)) * n_groups;      // < 2^31 (checked by the host)
-    const long long w_idx = blockIdx.x / CL, w_cnt = gridDim.x / CL;
-    const int u0 = (int)(n_units * w_idx / w_cnt), u1 = (int)(n_units * (w_idx + 1) / w_cnt);
+    auto unit_range = [&](int& u0, int& u1) {
+        const long long n_units = ((live_rows() + 128 * CL - 1) / (128 * CL)) * n_groups;   // < 2^31 (checked by the host)
+        const long long w_idx = blockIdx.x / CL, w_cnt = gridDim.x / CL;
+        u0 = (int)(n_units * w_idx / w_cnt); u1 = (int)(n_units * (w_idx + 1) / w_cnt);
+    };
+    auto cluster_rank = [&]() -> uint32_t { return (CL == 2) ? cluster_ctarank() : 0u; };
 #define CMBPO_TILE_OF(u) ((int)((u) / n_groups) * CL + (int)cta_rank)
 
     // (The pool is the CTA's own allocation of 640 x 96 registers: the 128 x (96 - 32) released by the
@@ -245,8 +265,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     // bound ptxas serialises them through one temporary: ~2000 instead of ~500 cycles per drain).
     if (warp < 4) {
     asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
+    int u0, u1;
+    unit_range(u0, u1);
     if (warp == 0) {
         // ===== main weight producer: layer-0 and layer-1 tiles, 32 KB per stage =====
+        const uint32_t cta_rank = cluster_rank();
         uint32_t s = 0, ph = 0;
         for (int u = u0; u < u1; ++u) {
             {
@@ -368,14 +391,14 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         // every wait is issued in the MIDDLE of a batch (after its first 8 MMAs): the W_FULL wait of the NEXT stage
         // and the hoisted accumulator hand-off; at a batch boundary only the commits remain.
         constexpr bool SPLIT = SINGLE && TPS == 4;
-        // stages this CTA consumes in total (the W_FULL wait runs one stage ahead only while a next stage exists)
-        const uint32_t total_stages = (uint32_t)(u1 - u0) * (uint32_t)(NC / G0 + NHID * NC * (KP / TPS));
-        uint32_t q_stage = 0;
+        // stages this CTA has still to consume, the current one excluded (the W_FULL wait runs one stage ahead only
+        // while a next stage exists).  A count down: one register, where a count up and its limit took two.
+        uint32_t stages_left = (uint32_t)(u1 - u0) * (uint32_t)(NC / G0 + NHID * NC * (KP / TPS));
         uint32_t pre_n = 0;                 // upcoming ring stages whose W_FULL phase was already seen complete
         if (!SINGLE || elect_one()) {
         int cur_tile = -1;
         for (int u = u0; u < u1; ++u) {
-            const int tile = CMBPO_TILE_OF(u);
+            const int tile = u / n_groups;          // (the tile pair when CL == 2)
             if (tile != cur_tile) {                 // a new row tile: its XA panel must have landed
                 cur_tile = tile;
                 mbar_wait(bar + X_FULL, it & 1);
@@ -385,7 +408,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
             {
                 for (int j0 = 0; j0 < NC; j0 += G0) {       // layer 0: D = XA x W0 chunk (G0 chunks per stage)
                     if (pre_n) --pre_n; else mbar_wait(bar + W_FULL + s, ph);
-                    ++q_stage;
+                    --stages_left;
 #pragma unroll
                     for (int jj = 0; jj < G0; ++jj) {
                         // one chunk per instruction, buffer = chunk parity: the two epilogue pairs run as
@@ -427,9 +450,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     }
                     for (int kq = 0; kq < KP / TPS; ++kq) {
                         if (pre_n) --pre_n; else mbar_wait(bar + W_FULL + s, ph);      // TMA completion: no tcgen05 fence needed
-                        ++q_stage;
+                        --stages_left;
                         auto mid_waits = [&]() {
-                            if (SPLIT && q_stage < total_stages) {       // the NEXT stage's weights
+                            if (SPLIT && stages_left > 0) {       // the NEXT stage's weights
                                 const uint32_t ns = (s + 1 == NSM) ? 0u : s + 1, nph = (s + 1 == NSM) ? (ph ^ 1u) : ph;
                                 mbar_wait(bar + W_FULL + ns, nph);
                                 pre_n = 1;
@@ -469,6 +492,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
     }
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
+        int u0, u1;
+        unit_range(u0, u1);
+        const long long n_rows = live_rows();
+        const uint32_t cta_rank = cluster_rank();
         // ===== epilogue: 4 warpgroups; pair (wg>>1) owns accumulator buffer (wg>>1), half (wg&1) its columns =====
         const int wg = (warp - 4) >> 2;
         const uint32_t pair = (uint32_t)wg >> 1, half = (uint32_t)wg & 1;
@@ -477,8 +504,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         const uint32_t lane_base = (uint32_t)(wq * 32) << 16;
         const uint32_t bar_a = smem_u32(bar);
         uint32_t g = 0, m = 0, c1 = 0;
-        // deferred OUT epilogue: the four warpgroups split the NP output columns (16 or 32 each)
-        int prev_e = 0; long long prev_grow = 0; uint32_t prev_m = 0; bool have_prev = false;
+        // deferred OUT epilogue: the four warpgroups split the NP output columns (16 or 32 each).  It drains unit `up`,
+        // the `mp`-th unit of this CTA; both follow from the loop counters, so no state of the previous unit is kept
+        // live across the unit loop (those registers were spilled to local memory)
         const int etid = (int)threadIdx.x - 128;                      // 0..511 among the epilogue threads
         // input scaler -> shared memory (identity when the net has none)
         if (etid < 64) {
@@ -487,8 +515,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
         }
         epi_bar();
         const int out_cw = (G > 1) ? p.NP : ((p.NP <= 64) ? 16 : 32);
-        auto out_epilogue = [&]() {
-            mbar_wait(bar + OUT_FULL, prev_m & 1);
+        auto out_epilogue = [&](int up, uint32_t mp) {
+            const int prev_e = up % n_groups;
+            const long long prev_grow = (long long)CMBPO_TILE_OF(up) * 128 + row;
+            mbar_wait(bar + OUT_FULL, mp & 1);
             tc_fence_after();
             const int c_begin = wg * out_cw;
             uint32_t r[32];
@@ -525,15 +555,13 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     }
                 }
             }
-            have_prev = false;
         };
         int cur_tile = -1;
-        long long grow = 0;
         for (int u = u0; u < u1; ++u) {
             const int tile = CMBPO_TILE_OF(u);
             const bool new_tile = tile != cur_tile;
             cur_tile = tile;
-            grow = (long long)tile * 128 + row;
+            const long long grow = (long long)tile * 128 + row;
             if (new_tile && wg == 0) {
                 const bool feed = grow < n_rows;
                 const float* xr = p.x + grow * p.ldx;
@@ -581,16 +609,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 // were copied to shared memory by the layer-2 producer warp.
                 const float* sb = sBias + (m & 1) * (BIAS_SLOT / 4);
                 mbar_wait_a(bar_a + 8 * (B_FULL + (m & 1)), (m >> 1) & 1);
+#pragma unroll 1
                 for (int i = 0; i < NC / 2; ++i) {               // layer-0 chunk j -> H1 columns
                     const int j = 2 * i + (int)pair;
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1;
-                    mbar_wait(bar + D_FULL + buf, n & 1);
-                    tc_fence_after();
                     // WO, NMID = 1: H1 is the previous unit's layer-2 A operand (see the kernel comment)
-                    const uint32_t h1_free = (WO && COL_LAST == COL_H1 && have_prev && i == 0) ? bar_a + 8 * OUT_FULL : 0u;
-                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, p.fold ? nullptr : sb + j * 64 + half * 32,
+                    const uint32_t h1_free = (WO && COL_LAST == COL_H1 && m > 0 && i == 0) ? bar_a + 8 * OUT_FULL : 0u;
+                    drain32<FMT, ACT>(bar_a + 8 * (D_FULL + buf), n & 1, tmem + COL_D + buf * 64 + half * 32 + lane_base, p.fold ? nullptr : sb + j * 64 + half * 32,
                                       tmem + COL_H1 + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf),
-                                      h1_free, WO ? (prev_m & 1) : 0u,
+                                      h1_free, WO ? ((m - 1) & 1) : 0u,
                                       ACT == 0 && p.member_act[e * G + j / CPM] != CMBPO_ACT_TANH);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * H1_FULL);
@@ -599,16 +626,15 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 // The previous member's OUT accumulator is drained HERE, after this member's layer-0
                 // drains: the accumulator is not touched again before this member's first layer-2
                 // MMA, so the global stores stay off the MMA warp's critical path.
-                if (have_prev) out_epilogue();
+                if (m > 0) out_epilogue(u - 1, m - 1);
                 if (NMID > 0) {
                     for (int lyr = 1; lyr <= NMID; ++lyr) {      // middle layer lyr: chunk j -> the other hidden buffer
                         const uint32_t col_dst = (lyr & 1) ? COL_HB : COL_H1;
+#pragma unroll 1
                         for (int i = 0; i < NC / 2; ++i) {
                             const int j = 2 * i + (int)pair;
                             const uint32_t gg = g + j, buf = pair, n = gg >> 1;
-                            mbar_wait(bar + D_FULL + buf, n & 1);
-                            tc_fence_after();
-                            drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + lyr * HD + j * 64 + half * 32,
+                            drain32<FMT, ACT>(bar_a + 8 * (D_FULL + buf), n & 1, tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + lyr * HD + j * 64 + half * 32,
                                               tmem + col_dst + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u);
                             __syncwarp();
                             if (lane == 0) mbar_arrive_a(bar_a + 8 * H1_FULL);
@@ -617,17 +643,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     }
                 }
                 if constexpr (WO) {
+#pragma unroll 1
                 for (int i = 0; i < NC / 2; ++i) {               // last hidden layer, chunk j -> buffer LAST, K panel j
                     const int j = 2 * i + (int)pair;
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1;
-                    mbar_wait(bar + D_FULL + buf, n & 1);
-                    tc_fence_after();
-                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + NHID * HD + j * 64 + half * 32,
+                    drain32<FMT, ACT>(bar_a + 8 * (D_FULL + buf), n & 1, tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + NHID * HD + j * 64 + half * 32,
                                       tmem + COL_LAST + j * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf), 0u, 0u);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * (HL_FULL + j));
                 }
                 } else
+#pragma unroll 1
                 for (int i = 0; i < NC / 2; ++i) {               // last hidden layer, chunk j -> an H2 buffer
                     const int j = 2 * i + (int)pair;
                     const uint32_t gg = g + j, buf = pair, n = gg >> 1, cc = c1 + j;
@@ -640,10 +666,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                     const uint32_t hbar = cc & 1, hn = cc >> 1, hb = (nh2 == 2) ? hbar : 0;
                     const uint32_t h2_free = (nh2 == 2) ? bar_a + 8 * (H2_EMPTY + hbar) : (cc == 0 ? 0u : bar_a + 8 * (H2_EMPTY + (hbar ^ 1)));
                     const uint32_t h2_par = (nh2 == 2) ? ((hn & 1) ^ 1) : ((((cc - 1) >> 1)) & 1);
-                    mbar_wait(bar + D_FULL + buf, n & 1);
-                    tc_fence_after();
-                    drain32<FMT, ACT>(tmem + COL_D + buf * 64 + half * 32 + lane_base, sb + NHID * HD + j * 64 + half * 32,
-                                      tmem + COL_H2 + hb * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf),
+                    drain32<FMT, ACT>(bar_a + 8 * (D_FULL + buf), n & 1, tmem + COL_D + buf * 64 + half * 32 + lane_base,
+                                      sb + NHID * HD + j * 64 + half * 32, tmem + COL_H2 + hb * 32 + half * 16 + lane_base, bar_a + 8 * (D_EMPTY + buf),
                                       h2_free, h2_par, ACT == 0 && p.member_act[e * G + j / CPM] != CMBPO_ACT_TANH);
                     __syncwarp();
                     if (lane == 0) mbar_arrive_a(bar_a + 8 * (H2_FULL + hbar));
@@ -651,11 +675,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) ens_mlp3_tc_kernel(const TcParams
                 __syncwarp();
                 if (lane == 0) mbar_arrive_a(bar_a + 8 * (B_EMPTY + (m & 1)));     // the bias buffer may be refilled
                 g += NC; c1 += NC;
-                prev_e = e; prev_grow = grow; prev_m = m; have_prev = true;
                 ++m;
             }
         }
-        if (have_prev) out_epilogue();
+        if (m > 0) out_epilogue(u1 - 1, m - 1);
     }
     tc_fence_before();
     __syncthreads();
